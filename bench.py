@@ -15,7 +15,12 @@ chain at 1M customers in total and splits it over the ranks instead.
 
 The timed `value` has the data resident in HBM (inputs 768 MB >> 126 MB L2, so every sweep streams
 from HBM; no extra L2 flush).  `e2e` is the same metric through the reference-facing call with HOST
-buffers: upload of the views from pinned memory, state set, K sweeps, read-back of table_of.
+buffers: upload of the views from pinned memory, state set, K sweeps, read-back of table_of.  K is --steps, as in
+the timed `value`; at small K the upload and the state set dominate it (a caller's chain runs thousands of sweeps).
+
+`--dump-outputs DIR` writes the chain state the timed sweeps leave behind (what mvg_get_state returns after the last
+timed sweep) as DIR/<name>.npy, so that two builds can be compared output for output on identical seeded inputs.
+Only the C3 workload (the default) dumps; c1, c2, c5 and --impl reference refuse the flag.
 """
 from __future__ import annotations
 
@@ -31,6 +36,7 @@ from pathlib import Path
 import numpy as np
 
 ROOT = Path(__file__).resolve().parent
+sys.dont_write_bytecode = True          # the tree may be read-only: nothing is written into it
 for p in (ROOT, ROOT / "multiview-clustering_b200"):
     if str(p) not in sys.path:
         sys.path.insert(0, str(p))
@@ -85,7 +91,13 @@ def parse():
     ap.add_argument("--no-checks", action="store_true", help="skip the sharded-vs-one-GPU replay and the CPU-mirror spot check")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-rows", type=int, default=0, help="rows of the CPU sample (0: sized for ~15 s)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="C3 only (the other workloads and --impl reference refuse it): "
+                    "write the state after the last timed sweep as DIR/<name>.npy (table_of of every row, per-table counts "
+                    "and sums, hyperparameters; float32/float64)")
+    args = ap.parse_args()
+    if args.dump_outputs and (args.workload != "c3" or args.impl != "b200"):
+        ap.error("--dump-outputs applies to the C3 workload of --impl b200")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------
@@ -682,9 +694,9 @@ def _main(args, out):
         elif ok:
             s.p2p_disable()                                     # a peer could not map the buffers: everybody uses NCCL
 
-    def timed_run(w, steps, warmup, sample_clocks, incremental=None):
+    def timed_run(w, steps, warmup, sample_clocks, incremental=None, keep_state=False):
         """W warm-up sweeps, then `steps` sweeps timed on the device (CUDA events on the library's stream, barrier and
-        synchronize on both sides, max over ranks)."""
+        synchronize on both sides, max over ranks).  keep_state: also return the state the last timed sweep left."""
         s = make_sampler(w, attach=True, debug_export=2 if args.role_profile else 0, incremental=incremental)
         enable_p2p(s)
         w.set_state(s)
@@ -704,6 +716,7 @@ def _main(args, out):
         wall_ms = 1e3 * (time.perf_counter() - t_wall)
         if clocks:
             clocks.stop_flag = True
+        state = s.get_state() if keep_state else None         # before profile_sweep below, which sweeps again
         t = torch.tensor([s.last_sweep_ms()], device="cuda")
         if dist is not None:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -722,7 +735,7 @@ def _main(args, out):
         prof = [s.profile_sweep(do_hyper) for _ in range(5)]      # per-kernel device times of a few extra sweeps
         kern = {k: float(np.median([p[k] for p in prof])) for k in prof[0]}
         return {"s": s, "dev_ms": dev_ms, "wall_ms": wall_ms, "launches": s.launch_count() - l0, "kern": kern, "inreg": inreg,
-                "clocks": clocks.summary() if clocks else None}
+                "clocks": clocks.summary() if clocks else None, "state": state}
 
     def roofline_of(w, kern, traffic, inreg=None):
         alg_bytes = w.n_local * (sum(DIMS) * 4 + 8)
@@ -745,8 +758,10 @@ def _main(args, out):
     # ---------------- the headline run: `--scaling` (default strong: north_star's N = 1M split over the GPUs) ----------
     n_total = args.rows * world if args.scaling == "weak" else args.rows
     W = Workload(n_total, args.k_true)
-    R = timed_run(W, args.steps, args.warmup, sample_clocks=True)
+    R = timed_run(W, args.steps, args.warmup, sample_clocks=True, keep_state=bool(args.dump_outputs))
     s = R["s"]
+    if args.dump_outputs:
+        dump_state(R["state"], W.lo, args.dump_outputs, dist, rank, world)
     ms_per_step = R["dev_ms"] / args.steps
     updates = n_total * len(DIMS) * CAP
     value = updates * args.steps / (R["dev_ms"] * 1e-3)
@@ -772,7 +787,7 @@ def _main(args, out):
     # ---------------- e2e: one chain through the C ABI with HOST buffers ---------------------------------------------------
     e2e = None
     if not args.no_e2e:
-        k_e2e = max(args.steps, 1000)            # a chain, not an upload: the reference's own script runs M = 10 000 sweeps per call (New_Simulation.R:123-132)
+        k_e2e = args.steps
         thin = max(1, k_e2e // 4)
         s2 = make_sampler(W, attach=False)       # handle (+ borrowed communicator): set-up, not part of a chain's run
         barrier()
@@ -920,6 +935,29 @@ def _main(args, out):
         print(json.dumps(line), file=out)
     if dist is not None:
         dist.destroy_process_group()
+
+
+def dump_state(st, lo, out_dir, dist, rank, world):
+    """The state after the last timed sweep as <out_dir>/<name>.npy: table_of in row order (gathered from the ranks; every
+    row up to 8M rows, beyond that every k-th row so that the dump stays under 64 MB), the per-table counts and sums and
+    the hyperparameters, which every rank holds alike."""
+    tab = st["table_of"]
+    if dist is not None:
+        parts = [None] * world
+        dist.all_gather_object(parts, (lo, tab))
+        tab = np.concatenate([p[1] for p in sorted(parts, key=lambda p: p[0])])
+    if rank != 0:
+        return
+    tab = tab[::-(-len(tab) // 8_000_000)]
+    out = {"table_of": tab.astype(np.float32), "n_t": st["n_t"].astype(np.float32),
+           "dish_of": st["dish_of"].astype(np.float32), "n_vk": st["n_vk"].astype(np.float32),
+           "l_vk": st["l_vk"].astype(np.float32), "sum_y": np.stack(st["S1"]), "sum_y2": st["sum_y2"],
+           "alpha_v": st["alpha_v"], "sigma_v": st["sigma_v"], "tau_v": st["tau_v"],
+           "alpha_sigma_global": np.array([st["alpha_g"], st["sigma_g"]])}
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, a in out.items():
+        np.save(d / f"{name}.npy", a)
 
 
 def spot_check_draws(mvc_b200, W, device, engine):

@@ -58,6 +58,19 @@ def c1_data(n=500, seed=1999):
     return [v1.astype(np.float32), v2.astype(np.float32)], [z1, z2]
 
 
+def reference_chain(seed, n, M, burn, thin):
+    """Saved states of the reference's run_gibbs_cpp on c1_data(n) (tests/golden/reference_chains.npz; its "source" entry
+    says what wrote them), in the form pyoracle.ref_run_gibbs returns them, and the number of uniforms + normals drawn."""
+    z = np.load(Path(__file__).parent / "golden" / "reference_chains.npz")
+    key = f"{seed}_{n}_{M}_{burn}_{thin}"
+    tab, T, dish, hyp = (z[f"{key}/{k}"] for k in ("table_of", "T", "dish_of", "hypers"))
+    d = dish.shape[1]
+    states = [{"table_of": tab[s].astype(np.int32), "dish_of": dish[s, :, :T[s]].astype(np.int32),
+               "alpha_v": hyp[s, :d], "sigma_v": hyp[s, d:2 * d], "tau_v": hyp[s, 2 * d:3 * d],
+               "alpha_global": hyp[s, 3 * d], "sigma_global": hyp[s, 3 * d + 1]} for s in range(len(T))]
+    return states, int(z[f"{key}/calls"])
+
+
 @pytest.fixture(scope="session")
 def oracle():
     import pyoracle

@@ -11,7 +11,7 @@
 """
 import numpy as np
 import pytest
-from conftest import c1_data, make_mixture
+from conftest import c1_data, make_mixture, reference_chain
 
 pytestmark = pytest.mark.gpu
 RTOL_LOGLIK = 1e-5     # north_star: "<= 1e-5 FP32"
@@ -214,7 +214,7 @@ def test_error_codes_and_ordering():
     s.close()
 
 
-def test_run_gibbs_posterior_summaries_match_reference(oracle):
+def test_run_gibbs_posterior_summaries_match_reference():
     """north_star's third bullet: posterior summaries of a long GPU chain (synchronous sweeps)
     against the sequential reference chain on config-1 data: ARI vs truth, kernel variance, cluster count."""
     from sklearn.metrics import adjusted_rand_score as ari
@@ -228,13 +228,11 @@ def test_run_gibbs_posterior_summaries_match_reference(oracle):
                      for s in range(30)])
     tau = np.array([res["tau_v"][v].mean() for v in range(2)])
     assert aris[:, 0].mean() > 0.85 and aris[:, 1].mean() > 0.75, aris.mean(0)
-    if oracle.have_ref():
-        y = np.stack([v.astype(np.float64) for v in views])
-        tr = oracle.ref_run_gibbs(y, 1500, 1200, 10, seed=1999)
-        ref_ari = np.array([[ari(truth[v], t["dish_of"][v][t["table_of"]]) for v in range(2)] for t in tr])
-        ref_tau = np.array([[t["tau_v"][v] for v in range(2)] for t in tr]).mean(0)
-        assert np.all(np.abs(aris.mean(0) - ref_ari.mean(0)) < 0.12), (aris.mean(0), ref_ari.mean(0))
-        assert np.all(np.abs(tau / ref_tau - 1.0) < 0.25), (tau, ref_tau)
+    tr, _ = reference_chain(1999, 500, 1500, 1200, 10)
+    ref_ari = np.array([[ari(truth[v], t["dish_of"][v][t["table_of"]]) for v in range(2)] for t in tr])
+    ref_tau = np.array([[t["tau_v"][v] for v in range(2)] for t in tr]).mean(0)
+    assert np.all(np.abs(aris.mean(0) - ref_ari.mean(0)) < 0.12), (aris.mean(0), ref_ari.mean(0))
+    assert np.all(np.abs(tau / ref_tau - 1.0) < 0.25), (tau, ref_tau)
 
 
 def _chain_summaries(table_of, dish_of, hyp_tau, truth, n):
@@ -256,18 +254,16 @@ def _chain_summaries(table_of, dish_of, hyp_tau, truth, n):
             "cocl": [c / S for c in cocl], "tau": np.array([np.mean(t) for t in hyp_tau])}
 
 
-def test_long_chain_statistics_against_the_sequential_reference(oracle):
+def test_long_chain_statistics_against_the_sequential_reference():
     """north_star's third correctness bullet, stated: over 4 seeds of config 1 (N = 500, two scalar views, 2000 sweeps,
-    the last 500 kept every 10th) the GPU chain and the UNMODIFIED sequential reference (oracle/_ref, run_gibbs_cpp) agree
+    the last 500 kept every 10th) the GPU chain and the UNMODIFIED sequential reference (run_gibbs_cpp; its saved states are
+    in tests/golden/reference_chains.npz) agree
     on the per-view number of clusters (dishes), the pooled co-clustering matrix, the ARI against the truth and the
     kernel variances.  The number of TABLES is where a synchronous sweep differs from the sequential one (several
     customers open tables in the same sweep; tables sharing a dish do not change the clustering): it is printed, and the
     blocked sweep (mvg_set_sweep_blocks: statistics refreshed between row blocks) must move it towards the reference."""
     import mvc_b200
-    if not oracle.have_ref():
-        pytest.skip("compiled reference not available")
     views, truth = c1_data(500)
-    y = np.stack([v.astype(np.float64) for v in views])
     n, seeds = 500, (1999, 7, 42, 2024)
     M, burn, thin = 2000, 1500, 10
 
@@ -278,7 +274,7 @@ def test_long_chain_statistics_against_the_sequential_reference(oracle):
 
     ref_runs, gpu_runs, blk_runs = [], [], []
     for sd in seeds:
-        tr = oracle.ref_run_gibbs(y, M, burn, thin, seed=sd)
+        tr, _ = reference_chain(sd, n, M, burn, thin)
         ref_runs.append(_chain_summaries([t["table_of"] for t in tr], [t["dish_of"] for t in tr],
                                          [[t["tau_v"][v] for t in tr] for v in range(2)], truth, n))
         for blocks, runs in ((1, gpu_runs), (32, blk_runs)):

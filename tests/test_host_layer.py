@@ -8,7 +8,7 @@ from pathlib import Path
 
 import numpy as np
 import pytest
-from conftest import c1_data
+from conftest import c1_data, reference_chain
 
 ROOT = Path(__file__).resolve().parents[1]
 HOST = ROOT / "multiview-clustering_b200" / "host"
@@ -90,12 +90,11 @@ def test_run_gibbs_cpp_through_the_host_layer_equals_the_c_abi_chain():
 
 
 @pytest.mark.gpu
-def test_utils_inspectors_on_the_mirrored_state_equal_the_compiled_reference(oracle):
+def test_utils_inspectors_on_the_mirrored_state_equal_the_fp64_restatement(oracle):
     """multiview_utils.h over the device chain: compute_table_probs_with_cache / compute_f_vk on the state mirrored from
-    the GPU give what the UNMODIFIED reference (oracle/_ref/libmvref.so) gives for the same state; saved_loglik is
-    filled on every kept sweep; the single-customer mutators raise."""
-    if not oracle.have_ref():
-        pytest.skip("compiled reference not available")
+    the GPU give the weights of the FP64 restatement (oracle/mv_oracle.c, whose row weights test_oracle_vs_reference pins
+    to vectors from the compiled reference at 2e-11) for the same state; saved_loglik is filled on every kept sweep; the
+    single-customer mutators raise."""
     views, _ = c1_data(300)
     y = np.ascontiguousarray(np.stack([v.astype(np.float64) for v in views]))
     L = build_host()
@@ -113,12 +112,18 @@ def test_utils_inspectors_on_the_mirrored_state_equal_the_compiled_reference(ora
         dish[v] = row
     hyp = np.empty(8)
     L.host_final_hypers(hyp.ctypes.data_as(C.POINTER(C.c_double)))
-    K = np.array([dish[v].max() + 1 for v in range(2)], np.int32)
-    oracle.ref_load(y, tab, dish, K, hyp[0:2], hyp[2:4], hyp[4:6], hyp[6], hyp[7])
+    cap = max(T, int(dish.max()) + 1) + 1                       # one slot free for a new table
+    dish_cap = np.pad(dish, ((0, 0), (0, cap - T)), constant_values=-1)
     L.host_f_vk.restype = C.c_double
     L.host_f_vk_new.restype = C.c_double
     for i in (0, 17, 150, 299):
-        pe, pn = oracle.ref_table_probs(i, T)
+        # the weights of customer i while it is seated = the oracle's leave-one-out weights of a copy of row i at its table
+        o = oracle.OracleState([np.append(y[v], y[v][i]).astype(np.float32) for v in range(2)], cap)
+        o.alpha_v[:], o.sigma_v[:], o.tau_v[:] = hyp[0:2], hyp[2:4], hyp[4:6]
+        o.alpha_g, o.sigma_g = hyp[6], hyp[7]
+        o.set_assignment(np.append(tab, tab[i]), dish_cap)
+        w = np.exp(o.row_logweights(len(tab)))
+        pe, pn = w[:T], w[cap]
         hpe, hpn = np.zeros(T), C.c_double()
         assert L.host_table_probs(i, hpe.ctypes.data_as(C.POINTER(C.c_double)), C.byref(hpn)) == T, L.host_last_error()
         # the mirror holds the device's FP32-tree sums: the statistics agree to 1e-5, so do the weights
@@ -129,17 +134,15 @@ def test_utils_inspectors_on_the_mirrored_state_equal_the_compiled_reference(ora
 
 
 @pytest.mark.gpu
-def test_run_gibbs_cpp_sequential_engine_equals_the_compiled_reference(oracle):
+def test_run_gibbs_cpp_sequential_engine_equals_the_compiled_reference():
     """mvhost::sequential = true: run_gibbs_cpp (host C++, the reference's signature) on MVG_ENGINE_SEQ returns the partitions
     the UNMODIFIED reference returns for the same data and seed — chain-level integer equality through the host layer."""
-    if not oracle.have_ref():
-        pytest.skip("compiled reference not available")
     views, _ = c1_data(300)
     y = np.ascontiguousarray(np.stack([v.astype(np.float64) for v in views]))
     L = build_host()
     L.host_last_error.restype = C.c_char_p
     S = L.host_run_seq(300, 2, y.ctypes.data_as(C.POINTER(C.c_double)), 200, 100, 20, C.c_ulonglong(11))
-    tr = oracle.ref_run_gibbs(y, 200, 100, 20, seed=11)
+    tr, _ = reference_chain(11, 300, 200, 100, 20)
     assert S == len(tr) == 5, L.host_last_error()
     for s in range(S):
         tab = np.empty(300, np.int32)

@@ -1,6 +1,6 @@
 """MVG_ENGINE_SEQ (csrc/mv_seq_core.h): the reference's sequential sampler restated for one thread of control.
-Chain-level parity with the UNMODIFIED reference (oracle/_ref/libmvref.so, run_gibbs_cpp) driven by the same call-ordered
-Philox stream:
+Chain-level parity with the UNMODIFIED reference (run_gibbs_cpp, saved states in tests/golden/reference_chains.npz) driven by
+the same call-ordered Philox stream:
 
   * CPU (here): the same source compiled for the host (tests/seq_host_check.cpp, test scaffolding) visits the same states
     as the reference — table_of, dish_of of every kept sweep identical, hyperparameters bitwise equal, the same number of
@@ -13,7 +13,7 @@ from pathlib import Path
 
 import numpy as np
 import pytest
-from conftest import c1_data
+from conftest import c1_data, reference_chain
 
 ROOT = Path(__file__).resolve().parents[1]
 OUT = ROOT / "tests" / "_build" / "libseqhost.so"
@@ -48,13 +48,10 @@ def _compare(tr, tab, T, dish, hyp, d, exact_hypers):
 
 
 @pytest.mark.parametrize("seed,n,M,burn,thin", [(1999, 500, 300, 100, 10), (7, 500, 400, 0, 40), (42, 200, 500, 250, 25)])
-def test_sequential_core_follows_the_compiled_reference_state_for_state(oracle, seed, n, M, burn, thin):
-    if not oracle.have_ref():
-        pytest.skip("compiled reference not available")
+def test_sequential_core_follows_the_compiled_reference_state_for_state(seed, n, M, burn, thin):
     y, _ = _data(n)
     d = y.shape[0]
-    tr = oracle.ref_run_gibbs(y, M, burn, thin, seed=seed)
-    ref_calls = oracle.ref().ref_uniform_calls() + oracle.ref().ref_normal_calls()
+    tr, ref_calls = reference_chain(seed, n, M, burn, thin)
     S, t_cap, k_cap = len(tr), 1024, 2 * M + 64
     tab = np.zeros((S, n), np.int32); T = np.zeros(S, np.int32); dish = np.zeros((S, d, t_cap), np.int32)
     hyp = np.zeros((S, 3 * d + 2)); calls = C.c_ulonglong()
@@ -69,14 +66,11 @@ def test_sequential_core_follows_the_compiled_reference_state_for_state(oracle, 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("seed,n,M,burn,thin", [(1999, 500, 300, 100, 10), (7, 500, 600, 0, 50)])
-def test_sequential_engine_on_the_device_follows_the_reference(oracle, seed, n, M, burn, thin):
+def test_sequential_engine_on_the_device_follows_the_reference(seed, n, M, burn, thin):
     import mvc_b200
-    if not oracle.have_ref():
-        pytest.skip("compiled reference not available")
     y, truth = _data(n)
     d = y.shape[0]
-    tr = oracle.ref_run_gibbs(y, M, burn, thin, seed=seed)
-    ref_calls = oracle.ref().ref_uniform_calls() + oracle.ref().ref_normal_calls()
+    tr, ref_calls = reference_chain(seed, n, M, burn, thin)
     res = mvc_b200.run_gibbs_seq([y[v] for v in range(d)], M, burn, thin, seed=seed)
     S = len(res["table_of"])
     assert S == len(tr) and res["stream_calls"] == ref_calls
