@@ -26,8 +26,9 @@
  * Semantics that differ from the reference BY DESIGN (DESIGN.md §2):
  *   - the sweep is synchronous: every customer is scored against the sweep-start statistics with
  *     only its own contribution removed, instead of seeing the moves of customers 0..i-1;
- *   - table and dish slots have a fixed capacity `cap`; a new table can only open in a slot that
- *     was free at sweep start, births are seated in global row order and the overflow stays put;
+ *   - table and dish slots have a fixed capacity `cap` (32, 64, 128 or 256; the reference's pool has no limit); a new
+ *     table can only open in a slot that was free at sweep start, births are seated in global row order and the
+ *     overflow stays put;
  *   - the random stream is Philox4x32-10 addressed by (seed, chain, sweep, row, slot) instead of
  *     R's call-ordered generator;
  *   - a customer for whom NO option has weight stays at its own table; the reference seats it at table 0 without drawing
@@ -80,7 +81,9 @@ typedef struct mvg_config {
   int64_t n_rows_global;   /* customers over all shards; == n_rows on one GPU */
   int64_t row_offset;      /* global index of this shard's row 0 (Philox addressing, birth order) */
   int32_t n_views;         /* d in the reference */
-  int32_t cap;             /* capacity of table slots and of dish slots per view (32 or 64) */
+  int32_t cap;             /* capacity of table slots and of dish slots per view: 32, 64, 128 or 256 (other values:
+                              MVG_EUNSUPPORTED).  128 and 256 run on the CUDA-core engine only: MVG_ENGINE_AUTO picks
+                              it, an explicit MVG_ENGINE_TCGEN05 / _FAST is MVG_EUNSUPPORTED */
   uint64_t seed;           /* Philox key (echo of set.seed(1999), New_Simulation.R:12) */
   uint32_t chain;          /* chain id, folded into the Philox key */
   int32_t engine;          /* MVG_ENGINE_* : which likelihood+draw kernel */
@@ -162,8 +165,8 @@ int mvg_sweep(mvg_handle* h, int32_t n_sweeps, int32_t do_hyper);
  *                                fixed order, into running FP64 sums; every `rebuild_every`-th sweep is a full rebuild,
  *                                which bounds the rounding drift (counts are integers and exact either way).  The
  *                                sweep then streams the features ONCE instead of twice.  Available where the tile
- *                                statistics kernel is (cap 64, up to three dense views of dim 64); elsewhere it falls
- *                                back to rebuilding. */
+ *                                statistics kernel is (cap 64, up to three dense views of dim 64); elsewhere (cap 32,
+ *                                128, 256, other view shapes) it falls back to rebuilding. */
 enum { MVG_STATS_REBUILD = 0, MVG_STATS_INCREMENTAL = 1 };
 int mvg_set_stats_mode(mvg_handle* h, int32_t mode, int32_t rebuild_every);
 /* Blocked sweeps: one sweep becomes `blocks` passes; pass b redraws the customers with (global row) % blocks == b

@@ -297,7 +297,8 @@ int mvg_create(const mvg_config* cfg, mvg_handle** out) {
   if (cfg->abi_version != MVG_ABI_VERSION) return fail(nullptr, MVG_EINVAL, "abi_version mismatch");
   if (cfg->n_rows <= 0 || cfg->n_rows > 0x7fffffffLL) return fail(nullptr, MVG_EINVAL, "n_rows out of range");
   if (cfg->n_views <= 0 || cfg->n_views > kMaxViews) return fail(nullptr, MVG_EINVAL, "n_views out of range");
-  if (cfg->cap != 32 && cfg->cap != 64) return fail(nullptr, MVG_EUNSUPPORTED, "cap must be 32 or 64");
+  if (cfg->cap != 32 && cfg->cap != 64 && cfg->cap != 128 && cfg->cap != 256)
+    return fail(nullptr, MVG_EUNSUPPORTED, "cap must be 32, 64, 128 or 256");
   if (cfg->world < 1 || cfg->world > 16 || cfg->rank < 0 || cfg->rank >= cfg->world)
     return fail(nullptr, MVG_EINVAL, "rank/world out of range");
   if (cfg->n_rows_global < cfg->n_rows || cfg->row_offset < 0 || cfg->row_offset + cfg->n_rows > cfg->n_rows_global)

@@ -55,12 +55,15 @@ __global__ void k_counts_scatter(const Ctx c, const int delta) {
   }
 }
 
-__global__ void k_counts_tables(const Ctx c) {
+// MAXCAP: 64 (one mask word per slot) or 256; cap is a power of two <= MAXCAP.
+template <int MAXCAP>
+__global__ void k_counts_tables(const Ctx c, const int log2cap) {
+  constexpr int kWords = MAXCAP / 64;
   const int v = nth_count_view(c, blockIdx.y);
-  __shared__ int32_t s_dish[64];
-  __shared__ double s_den[64];
-  __shared__ float s_l2zero[64];                 // log2 theta of a word the dish has never seen: most cells of the table
-  __shared__ unsigned long long s_mask[64];      // the table slots serving the same dish as slot t
+  __shared__ int32_t s_dish[MAXCAP];
+  __shared__ double s_den[MAXCAP];
+  __shared__ float s_l2zero[MAXCAP];                         // log2 theta of a word the dish has never seen: most cells of the table
+  __shared__ unsigned long long s_mask[MAXCAP][kWords];      // the table slots serving the same dish as slot t
   const int cap = c.cap;
   if (threadIdx.x < cap) {
     const int k = c.dish_of[v * cap + threadIdx.x];
@@ -71,10 +74,14 @@ __global__ void k_counts_tables(const Ctx c) {
   }
   __syncthreads();
   if (threadIdx.x < cap) {
-    unsigned long long m = 0ull;
     const int k = s_dish[threadIdx.x];
-    if (k >= 0) for (int t2 = 0; t2 < cap; ++t2) if (s_dish[t2] == k) m |= 1ull << t2;
-    s_mask[threadIdx.x] = m;
+#pragma unroll
+    for (int wi = 0; wi < kWords; ++wi) {
+      unsigned long long m = 0ull;
+      if (k >= 0) for (int j = 0; j < 64 && 64 * wi + j < cap; ++j) if (s_dish[64 * wi + j] == k) m |= 1ull << j;
+      s_mask[threadIdx.x][wi] = m;
+    }
+    s_mask[threadIdx.x][threadIdx.x >> 6] &= ~(1ull << (threadIdx.x & 63));   // the slot itself is read first
   }
   __syncthreads();
   // (every view's scatter has read table_prev by now — this kernel follows it in the stream: the seating the counts now
@@ -82,16 +89,17 @@ __global__ void k_counts_tables(const Ctx c) {
   if (blockIdx.y == 0)
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < c.n_rows; i += gridDim.x * blockDim.x) c.table_prev[i] = c.table_cur[i];
   const size_t total = (size_t)c.vocab[v] * cap;
-  const int shift = (cap == 64) ? 6 : 5;
   for (size_t e = (size_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (size_t)gridDim.x * blockDim.x) {
-    const int t = (int)(e & (size_t)(cap - 1));             // cap is 32 or 64 (mvg_create): no 64-bit division per cell
-    const size_t w = e >> shift;
+    const int t = (int)(e & (size_t)(cap - 1));             // cap is a power of two (mvg_create): no 64-bit division per cell
+    const size_t w = e >> log2cap;
     int32_t cd = 0;
     float l2 = 0.0f;
     if (s_dish[t] >= 0) {
       const int32_t* row = c.cnt_t[v] + w * cap;
       cd = row[t];                                              // usually the dish's only table
-      for (unsigned long long m = s_mask[t] & ~(1ull << t); m; m &= m - 1ull) cd += row[__ffsll((long long)m) - 1];
+#pragma unroll
+      for (int wi = 0; wi < kWords; ++wi)
+        for (unsigned long long m = s_mask[t][wi]; m; m &= m - 1ull) cd += row[64 * wi + __ffsll((long long)m) - 1];
       l2 = (cd == 0) ? s_l2zero[t] : (float)log2(((double)c.count_beta + (double)cd) / s_den[t]);
     }
     c.cnt_d[v][e] = cd;
@@ -152,8 +160,17 @@ __global__ void __launch_bounds__(512) k_counts_loglik(const Ctx c) {
           const int cl = __shfl_sync(0xffffffffu, col_l, src);
           xs[u] = __shfl_sync(0xffffffffu, xv_l, src);
           const float* p = l2t + (size_t)cl * CAP + lane * PER;
-          if (PER == 2) { const float2 t2 = __ldg(reinterpret_cast<const float2*>(p)); lv[u][0] = t2.x; lv[u][PER - 1] = t2.y; }
-          else lv[u][0] = __ldg(p);
+          if constexpr (PER >= 4) {
+#pragma unroll
+            for (int q = 0; q < PER; q += 4) {
+              const float4 t4 = __ldg(reinterpret_cast<const float4*>(p) + q / 4);
+              lv[u][q] = t4.x; lv[u][q + 1] = t4.y; lv[u][q + 2] = t4.z; lv[u][q + 3] = t4.w;
+            }
+          } else if constexpr (PER == 2) {
+            const float2 t2 = __ldg(reinterpret_cast<const float2*>(p)); lv[u][0] = t2.x; lv[u][PER - 1] = t2.y;
+          } else {
+            lv[u][0] = __ldg(p);
+          }
         }
 #pragma unroll
         for (int u = 0; u < kFlight; ++u) {
@@ -177,8 +194,13 @@ cudaError_t launch_counts_loglik(const Ctx& c, cudaStream_t s) {
   int blocks = (c.n_rows + 15) / 16;               // 16 warps per block
   if (blocks > 148 * 4) blocks = 148 * 4;
   const dim3 grid(blocks, c.n_count_views);         // all count views in one launch
-  if (c.cap == 64) k_counts_loglik<64><<<grid, 512, 0, s>>>(c);
-  else k_counts_loglik<32><<<grid, 512, 0, s>>>(c);
+  switch (c.cap) {
+    case 32: k_counts_loglik<32><<<grid, 512, 0, s>>>(c); break;
+    case 64: k_counts_loglik<64><<<grid, 512, 0, s>>>(c); break;
+    case 128: k_counts_loglik<128><<<grid, 512, 0, s>>>(c); break;
+    case 256: k_counts_loglik<256><<<grid, 512, 0, s>>>(c); break;
+    default: return cudaErrorInvalidValue;
+  }
   return cudaGetLastError();
 }
 
@@ -204,7 +226,9 @@ cudaError_t launch_counts_rebuild(const Ctx& c, bool delta, cudaStream_t s) {
   k_counts_scatter<<<dim3(blocks, c.n_count_views), 256, 0, s>>>(c, delta ? 1 : 0);
   int tb = (int)((max_cells + 255) / 256);
   if (tb > 148 * 8) tb = 148 * 8;
-  k_counts_tables<<<dim3(tb, c.n_count_views), 256, 0, s>>>(c);
+  const int log2cap = __builtin_ctz((unsigned)c.cap);
+  if (c.cap <= 64) k_counts_tables<64><<<dim3(tb, c.n_count_views), 256, 0, s>>>(c, log2cap);
+  else k_counts_tables<256><<<dim3(tb, c.n_count_views), 256, 0, s>>>(c, log2cap);   // one thread per slot: 256 threads
   return cudaGetLastError();
 }
 

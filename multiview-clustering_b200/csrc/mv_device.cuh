@@ -407,4 +407,130 @@ struct RowEpilogue {
   }
 };
 
+// The same draw for CAP = 128 / 256 (CUDA-core engine).  There, CAP running log-weights per thread do not fit in registers,
+// so they live in shared memory — float2 pairs (2i, 2i+1) at lw[i * NT], one column per thread of an NT-thread block — and
+// the caller hands over the dot products 16 tables at a time, in ascending table order, instead of all CAP at once.  The
+// arithmetic is RowEpilogue's operation for operation (oracle/mv_oracle.c:mvo_stageB_f32_mixed restates it for any cap):
+// per view each half streams its log-sum-exp over ascending chunks, the halves merge half A first, and the draw takes
+// the per-half totals (partial sums over t mod 4, fixed tree) and scans half B from HA.
+template <int CAP, int NT>
+struct WideRowEpilogue {
+  static constexpr int HALF = CAP / 2;
+  static_assert(HALF % kEpiChunk == 0, "half of the table capacity must be a multiple of the epilogue chunk");
+  float2* lw;            // this thread's column of the block's [CAP/2][NT] array
+  int t0, single;
+  float lnew;
+  // per view
+  float mx, s, mxA, sA, nxx, A1r, C1r;
+  int k0, lone0;
+
+  __device__ __forceinline__ float2& at(int i) const { return lw[i * NT]; }
+
+  __device__ __forceinline__ void begin(float2* lw_col, const TableMass* __restrict__ tm, const float* __restrict__ lm,
+                                        const GlobalParam& g, int t0_) {
+    lw = lw_col;
+    t0 = t0_;
+    const TableMass own = tm[t0_];
+    single = own.single;
+    lnew = single ? g.LMN1 : g.LMN0;
+    for (int i = 0; i < CAP / 2; ++i)             // the customer's own table counts n_t - 1
+      at(i) = make_float2((2 * i == t0_) ? own.LM1 : lm[2 * i], (2 * i + 1 == t0_) ? own.LM1 : lm[2 * i + 1]);
+  }
+
+  // A dense view: A1r / C1r from the own table; a count view overrides them after this call (see RowEpilogue::view_counts).
+  __device__ __forceinline__ void view_begin(const PairHot* __restrict__ hot, const TableCold* __restrict__ cold, float xx) {
+    const TableCold own = cold[t0];
+    k0 = reinterpret_cast<const int32_t*>(&hot[t0 >> 1].dish0)[t0 & 1];
+    lone0 = own.lone; A1r = own.A1; C1r = own.C1;
+    nxx = -xx;
+    mx = kMasked;
+    s = 0.0f;
+  }
+
+  // Tables base .. base+15 (base a multiple of 16, called in ascending order): acc[j] = x . m_{base + j}.
+  __device__ __forceinline__ void chunk(const PairHot* __restrict__ hot, const TableCold* __restrict__ cold, int base,
+                                        const float (&acc)[kEpiChunk]) {
+    if (base == HALF) { mxA = mx; sA = s; mx = kMasked; s = 0.0f; }   // half A is complete
+    float2 term[kEpiChunk / 2];
+    float c0 = kMasked, c1 = kMasked;
+    const float2 two = splat2(2.0f), nxx2 = splat2(nxx);
+#pragma unroll
+    for (int p = 0; p < kEpiChunk / 2; ++p) {
+      const int i = base / 2 + p;
+      const float4 qa = reinterpret_cast<const float4*>(&hot[i])[0];   // A0 A1 C0 C1
+      const float4 qb = reinterpret_cast<const float4*>(&hot[i])[1];   // W0 W1 dish0 dish1
+      const float2 e = ffma2(two, make_float2(acc[2 * p], acc[2 * p + 1]), nxx2);
+      float2 L = ffma2(make_float2(qa.x, qa.y), e, make_float2(qa.z, qa.w));
+      const bool same0 = __float_as_int(qb.z) == k0, same1 = __float_as_int(qb.w) == k0;
+      if (same0) L.x = __fmaf_rn(A1r, e.x, C1r);     // leave-one-out only where the dish is the customer's own
+      if (same1) L.y = __fmaf_rn(A1r, e.y, C1r);
+      at(i) = fadd2(at(i), L);
+      float2 w = make_float2(qb.x, qb.y);
+      if (same0 && single) w.x = cold[2 * i].W1;
+      if (same1 && single) w.y = cold[2 * i + 1].W1;
+      term[p] = fadd2(L, w);
+      c0 = fmaxf(c0, term[p].x);
+      c1 = fmaxf(c1, term[p].y);
+    }
+    const float mn = fmaxf(mx, fmaxf(c0, c1));
+    s = __fmul_rn(s, exp2m(__fadd_rn(mx, -mn)));
+    mx = mn;
+    const float2 nmn2 = splat2(-mn);
+    float2 pa = splat2(0.0f), pb = splat2(0.0f);        // partial sums over j mod 4 = (0,1) and (2,3)
+#pragma unroll
+    for (int p = 0; p < kEpiChunk / 2; p += 2) {
+      pa = fadd2(pa, exp2w2<false>(fadd2(term[p], nmn2)));
+      pb = fadd2(pb, exp2w2<false>(fadd2(term[p + 1], nmn2)));
+    }
+    s = __fadd_rn(s, __fadd_rn(__fadd_rn(pa.x, pa.y), __fadd_rn(pb.x, pb.y)));
+  }
+
+  // After the last chunk of a view; xx = |x|^2 (dense) or the row's token total (count view).
+  __device__ __forceinline__ void view_end(const ViewParam& vp, float xx) {
+    lnew = __fadd_rn(lnew, merge_view<false>(mxA, sA, mx, s, vp, xx, single, lone0));
+  }
+
+  // lw <- 2^(lw - M) over half h; returns the half's total (partial sums over t mod 4, then a fixed tree).
+  __device__ __forceinline__ float weights(int h, float M) {
+    const float2 nM2 = splat2(-M);
+    float2 qa = splat2(0.0f), qb = splat2(0.0f);
+    for (int i = h * HALF / 2; i < (h + 1) * HALF / 2; i += 2) {
+      const float2 wa = exp2w2<false>(fadd2(at(i), nM2)), wb = exp2w2<false>(fadd2(at(i + 1), nM2));
+      at(i) = wa;     qa = fadd2(qa, wa);
+      at(i + 1) = wb; qb = fadd2(qb, wb);
+    }
+    return __fadd_rn(__fadd_rn(qa.x, qa.y), __fadd_rn(qb.x, qb.y));
+  }
+
+  __device__ __forceinline__ int finish(float uf) {
+    float M0 = lnew, M1 = kMasked;
+    for (int i = 0; i < CAP / 2; ++i) { const float2 q = at(i); M0 = fmaxf(M0, q.x); M1 = fmaxf(M1, q.y); }
+    const float M = fmaxf(M0, M1);
+    if (!(M > -1.0e29f)) return t0;     // nothing has weight: stay (cf. multiview_gibbs.cpp:172-176)
+    const float HA = weights(0, M), HB = weights(1, M);
+    const float total = __fadd_rn(__fadd_rn(HA, HB), exp2m(__fadd_rn(lnew, -M)));
+    const float target = __fmul_rn(uf, total);
+    int cnt = 0;
+    for (int h = 0; h < 2; ++h) {
+      float cum = h ? HA : 0.0f;
+      for (int i = h * HALF / 2; i < (h + 1) * HALF / 2; ++i) {
+        const float2 q = at(i);
+        cum = __fadd_rn(cum, q.x);
+        cnt += (target < cum) ? 0 : 1;
+        cum = __fadd_rn(cum, q.y);
+        cnt += (target < cum) ? 0 : 1;
+      }
+    }
+    if (cnt < CAP) return cnt;
+    if (lnew > -1.0e29f) return kNewTable;
+    int last = t0;                      // rounding fall-through with no new-table mass: last live table
+    for (int i = 0; i < CAP / 2; ++i) {
+      const float2 q = at(i);
+      if (q.x > 1.0e-30f) last = 2 * i;
+      if (q.y > 1.0e-30f) last = 2 * i + 1;
+    }
+    return last;
+  }
+};
+
 }  // namespace mv

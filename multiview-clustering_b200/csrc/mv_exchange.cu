@@ -256,9 +256,11 @@ __global__ void __launch_bounds__(256, 3) k_reduce_x(const Ctx c, const int mode
 cudaError_t launch_reduce_x(const Ctx& c, int mode, bool delta, const XchgPeers& peers, unsigned char* recv_local, cudaStream_t s) {
   const XchgLayout L = xchg_layout(c);
   const int n_el = (int)L.n_units;
-  int nb = (n_el + 31) / 32;
-  if (nb > 148 * 3) nb = 148 * 3;              // every block of one launch is resident at once (3 per SM by the launch bounds): peers wait for each other's pushes
+  // every block of one launch, the `extra` ones included, is resident at once (3 per SM by the launch bounds): peers wait
+  // for each other's pushes
   const int extra = (mode == 1) ? c.world : 0;
+  int nb = (n_el + 31) / 32;
+  if (nb > 148 * 3 - extra) nb = 148 * 3 - extra;
   return launch_chain(k_reduce_x, dim3(nb + extra), dim3(256), 0, s, c.pdl != 0, c, mode, delta ? 1 : 0, nb, peers, recv_local, L);
 }
 

@@ -326,11 +326,59 @@ cudaError_t launch_stats(const Ctx& c, bool delta, cudaStream_t s) {
 // others read at their start (n_t, the sweep counter): the franchise CTA publishes those last, after every CTA has
 // announced that its reads are done (an arrival counter; all V + 1 CTAs are co-resident).
 constexpr int kFinThreads = 1024;
-constexpr int kMaxCap = 64;
 constexpr int kMaxWorld = 16;
 constexpr int kEppfSets = 4;             // (alpha, sigma) x (old, proposed): both Metropolis-Hastings steps of a level in one batch
 
+// A set of the slots (tables, dishes) of one level, one bit per slot in W 64-bit words; members are visited in ascending
+// order.
+template <int W>
+struct SlotSet {
+  unsigned long long w[W];
+  __device__ __forceinline__ void clear() {
+#pragma unroll
+    for (int i = 0; i < W; ++i) w[i] = 0ull;
+  }
+  __device__ __forceinline__ void set(int i) { w[i >> 6] |= 1ull << (i & 63); }
+  __device__ __forceinline__ int lowest() const {   // -1 if empty
+#pragma unroll
+    for (int i = 0; i < W; ++i) if (w[i]) return 64 * i + __ffsll((long long)w[i]) - 1;
+    return -1;
+  }
+  __device__ __forceinline__ int count() const {
+    int n = 0;
+#pragma unroll
+    for (int i = 0; i < W; ++i) n += __popcll(w[i]);
+    return n;
+  }
+  __device__ __forceinline__ int rank(int i) const {   // members below slot i
+    int n = 0;
+#pragma unroll
+    for (int j = 0; j < W; ++j) {
+      if (64 * j + 64 <= i) n += __popcll(w[j]);
+      else if (64 * j < i) n += __popcll(w[j] & ((1ull << (i - 64 * j)) - 1ull));
+    }
+    return n;
+  }
+  __device__ __forceinline__ SlotSet without_lowest() const {
+    SlotSet r = *this;
+#pragma unroll
+    for (int i = 0; i < W; ++i) if (r.w[i]) { r.w[i] &= r.w[i] - 1ull; break; }
+    return r;
+  }
+  template <class F>
+  __device__ __forceinline__ void for_each(F f) const {
+#pragma unroll
+    for (int i = 0; i < W; ++i)
+      for (unsigned long long m = w[i]; m; m &= m - 1ull) f(64 * i + __ffsll((long long)m) - 1);
+  }
+};
+
+// MAXCAP: the largest table capacity the instance serves (64: cap 32 / 64; 256: cap 128 / 256).
+template <int MAXCAP>
 struct FinShared {
+  static constexpr int kMaxCap = MAXCAP;
+  static constexpr int kWords = MAXCAP / 64;
+  static constexpr int kBlocks = MAXCAP / 32;  // 32-cluster blocks of the batched EPPF
   int32_t n_new[kMaxCap];                 // customers per table after this sweep
   int32_t n_start[kMaxCap];               // ... at sweep start
   int32_t free_slots[kMaxCap];
@@ -341,8 +389,8 @@ struct FinShared {
   int32_t cand_j[kMaxWorld * kMaxCap];
   int32_t cand_final[kMaxWorld * kMaxCap];
   int32_t ncand_total, nseat, nfree, err;
-  unsigned long long tmask[kMaxCap];      // bit t: table t serves dish k of this view (after births and deaths)
-  unsigned long long live;                // bit i: cluster i of this level has members (dishes: l_vk > 0; franchise: n_t > 0)
+  SlotSet<kWords> tmask[kMaxCap];         // bit t: table t serves dish k of this view (after births and deaths)
+  SlotSet<kWords> live;                   // bit i: cluster i of this level has members (dishes: l_vk > 0; franchise: n_t > 0)
   long long total;                        // items of this level (tables of the view; customers for the franchise)
   double s2t[kMaxCap];                    // sums of squared norms per table (working copy of S2t[v])
   double s2k[kMaxCap];                    //   and per dish
@@ -350,8 +398,8 @@ struct FinShared {
   int32_t table_of_dish[kMaxCap];         // at sweep start: lowest table slot serving dish k, -1 = none
   double s1sq[kMaxCap];                   // |S1k|^2, later |m_t|^2
   double sse[kMaxCap];                    // max(0, S2k - |S1k|^2 / n_k)     (multiview_hyper.cpp:191-193)
-  double termA[kEppfSets][4];             // scratch of the batched EPPF evaluations: per set, per 32-cluster block
-  double termB[kEppfSets][4];
+  double termA[kEppfSets][kBlocks];       // scratch of the batched EPPF evaluations: per set, per 32-cluster block
+  double termB[kEppfSets][kBlocks];
   double termC[kEppfSets][4];             // per set: lgamma(alpha + M), lgamma(alpha + 1), lgamma(1 - sigma)
   double eppf[kEppfSets];
   double s_alpha[kEppfSets], s_sigma[kEppfSets];
@@ -364,7 +412,8 @@ struct FinShared {
   double warm[2];                         // sink of the instruction-cache warm-up calls
 };
 
-constexpr int kFinSharedBytes = (int)((sizeof(FinShared) + 15) & ~(size_t)15);
+template <int MAXCAP>
+__host__ __device__ constexpr int fin_shared_bytes() { return (int)((sizeof(FinShared<MAXCAP>) + 15) & ~(size_t)15); }
 
 // (The out-of-line helpers below take scalars and pointers, never `const Ctx&`: taking the address of the kernel
 // parameter makes every thread copy the whole 1.5 KB struct into its local memory at kernel start.)
@@ -406,7 +455,8 @@ __device__ __forceinline__ void group_sync(int bar_id, int gthreads) {
 // thread per set adds the blocks in ascending order (the order of oracle/mv_oracle.c:eppf_core).
 // Called by ONE group of gthreads consecutive threads (gtid = index inside the group) synchronising on named barrier
 // bar_id; the rest of the CTA is busy with the dish statistics and the posterior means meanwhile.
-__device__ __noinline__ void eppf_batch(const int cap, const int32_t* counts, FinShared& S, const int gtid, const int gthreads,
+template <class FS>
+__device__ __noinline__ void eppf_batch(const int cap, const int32_t* counts, FS& S, const int gtid, const int gthreads,
                                         const int bar_id) {
   const int lane = gtid & 31, wid = gtid >> 5;
   group_sync(bar_id, gthreads);
@@ -421,7 +471,7 @@ __device__ __noinline__ void eppf_batch(const int cap, const int32_t* counts, Fi
         const double al = S.s_alpha[set], sg = S.s_sigma[set];
         const int cnt = counts[i];
         if (cnt > 0) {
-          const int r = __popcll(S.live & ((1ull << i) - 1ull));
+          const int r = S.live.rank(i);
           const double term = al + (double)r * sg;
           if (term <= 0.0) bad = true; else sa = fin_log(term);
         }
@@ -476,7 +526,8 @@ __device__ __noinline__ void eppf_batch(const int cap, const int32_t* counts, Fi
 // both candidates are evaluated up front — sets (a_old, s_old), (a_prop, s_old), (a_cur, s_prop), (a_prop, s_prop) in
 // ONE batch — so the two dependent steps cost one round of lgamma latencies instead of two.  Each EPPF value is the
 // same function of (alpha, sigma, counts) as in the sequential order, so the chain is unchanged.
-__device__ __forceinline__ void level_alpha_sigma(const int cap, const int32_t* counts, FinShared& S, const int gtid,
+template <class FS>
+__device__ __forceinline__ void level_alpha_sigma(const int cap, const int32_t* counts, FS& S, const int gtid,
                                                   const int gthreads, const int bar_id, const bool enabled) {
   double a_cur = 0.0, a_old = 0.0, a_prop = 0.0, s_old = 0.0, s_prop = 0.0;
   if (gtid == 0 && enabled) {
@@ -549,7 +600,8 @@ __device__ __noinline__ double log_f_dish_counts(const int32_t* __restrict__ rp,
 // The Philox numbers of one level's hyper step, by the calling warp's lanes 0..5: rn/lu[which], which = 0 tau, 1 alpha,
 // 2 sigma.  Stream positions are those the reference's sequential code would use: tau_v at v, (alpha_v, sigma_v) at
 // V + 2v, the franchise pair at 3V.  `first`..`last`: the range of `which` this call draws.
-__device__ __forceinline__ void draw_level_randoms(FinShared& S, uint64_t seed, uint32_t chain, uint32_t sweep, int V, int v,
+template <class FS>
+__device__ __forceinline__ void draw_level_randoms(FS& S, uint64_t seed, uint32_t chain, uint32_t sweep, int V, int v,
                                                    bool is_view, int first, int last, int lane) {
   const int which = first + (lane >> 1);
   if (which > last || lane >= 2 * (last - first + 1)) return;
@@ -558,9 +610,12 @@ __device__ __forceinline__ void draw_level_randoms(FinShared& S, uint64_t seed, 
   else S.rn[which] = dev_normal(seed, chain, sweep, idx);
 }
 
+template <int MAXCAP>
 __global__ void __launch_bounds__(kFinThreads, 1) k_finalize(const Ctx c, const int32_t flags, const int32_t s1_in_smem) {
   extern __shared__ __align__(16) unsigned char fin_smem[];
-  FinShared& S = *reinterpret_cast<FinShared*>(fin_smem);
+  using FS = FinShared<MAXCAP>;
+  using Set = SlotSet<FS::kWords>;
+  FS& S = *reinterpret_cast<FS*>(fin_smem);
   // Programmatic dependent launch: the next sweep's draw kernel may be scheduled now (its CTAs set themselves up and
   // start streaming features on the idle SMs; they wait for this grid's completion before they touch its results).
   pdl_trigger();
@@ -576,7 +631,7 @@ __global__ void __launch_bounds__(kFinThreads, 1) k_finalize(const Ctx c, const 
   // (mvg_sweep / mvg_sync report it; csrc/mv_exchange.cu).
   // The per-table sums of this view, S1t [cap][D], live in shared memory behind FinShared when they fit (32 KB at C3):
   // the dish statistics and the posterior means are then built from on-chip data instead of global round trips.
-  double* const S1t = s1_in_smem ? reinterpret_cast<double*>(fin_smem + kFinSharedBytes) : (c.S1t + (size_t)cap * doff);
+  double* const S1t = s1_in_smem ? reinterpret_cast<double*>(fin_smem + fin_shared_bytes<MAXCAP>()) : (c.S1t + (size_t)cap * doff);
   const uint32_t sweep = *reinterpret_cast<volatile uint32_t*>(c.sweep);
   double& alpha_l = S.hyp[0];                       // alpha_v / alpha_global
   double& sigma_l = S.hyp[1];                       // sigma_v / sigma_global
@@ -657,7 +712,7 @@ __global__ void __launch_bounds__(kFinThreads, 1) k_finalize(const Ctx c, const 
       int n = 0;
       for (int g = 0; g < c.world; ++g) {
         const int nc = pkt_i32(c, g, c.pkt.off_hdr)[0];
-        for (int j = 0; j < nc && n < kMaxWorld * kMaxCap; ++j) { S.cand_g[n] = g; S.cand_j[n] = j; ++n; }
+        for (int j = 0; j < nc && n < kMaxWorld * MAXCAP; ++j) { S.cand_g[n] = g; S.cand_j[n] = j; ++n; }
       }
       S.ncand_total = n;
       S.nseat = n < nf ? n : nf;
@@ -811,8 +866,9 @@ __global__ void __launch_bounds__(kFinThreads, 1) k_finalize(const Ctx c, const 
       if (tot != (long long)c.n_global) atomicOr(&S.err, 4);
     }
     if (tid == 0) {
-      unsigned long long m = 0ull;
-      for (int i = 0; i < cap; ++i) if (S.n_new[i] > 0) m |= 1ull << i;
+      Set m;
+      m.clear();
+      for (int i = 0; i < cap; ++i) if (S.n_new[i] > 0) m.set(i);
       S.live = m;
       S.total = (long long)c.n_global;
     }
@@ -884,21 +940,21 @@ __global__ void __launch_bounds__(kFinThreads, 1) k_finalize(const Ctx c, const 
     // one warp per dish k: which tables serve it (ballots over the table slots), how many customers they hold
     const int lane = tid & 31, wid = tid >> 5;
     for (int k = wid; k < cap; k += kFinThreads / 32) {
-      unsigned long long m = 0ull;
+      Set m;
+      m.clear();
       int n = 0;
       double s2 = 0.0;
       for (int base = 0; base < cap; base += 32) {
         const int t = base + lane;
         const bool mine = (t < cap) && (S.dish[t] == k);
-        m |= (unsigned long long)__ballot_sync(0xffffffffu, mine) << base;
+        m.w[base >> 6] |= (unsigned long long)__ballot_sync(0xffffffffu, mine) << (base & 63);
       }
       if (lane == 0) {
-        for (unsigned long long r = m; r; r &= r - 1ull) {         // ascending table order (usually one table)
-          const int t = __ffsll((long long)r) - 1;
+        m.for_each([&](int t) {                                      // ascending table order (usually one table)
           n += S.n_new[t];
           s2 += S.s2t[t];
-        }
-        const int l = __popcll(m);
+        });
+        const int l = m.count();
         S.l_live[k] = l;
         S.n_vk[k] = n;
         S.s2k[k] = s2;
@@ -923,9 +979,10 @@ __global__ void __launch_bounds__(kFinThreads, 1) k_finalize(const Ctx c, const 
   if (tid >= kGroupThreads) {
     const int gtid = tid - kGroupThreads;
     if (gtid == 0) {                            // live mask and item total of this level
-      unsigned long long m = 0ull;
+      Set m;
+      m.clear();
       long long tot = 0;
-      for (int i = 0; i < cap; ++i) { if (S.l_live[i] > 0) m |= 1ull << i; tot += S.l_live[i]; }
+      for (int i = 0; i < cap; ++i) { if (S.l_live[i] > 0) m.set(i); tot += S.l_live[i]; }
       S.live = m;
       S.total = tot;
     }
@@ -946,13 +1003,13 @@ __global__ void __launch_bounds__(kFinThreads, 1) k_finalize(const Ctx c, const 
       } else {
         for (int k = wid; k < cap; k += kStatWarps) {
           double* S1k_vk = c.S1k + (size_t)cap * doff + (size_t)k * D;
-          const unsigned long long mask = S.tmask[k];
-          const int t1 = __ffsll((long long)mask) - 1;             // usually the only table of the dish
-          const unsigned long long more = mask & (mask - 1ull);
+          const Set mask = S.tmask[k];
+          const int t1 = mask.lowest();                              // usually the only table of the dish
+          const Set more = mask.without_lowest();
           double q = 0.0;
           for (int dd = lane; dd < D; dd += 32) {
             double sum = (t1 >= 0) ? S1t[t1 * D + dd] : 0.0;
-            for (unsigned long long m = more; m; m &= m - 1ull) sum += S1t[(__ffsll((long long)m) - 1) * D + dd];
+            more.for_each([&](int t) { sum += S1t[t * D + dd]; });
             S1k_vk[dd] = sum;
             q += sum * sum;
           }
@@ -1034,13 +1091,15 @@ __global__ void __launch_bounds__(kFinThreads, 1) k_finalize(const Ctx c, const 
           const double nk = (double)S.n_vk[k];
           A_f = (float)(kLog2e * ((tau_l + nk) / (2.0 * tau_l * (tau_l + nk + 1.0))));
         }
-        const unsigned long long mask = (k >= 0) ? S.tmask[k] : 0ull;
-        const int t1 = __ffsll((long long)mask) - 1;
-        const unsigned long long more = mask & (mask - 1ull);
+        Set mask;
+        if (k >= 0) mask = S.tmask[k];
+        else mask.clear();
+        const int t1 = mask.lowest();
+        const Set more = mask.without_lowest();
         double mm = 0.0;
         for (int dd = lane; dd < D; dd += 32) {
           double s1 = (t1 >= 0) ? S1t[t1 * D + dd] : 0.0;
-          for (unsigned long long m = more; m; m &= m - 1ull) s1 += S1t[(__ffsll((long long)m) - 1) * D + dd];
+          more.for_each([&](int t) { s1 += S1t[t * D + dd]; });
           const float m = (float)(s1 * rden);
           c.mean[off + dd] = m;
           if (c.mean_hi) {
@@ -1077,7 +1136,7 @@ __global__ void __launch_bounds__(kFinThreads, 1) k_finalize(const Ctx c, const 
       // total of the dish for the leave-one-out term of the kernel
       q.A = 0.5f; q.C = 0.f; q.A1 = 0.f;
       q.C1 = (float)((double)c.vocab[v] * (double)c.count_beta + S.s2k[k]);
-      const bool rep = (__ffsll((long long)S.tmask[k]) - 1 == t);
+      const bool rep = (S.tmask[k].lowest() == t);
       const double w = (double)S.l_live[k] - sigma_l, w1 = w - 1.0;
       q.W = (rep && w > 0.0) ? (float)fin_log2(w) : kMasked;
       q.W1 = (rep && w1 > 0.0) ? (float)fin_log2(w1) : kMasked;
@@ -1097,7 +1156,7 @@ __global__ void __launch_bounds__(kFinThreads, 1) k_finalize(const Ctx c, const 
       } else {
         q.A1 = 0.f; q.C1 = kMasked;
       }
-      const bool rep = (__ffsll((long long)S.tmask[k]) - 1 == t);      // lowest table of its dish
+      const bool rep = (S.tmask[k].lowest() == t);      // lowest table of its dish
       const double w = (double)S.l_live[k] - sigma_l, w1 = w - 1.0;
       q.W = (rep && w > 0.0) ? (float)fin_log2(w) : kMasked;
       q.W1 = (rep && w1 > 0.0) ? (float)fin_log2(w1) : kMasked;
@@ -1105,7 +1164,7 @@ __global__ void __launch_bounds__(kFinThreads, 1) k_finalize(const Ctx c, const 
       q.lone = (S.l_live[k] == 1);
     }
     c.tparam[i] = q;
-    c.tsame[i] = (k >= 0) ? S.tmask[k] : 0ull;
+    if constexpr (MAXCAP <= 64) c.tsame[i] = (k >= 0) ? S.tmask[k].w[0] : 0ull;   // read by the tensor-core engine (cap 64) only
   }
   if (tid == 12 * 32) {
     const double tau = tau_l;
@@ -1131,16 +1190,22 @@ __global__ void __launch_bounds__(kFinThreads, 1) k_finalize(const Ctx c, const 
   if (tid == 0) kclock_end(c.kclock + kClockFinalize, gridDim.x);
 }
 
-cudaError_t launch_finalize(const Ctx& c, int32_t flags, cudaStream_t s) {
-  if (c.cap > kMaxCap || c.world > kMaxWorld || c.V > kMaxViews) return cudaErrorInvalidValue;
+template <int MAXCAP>
+static cudaError_t launch_finalize_cap(const Ctx& c, int32_t flags, cudaStream_t s) {
   int dmax = 0;
   for (int v = 0; v < c.V; ++v) dmax = c.D[v] > dmax ? c.D[v] : dmax;
   const size_t s1_bytes = sizeof(double) * (size_t)c.cap * dmax;
-  const int s1_in_smem = (kFinSharedBytes + s1_bytes <= (size_t)227 * 1024) ? 1 : 0;
-  const int smem = kFinSharedBytes + (s1_in_smem ? (int)s1_bytes : 0);
-  cudaError_t e = cudaFuncSetAttribute(k_finalize, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+  const int s1_in_smem = (fin_shared_bytes<MAXCAP>() + s1_bytes <= (size_t)227 * 1024) ? 1 : 0;
+  const int smem = fin_shared_bytes<MAXCAP>() + (s1_in_smem ? (int)s1_bytes : 0);
+  cudaError_t e = cudaFuncSetAttribute(k_finalize<MAXCAP>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
   if (e != cudaSuccess) return e;
-  return launch_chain(k_finalize, dim3(c.V + 1), dim3(kFinThreads), (size_t)smem, s, c.pdl != 0, c, flags, (int32_t)s1_in_smem);
+  return launch_chain(k_finalize<MAXCAP>, dim3(c.V + 1), dim3(kFinThreads), (size_t)smem, s, c.pdl != 0, c, flags, (int32_t)s1_in_smem);
+}
+
+// The cap-64 instance keeps the shared-memory footprint of the small capacities; 128 and 256 take the wide one.
+cudaError_t launch_finalize(const Ctx& c, int32_t flags, cudaStream_t s) {
+  if (c.cap > 256 || c.world > kMaxWorld || c.V > kMaxViews) return cudaErrorInvalidValue;
+  return c.cap <= 64 ? launch_finalize_cap<64>(c, flags, s) : launch_finalize_cap<256>(c, flags, s);
 }
 
 // =============================================================================================

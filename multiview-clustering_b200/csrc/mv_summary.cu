@@ -22,7 +22,7 @@ __global__ void k_labels(const Ctx c, int32_t* __restrict__ out) {
 
 // view < 0: tables; else dishes of that view.  One thread per 4 consecutive j of a row i.
 __global__ void __launch_bounds__(256) k_cocluster(const Ctx c, const int view, uint32_t* __restrict__ counts) {
-  __shared__ int32_t s_dish[64];
+  __shared__ int32_t s_dish[256];                 // cap <= 256 = blockDim.x (mvg_create)
   if (threadIdx.x < c.cap) s_dish[threadIdx.x] = (view < 0) ? (int32_t)threadIdx.x : c.dish_of[view * c.cap + threadIdx.x];
   __syncthreads();
   const int n = c.n_rows;

@@ -52,7 +52,7 @@ extern std::vector<double> saved_sigma_global;
 // ---- additions (not in the reference): the device chain behind the mirror -------------------------
 struct mvg_handle;
 namespace mvhost {
-extern int table_capacity;          // table / dish slots per view on the device (32 or 64; default 64)
+extern int table_capacity;          // table / dish slots per view on the device (32, 64, 128 or 256; default 64)
 extern unsigned long long seed;     // Philox key (set.seed(1999) of New_Simulation.R:12 by default)
 extern int engine;                  // MVG_ENGINE_* (0 = automatic)
 extern std::vector<int> view_dim;   // D_v; empty = all 1 (the reference's scalar views)
