@@ -138,6 +138,17 @@ int mvg_upload_view_csr(mvg_handle* h, int32_t v, const int32_t* rowptr, const i
                         int64_t nnz, int32_t vocab);
 /* Symmetric Dirichlet pseudo-count beta of the count views (default 0.5); before the first state call. */
 int mvg_set_count_beta(mvg_handle* h, double beta);
+/* The likelihood of every count view of the handle (DESIGN.md §4.5):
+ *   MVG_COUNT_PLUGIN (default)  the plug-in multinomial above;
+ *   MVG_COUNT_DIRMULT           the exact collapsed conditional of a Dirichlet-multinomial mixture,
+ *       log f_vk(x) = sum_w [lnΓ(beta + c_kw + x_w) - lnΓ(beta + c_kw)] - [lnΓ(W beta + C_k + n) - lnΓ(W beta + C_k)],
+ *       n = sum_w x_w (c_kw, C_k without the row for its own dish; c = C = 0 for a new dish), so that the sweep samples
+ *       the posterior of that model.  Counts must be non-negative integers (mvg_upload_view_csr checks it) and rows
+ *       shorter than 2^24 tokens.
+ * Like mvg_set_count_beta: before the first state call (afterwards MVG_ESTATE); another value is MVG_EINVAL.  A handle
+ * that never calls it runs the plug-in kernels unchanged. */
+enum { MVG_COUNT_PLUGIN = 0, MVG_COUNT_DIRMULT = 1 };
+int mvg_set_count_likelihood(mvg_handle* h, int32_t model);
 
 /* ---- state ----------------------------------------------------------------------------- */
 int mvg_init_state_reference(mvg_handle* h);
@@ -232,15 +243,23 @@ typedef struct mvg_params_host {
 } mvg_params_host;
 int mvg_get_params(mvg_handle* h, const mvg_params_host* out);
 /* With debug_export: per-row stage-A outputs of the LAST sweep: acc [n_rows][V][cap] dot products
- * x.m and xx [n_rows][V] squared norms, plus the raw draw (before births are seated) [n_rows]. */
+ * x.m and xx [n_rows][V] squared norms, plus the raw draw (before births are seated) [n_rows].  A count view: acc is
+ * log2 f under each table's dish and xx what the new-dish term read, the token total (plug-in) or -log2 f_new
+ * (MVG_COUNT_DIRMULT). */
 int mvg_get_debug_rows(mvg_handle* h, float* acc, float* xx, int32_t* choice);
 /* Tensor-core engines, with debug_export: acc above holds the dot products with the PRE-SCALED means b = 2 A m (the data
  * term of log2 f), and lnew [n_rows] the log2 weight of a new table as the kernel evaluated it (MUFU log-sum-exp: a float
  * statistic inside the stated tolerance; the CPU mirror checks it and draws from it). */
 int mvg_get_debug_lnew(mvg_handle* h, float* lnew);
 /* Count view v: the tables of the NEXT sweep, host [vocab][cap] each (NULL skips): log2 theta of the dish each
- * table slot serves, that dish's word counts, and the word counts per table slot. */
+ * table slot serves, that dish's word counts, and the word counts per table slot.  Under MVG_COUNT_DIRMULT the first
+ * output holds log2(beta + c) of the dish's count c instead of log2 theta. */
 int mvg_get_count_tables(mvg_handle* h, int32_t v, float* log2_theta, int32_t* dish_counts, int32_t* table_counts);
+/* MVG_COUNT_DIRMULT, count view v: *n_max = its longest row in tokens (any model; den may be NULL), and den (host
+ * [n_max+1][cap], length-major) the denominator table of the NEXT sweep, den[n][t] = sum_{j<n} log2(W beta + C_k + j)
+ * of the dish k table slot t serves (0 for a free slot), formed in FP64 and rounded once.  den under the plug-in model:
+ * MVG_ESTATE. */
+int mvg_get_count_den(mvg_handle* h, int32_t v, float* den, int32_t* n_max);
 /* With debug_export, count views: loo [n_rows][V] leave-one-out log2 f of every row under its own dish (LAST sweep). */
 int mvg_get_debug_loo(mvg_handle* h, float* loo);
 /* Births of the LAST sweep: rows (global index) seated at new tables in order, and the
@@ -269,7 +288,9 @@ void* mvg_stream(mvg_handle* h);
 /* Joint log marginal likelihood of the data given the current partition: the sum over live dishes of the
  * reference's log p(y_S) (multiview_utils.cpp:316-320, per coordinate).  This is what the reference's
  * declared-but-never-defined compute_log_likelihood() (multiview_gibbs.h:13) / saved_loglik
- * (multiview_state.h:38) would hold.  per_view: [V] or NULL. */
+ * (multiview_state.h:38) would hold.  per_view: [V] or NULL.  A count view under MVG_COUNT_DIRMULT contributes the
+ * collapsed marginal of the partition up to the multinomial coefficients (which do not depend on it):
+ *   sum over live dishes k of  sum_w [lnΓ(beta + c_kw) - lnΓ(beta)] - lnΓ(W beta + C_k) + lnΓ(W beta). */
 int mvg_log_likelihood(mvg_handle* h, double* total, double* per_view);
 /* Cluster of every customer in every view, dish_of[v][table_of[i]]: get_final_clusters of
  * New_Simulation.R:135-149.  labels: host [V][n_rows]. */

@@ -259,6 +259,24 @@ int rebuild_pipeline(mvg_handle* h, int32_t flags, cudaEvent_t* marks /* 4 event
   return MVG_OK;
 }
 
+// MVG_COUNT_DIRMULT, at the first state call (beta and the views are frozen from then on): the denominator tables and the
+// per-row new-dish terms of every count view.  A no-op for the plug-in model.
+int prepare_count_model(mvg_handle* h) {
+  Ctx& c = h->c;
+  if (h->state_ready || !c.count_model || !c.n_count_views) return MVG_OK;
+  for (int v = 0; v < c.V; ++v) {
+    if (!c.kind[v]) continue;
+    if (c.cnt_nmax[v] >= (1 << 24))
+      return fail(h, MVG_EINVAL, "the Dirichlet-multinomial count likelihood needs rows of fewer than 2^24 tokens");
+    int rc;
+    if (!c.cnt_den[v] && (rc = dev_alloc(h, &c.cnt_den[v], (size_t)(c.cnt_nmax[v] + 1) * c.cap)) != MVG_OK) return rc;
+    if (!c.cnt_q[v] && (rc = dev_alloc(h, &c.cnt_q[v], (size_t)c.n_rows)) != MVG_OK) return rc;
+  }
+  MVG_CUDA(h, launch_counts_newdish(c, h->stream));
+  h->launches += 1;
+  return MVG_OK;
+}
+
 int launch_draw(mvg_handle* h, bool programmatic = false) {
   if (h->engine == MVG_ENGINE_TCGEN05 || h->engine == MVG_ENGINE_TCGEN05_FAST)
     MVG_CUDA(h, launch_draw_tc(h->c, h->tc_maps, h->engine == MVG_ENGINE_TCGEN05_FAST, programmatic, h->stream));
@@ -463,6 +481,15 @@ int mvg_set_count_beta(mvg_handle* h, double beta) {
   return MVG_OK;
 }
 
+int mvg_set_count_likelihood(mvg_handle* h, int32_t model) {
+  if (!h) return MVG_EINVAL;
+  if (model != MVG_COUNT_PLUGIN && model != MVG_COUNT_DIRMULT) return fail(h, MVG_EINVAL, "unknown count likelihood model");
+  if (h->state_ready) return fail(h, MVG_ESTATE, "the count likelihood is frozen after the first state call");
+  // (count values are checked to be non-negative integers at upload, whatever the model)
+  h->c.count_model = model;
+  return MVG_OK;
+}
+
 int mvg_upload_view_csr(mvg_handle* h, int32_t v, const int32_t* rowptr, const int32_t* col, const float* val,
                         int64_t nnz, int32_t vocab) {
   if (!h) return MVG_EINVAL;
@@ -479,6 +506,13 @@ int mvg_upload_view_csr(mvg_handle* h, int32_t v, const int32_t* rowptr, const i
     if (!(val[j] >= 0.0f) || val[j] > 16777216.0f || val[j] != (float)(int32_t)val[j])
       return fail(h, MVG_EINVAL, "count views hold non-negative integer counts (< 2^24)");
   }
+  int64_t n_max = 0;                 // the longest row in tokens: rows of the Dirichlet-multinomial denominator table
+  for (int64_t i = 0; i < n; ++i) {
+    int64_t tok = 0;
+    for (int32_t j = rowptr[i]; j < rowptr[i + 1]; ++j) tok += (int64_t)val[j];
+    n_max = tok > n_max ? tok : n_max;
+  }
+  if (n_max > 0x7fffffffLL) n_max = 0x7fffffffLL;   // (refused by the Dirichlet-multinomial model, prepare_count_model)
   MVG_CUDA(h, cudaSetDevice(h->cfg.device));
   for (void*& p : h->csr_owned[v]) { if (p) cudaFree(p); p = nullptr; }
   if (h->view_owned[v]) { cudaFree(h->view_owned[v]); h->view_owned[v] = nullptr; }
@@ -502,6 +536,7 @@ int mvg_upload_view_csr(mvg_handle* h, int32_t v, const int32_t* rowptr, const i
   Ctx& c = h->c;
   c.kind[v] = 1;
   c.vocab[v] = vocab;
+  c.cnt_nmax[v] = (int32_t)n_max;
   c.row_order[v] = static_cast<const int32_t*>(h->csr_owned[v][3]);
   c.D[v] = 0;
   c.x[v] = nullptr;
@@ -527,6 +562,20 @@ int mvg_get_count_tables(mvg_handle* h, int32_t v, float* log2_theta, int32_t* d
   return MVG_OK;
 }
 
+int mvg_get_count_den(mvg_handle* h, int32_t v, float* den, int32_t* n_max) {
+  if (!h) return MVG_EINVAL;
+  if (v < 0 || v >= h->c.V || !h->c.kind[v]) return fail(h, MVG_EINVAL, "not a count view");
+  if (n_max) *n_max = h->c.cnt_nmax[v];
+  if (!den) return MVG_OK;
+  if (!h->state_ready) return fail(h, MVG_ESTATE, "no state yet");
+  if (!h->c.count_model) return fail(h, MVG_ESTATE, "the plug-in count likelihood has no denominator table");
+  MVG_CUDA(h, cudaSetDevice(h->cfg.device));
+  const size_t cells = (size_t)(h->c.cnt_nmax[v] + 1) * h->c.cap;
+  MVG_CUDA(h, cudaMemcpyAsync(den, h->c.cnt_den[v], sizeof(float) * cells, cudaMemcpyDeviceToHost, h->stream));
+  MVG_CUDA(h, cudaStreamSynchronize(h->stream));
+  return MVG_OK;
+}
+
 int mvg_get_debug_loo(mvg_handle* h, float* loo) {
   if (!h || !loo) return MVG_EINVAL;
   if (!h->c.dbg_loo) return fail(h, MVG_ESTATE, "debug_export was not enabled");
@@ -542,6 +591,7 @@ int mvg_init_state_reference(mvg_handle* h) {
   h->counts_valid = false;           // the seating is replaced from outside: the word counts of count views start from zero
   MVG_CUDA(h, cudaSetDevice(h->cfg.device));
   int rc = ensure_layout(h);
+  if (rc == MVG_OK) rc = prepare_count_model(h);
   if (rc != MVG_OK) return rc;
   if (h->c.cap < 4) return fail(h, MVG_EINVAL, "reference initialisation needs cap >= 4");
   const uint32_t zero = 0;
@@ -561,6 +611,7 @@ int mvg_set_state(mvg_handle* h, const mvg_state_host* s) {
   h->counts_valid = false;           // the seating is replaced from outside: the word counts of count views start from zero
   MVG_CUDA(h, cudaSetDevice(h->cfg.device));
   int rc = ensure_layout(h);
+  if (rc == MVG_OK) rc = prepare_count_model(h);
   if (rc != MVG_OK) return rc;
   const Ctx& c = h->c;
   if (!s->table_of || !s->dish_of || !s->alpha_v || !s->sigma_v || !s->tau_v || !s->alpha_sigma_global)

@@ -12,9 +12,16 @@
 //                     bit-exact)
 //   k_counts_tables   per (word, table slot): the counts of the DISH the slot serves (sum over the slots of that
 //                     dish, ascending) and log2 theta, the table the likelihood kernel reads feature-major
+//
+// MVG_COUNT_DIRMULT (opt-in, DESIGN.md §4.5) replaces the plug-in by the exact collapsed conditional of a
+// Dirichlet-multinomial mixture, log f_vk(x) = sum_w [lnΓ(beta + c_kw + x_w) - lnΓ(beta + c_kw)]
+// - [lnΓ(W beta + C_k + n) - lnΓ(W beta + C_k)], n = |x| (oracle/mv_oracle_dm.c:mvod_counts_log_f_vk): the same
+// scatter and tables with log2(beta + c) cells plus a per-slot denominator table, and k_counts_loglik_dm for stage A.
 #include "mv_ctx.h"
 
 namespace mv {
+
+constexpr double kLog2eD = 1.4426950408889634074;
 
 __global__ void k_rowtotals(const int32_t* __restrict__ rowptr, const float* __restrict__ val, float* __restrict__ out, int n) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -56,7 +63,8 @@ __global__ void k_counts_scatter(const Ctx c, const int delta) {
 }
 
 // MAXCAP: 64 (one mask word per slot) or 256; cap is a power of two <= MAXCAP.
-template <int MAXCAP>
+// DM (MVG_COUNT_DIRMULT): the cell is log2(beta + cd) instead of log2 theta, and the denominator table follows the cells.
+template <int MAXCAP, bool DM>
 __global__ void k_counts_tables(const Ctx c, const int log2cap) {
   constexpr int kWords = MAXCAP / 64;
   const int v = nth_count_view(c, blockIdx.y);
@@ -70,7 +78,8 @@ __global__ void k_counts_tables(const Ctx c, const int log2cap) {
     s_dish[threadIdx.x] = k;
     // S2k of a count view holds the token total of the dish (an exact integer)
     s_den[threadIdx.x] = (k >= 0) ? (double)c.vocab[v] * (double)c.count_beta + c.S2k[v * cap + k] : 1.0;
-    s_l2zero[threadIdx.x] = (float)log2(((double)c.count_beta + 0.0) / s_den[threadIdx.x]);   // the cell expression at cd = 0
+    if constexpr (DM) s_l2zero[threadIdx.x] = (float)log2((double)c.count_beta);
+    else s_l2zero[threadIdx.x] = (float)log2(((double)c.count_beta + 0.0) / s_den[threadIdx.x]);   // the cell expression at cd = 0
   }
   __syncthreads();
   if (threadIdx.x < cap) {
@@ -100,11 +109,40 @@ __global__ void k_counts_tables(const Ctx c, const int log2cap) {
 #pragma unroll
       for (int wi = 0; wi < kWords; ++wi)
         for (unsigned long long m = s_mask[t][wi]; m; m &= m - 1ull) cd += row[64 * wi + __ffsll((long long)m) - 1];
-      l2 = (cd == 0) ? s_l2zero[t] : (float)log2(((double)c.count_beta + (double)cd) / s_den[t]);
+      if constexpr (DM) l2 = (cd == 0) ? s_l2zero[t] : (float)log2((double)c.count_beta + (double)cd);
+      else l2 = (cd == 0) ? s_l2zero[t] : (float)log2(((double)c.count_beta + (double)cd) / s_den[t]);
     }
     c.cnt_d[v][e] = cd;
     c.l2t[v][e] = l2;
   }
+  if constexpr (DM) {
+    // den[n][t] = sum_{j<n} log2(W beta + C_k + j) for every row length n <= n_max, in FP64 (lgamma_diff), rounded once
+    const size_t dcells = (size_t)(c.cnt_nmax[v] + 1) * cap;
+    for (size_t e = (size_t)blockIdx.x * blockDim.x + threadIdx.x; e < dcells; e += (size_t)gridDim.x * blockDim.x) {
+      const int t = (int)(e & (size_t)(cap - 1));
+      const int n = (int)(e >> log2cap);
+      c.cnt_den[v][e] = (s_dish[t] >= 0) ? (float)(kLog2eD * lgamma_diff(s_den[t], n)) : 0.0f;
+    }
+  }
+}
+
+// MVG_COUNT_DIRMULT, once per chain (beta is frozen at the first state call and the rows never change):
+// q[i] = -log2 f_new(x_i) = -(sum_w lnΓ(beta + x_w) - lnΓ(beta)  -  [lnΓ(W beta + n) - lnΓ(W beta)]) / ln 2, FP64, ascending
+// over the row's nonzeros, rounded once.  The draw's new-dish term reads it where the plug-in reads the token total.
+__global__ void k_counts_newdish(const Ctx c) {
+  const int v = nth_count_view(c, blockIdx.y);
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= c.n_rows) return;
+  const double beta = (double)c.count_beta;
+  double lf = 0.0;
+  int n = 0;
+  for (int j = c.rowptr[v][i]; j < c.rowptr[v][i + 1]; ++j) {
+    const int x = (int)c.val[v][j];
+    lf += lgamma_diff(beta, x);
+    n += x;
+  }
+  lf -= lgamma_diff((double)c.vocab[v] * beta, n);
+  c.cnt_q[v][i] = (float)(-kLog2eD * lf);
 }
 
 // Stage A of a count view: log2 f of every row under every table slot's dish, acc[i][t] = sum_j x_j l2t[col_j][t], and
@@ -189,11 +227,124 @@ __global__ void __launch_bounds__(512) k_counts_loglik(const Ctx c) {
   }
 }
 
+// Stage A of a count view under MVG_COUNT_DIRMULT: the same warp per row, row_order dealing and broadcast of the
+// nonzeros as k_counts_loglik.  Per table t (l2c = log2(beta + c) of the dish's count c of word w, from k_counts_tables):
+//   s_j = l2c[w_j][t], then for x_j > 1: s_j += log2m(beta + c + i), i = 1 .. x_j - 1;   a += s_j   (ascending j, x_j > 0)
+//   a -= den[n][t]                                                                          (n = |x|, the row's tokens)
+// The row's own dish, leave-one-out (counts c - x, total C_k - n, so the denominator is not the table's):
+//   term_j = sum_{i < x_j} log2m(beta + (c - x_j) + i);   loo += term_j   (ascending j)
+//   loo -= ld,  ld = sum_{j<n} log2m(W beta + C_k - n + j): lane l sums j = l, l+32, ... ascending, then an xor butterfly
+//   (offsets 16, 8, 4, 2, 1; IEEE addition commutes, so every lane holds the same value).
+// Every operation is one oracle/mv_oracle_dm.c:mvod_stageA_counts_f32 repeats bit for bit.
+template <int CAP>
+__global__ void __launch_bounds__(512) k_counts_loglik_dm(const Ctx c) {
+  const int v = nth_count_view(c, blockIdx.y);
+  constexpr int PER = CAP / 32;
+  const int lane = threadIdx.x & 31;
+  const int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, nwarps = (gridDim.x * blockDim.x) >> 5;
+  const int32_t* __restrict__ rp = c.rowptr[v];
+  const int32_t* __restrict__ colv = c.col[v];
+  const float* __restrict__ valv = c.val[v];
+  const float* __restrict__ l2c = c.l2t[v];
+  const int32_t* __restrict__ cdt = c.cnt_d[v];
+  const float* __restrict__ den = c.cnt_den[v];
+  const TableParam* __restrict__ tp = c.tparam + v * CAP;
+  const int32_t* __restrict__ order = c.row_order[v];
+  const float beta = c.count_beta;
+  constexpr int kFlight = 8;
+  for (int ri = warp; ri < c.n_rows; ri += nwarps) {
+    const int row = order ? __ldg(order + ri) : ri;
+    const int j0 = rp[row], j1 = rp[row + 1];
+    const int t0 = c.table_cur[row];
+    const float nf = c.xx[(size_t)v * c.xx_stride + row];
+    const int n = (int)nf;
+    const float lbase = __fadd_rn(tp[t0].C1, -nf);          // TableParam::C1 of a count view: W beta + C_k
+    float ld = 0.0f;
+    for (int j = lane; j < n; j += 32) ld = __fadd_rn(ld, log2m(__fadd_rn(lbase, (float)j)));
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) ld = __fadd_rn(ld, __shfl_xor_sync(0xffffffffu, ld, o));
+    float a[PER];
+#pragma unroll
+    for (int q = 0; q < PER; ++q) a[q] = 0.0f;
+    float aloo = 0.0f;
+    for (int jb = j0; jb < j1; jb += 32) {
+      const int j = jb + lane;
+      const bool has = j < j1;
+      const float xv_l = has ? __ldg(valv + j) : 0.0f;
+      const int col_l = has ? __ldg(colv + j) : 0;
+      float term_l = 0.0f;
+      if (has) {
+        const int xi = (int)xv_l;
+        const float b0 = __fadd_rn(beta, (float)(__ldg(cdt + (size_t)col_l * CAP + t0) - xi));
+        for (int i = 0; i < xi; ++i) term_l = __fadd_rn(term_l, log2m(__fadd_rn(b0, (float)i)));
+      }
+      const int cnt = min(32, j1 - jb);
+      for (int u0 = 0; u0 < cnt; u0 += kFlight) {
+        float lv[kFlight][PER], xs[kFlight];
+        int cls[kFlight];
+#pragma unroll
+        for (int u = 0; u < kFlight; ++u) {
+          const int src = min(u0 + u, cnt - 1);
+          cls[u] = __shfl_sync(0xffffffffu, col_l, src);
+          xs[u] = __shfl_sync(0xffffffffu, xv_l, src);
+          const float* p = l2c + (size_t)cls[u] * CAP + lane * PER;
+          if constexpr (PER >= 4) {
+#pragma unroll
+            for (int q = 0; q < PER; q += 4) {
+              const float4 t4 = __ldg(reinterpret_cast<const float4*>(p) + q / 4);
+              lv[u][q] = t4.x; lv[u][q + 1] = t4.y; lv[u][q + 2] = t4.z; lv[u][q + 3] = t4.w;
+            }
+          } else if constexpr (PER == 2) {
+            const float2 t2 = __ldg(reinterpret_cast<const float2*>(p)); lv[u][0] = t2.x; lv[u][PER - 1] = t2.y;
+          } else {
+            lv[u][0] = __ldg(p);
+          }
+        }
+#pragma unroll
+        for (int u = 0; u < kFlight; ++u) {
+          if (u0 + u < cnt) {                                  // warp-uniform
+            if (xs[u] > 1.0f) {                                // a repeated word (warp-uniform): the rising factorial
+              const int xi = (int)xs[u];
+              const int32_t* cp = cdt + (size_t)cls[u] * CAP + lane * PER;
+#pragma unroll
+              for (int q = 0; q < PER; ++q) {
+                const float bc = __fadd_rn(beta, (float)__ldg(cp + q));
+                float sq = lv[u][q];
+                for (int i = 1; i < xi; ++i) sq = __fadd_rn(sq, log2m(__fadd_rn(bc, (float)i)));
+                a[q] = __fadd_rn(a[q], sq);
+              }
+            } else if (xs[u] > 0.0f) {                         // (a stored zero count adds nothing)
+#pragma unroll
+              for (int q = 0; q < PER; ++q) a[q] = __fadd_rn(a[q], lv[u][q]);
+            }
+            aloo = __fadd_rn(aloo, __shfl_sync(0xffffffffu, term_l, u0 + u));
+          }
+        }
+      }
+    }
+    const float* dn = den + (size_t)n * CAP + lane * PER;
+    float* dst = c.cnt_acc[v] + (size_t)row * CAP + lane * PER;
+#pragma unroll
+    for (int q = 0; q < PER; ++q) dst[q] = __fadd_rn(a[q], -__ldg(dn + q));
+    if (lane == 0) c.cnt_loo[v][row] = __fadd_rn(aloo, -ld);
+  }
+}
+
 cudaError_t launch_counts_loglik(const Ctx& c, cudaStream_t s) {
   if (!c.n_count_views) return cudaSuccess;
   int blocks = (c.n_rows + 15) / 16;               // 16 warps per block
   if (blocks > 148 * 4) blocks = 148 * 4;
   const dim3 grid(blocks, c.n_count_views);         // all count views in one launch
+  if (c.count_model) {
+    switch (c.cap) {
+      case 32: k_counts_loglik_dm<32><<<grid, 512, 0, s>>>(c); break;
+      case 64: k_counts_loglik_dm<64><<<grid, 512, 0, s>>>(c); break;
+      case 128: k_counts_loglik_dm<128><<<grid, 512, 0, s>>>(c); break;
+      case 256: k_counts_loglik_dm<256><<<grid, 512, 0, s>>>(c); break;
+      default: return cudaErrorInvalidValue;
+    }
+    return cudaGetLastError();
+  }
   switch (c.cap) {
     case 32: k_counts_loglik<32><<<grid, 512, 0, s>>>(c); break;
     case 64: k_counts_loglik<64><<<grid, 512, 0, s>>>(c); break;
@@ -201,6 +352,12 @@ cudaError_t launch_counts_loglik(const Ctx& c, cudaStream_t s) {
     case 256: k_counts_loglik<256><<<grid, 512, 0, s>>>(c); break;
     default: return cudaErrorInvalidValue;
   }
+  return cudaGetLastError();
+}
+
+cudaError_t launch_counts_newdish(const Ctx& c, cudaStream_t s) {
+  if (!c.n_count_views || !c.count_model || c.n_rows <= 0) return cudaSuccess;
+  k_counts_newdish<<<dim3((c.n_rows + 255) / 256, c.n_count_views), 256, 0, s>>>(c);
   return cudaGetLastError();
 }
 
@@ -227,8 +384,14 @@ cudaError_t launch_counts_rebuild(const Ctx& c, bool delta, cudaStream_t s) {
   int tb = (int)((max_cells + 255) / 256);
   if (tb > 148 * 8) tb = 148 * 8;
   const int log2cap = __builtin_ctz((unsigned)c.cap);
-  if (c.cap <= 64) k_counts_tables<64><<<dim3(tb, c.n_count_views), 256, 0, s>>>(c, log2cap);
-  else k_counts_tables<256><<<dim3(tb, c.n_count_views), 256, 0, s>>>(c, log2cap);   // one thread per slot: 256 threads
+  if (c.count_model) {
+    if (c.cap <= 64) k_counts_tables<64, true><<<dim3(tb, c.n_count_views), 256, 0, s>>>(c, log2cap);
+    else k_counts_tables<256, true><<<dim3(tb, c.n_count_views), 256, 0, s>>>(c, log2cap);
+  } else if (c.cap <= 64) {
+    k_counts_tables<64, false><<<dim3(tb, c.n_count_views), 256, 0, s>>>(c, log2cap);
+  } else {
+    k_counts_tables<256, false><<<dim3(tb, c.n_count_views), 256, 0, s>>>(c, log2cap);   // one thread per slot: 256 threads
+  }
   return cudaGetLastError();
 }
 

@@ -64,6 +64,12 @@ struct Ctx {
   float* cnt_loo[kMaxViews];   // [N] the same under the row's own dish with the row removed
   float count_beta;            // symmetric Dirichlet pseudo-count
   int32_t n_count_views;
+  // MVG_COUNT_DIRMULT (count_model = 1, every count view of the handle; DESIGN.md §4.5): l2t holds log2(beta + cnt_d)
+  // instead of log2 theta, and
+  int32_t count_model;
+  int32_t cnt_nmax[kMaxViews]; // the longest row in tokens (known at upload)
+  float* cnt_den[kMaxViews];   // [n_max+1][cap] sum_{j<n} log2(W beta + C_k + j) of the dish each slot serves, length-major
+  float* cnt_q[kMaxViews];     // [N] -log2 f_new of every row (fixed once beta is): what the new-dish term reads
   int32_t* table_prev;         // [N] count views: the table every row's words are currently counted at in cnt_t
   float* xx;                // [V][xx_stride] squared norms of the rows (count views: the rows' total counts), computed once per upload
   int64_t xx_stride;        // n_rows rounded up to a multiple of 4
@@ -213,6 +219,7 @@ int stats_smem_bytes(const Ctx& c);
 cudaError_t launch_rowtotals(const int32_t* rowptr, const float* val, float* out, int n, cudaStream_t s);
 cudaError_t launch_counts_rebuild(const Ctx& c, bool delta, cudaStream_t s);   // per count view: word counts per table slot (from scratch, or only the rows that changed table), dish tables
 cudaError_t launch_counts_loglik(const Ctx& c, cudaStream_t s);    // per count view: log2 f of every row under every table
+cudaError_t launch_counts_newdish(const Ctx& c, cudaStream_t s);   // DIRMULT: cnt_q of every count view, once beta is frozen
 // posterior summaries (mv_summary.cu)
 cudaError_t launch_labels(const Ctx& c, int32_t* out, cudaStream_t s);
 cudaError_t launch_cocluster(const Ctx& c, int view, uint32_t* counts, cudaStream_t s);

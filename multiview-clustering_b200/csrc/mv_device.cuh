@@ -94,6 +94,29 @@ __device__ __forceinline__ float log2m(float s) {
   return __fadd_rn((float)e, r);
 }
 
+// ---- Dirichlet-multinomial count views (MVG_COUNT_DIRMULT): lnΓ(a + x) - lnΓ(a), FP64 --------------
+// a > 0, x >= 0 an integer.  Up to kLgdLoop the sum of log(a + j), j < x; above it a is first shifted to >= kLgdLoop by at
+// most kLgdLoop such terms, then the Stirling difference
+//   lnΓ(b) - lnΓ(a) = (a - 1/2) log1p(x / a) + x (log b - 1) + R(b) - R(a),   b = a + x,
+//   R(z) = 1/(12 z) - 1/(360 z^3) + 1/(1260 z^5) - 1/(1680 z^7)   (truncation < 1.3e-14 at z >= 16),
+// whose two main terms are both positive: no cancellation between large lnΓ values, and at most ~2 kLgdLoop logs per
+// call whatever x is (a long row's births and denominators do not become per-token loops).
+constexpr int kLgdLoop = 16;
+__device__ __forceinline__ double stirling_tail(double z) {
+  const double r = 1.0 / z, r2 = r * r;
+  return r * (1.0 / 12.0 - r2 * (1.0 / 360.0 - r2 * (1.0 / 1260.0 - r2 * (1.0 / 1680.0))));
+}
+static __device__ __noinline__ double lgamma_diff(double a, int x) {
+  double s = 0.0;
+  if (x <= kLgdLoop) {
+    for (int j = 0; j < x; ++j) s += log(a + (double)j);
+    return s;
+  }
+  while (a < (double)kLgdLoop) { s += log(a); a += 1.0; x -= 1; }
+  const double xd = (double)x, b = a + xd;
+  return s + (a - 0.5) * log1p(xd / a) + xd * (log(b) - 1.0) + (stirling_tail(b) - stirling_tail(a));
+}
+
 // ---- packed FP32 (sm_100 FFMA2 / FADD2): two IEEE-rounded operations per instruction ------------
 // Each half is rounded exactly like the scalar fmaf / add, so packing changes the instruction count,
 // not a single bit of the result (the CPU mirror stays scalar).

@@ -57,8 +57,9 @@ __global__ void __launch_bounds__(kSimtThreads, 2) k_draw_simt(const Ctx c) {
         if (tid == 0) s_vp = c.vparam[v];
         __syncthreads();
         // k_counts_loglik (mv_counts.cu, one warp per row) left the CAP log2 f values of every customer and its
-        // leave-one-out value in global memory (L2-resident at Reuters size); here: the common per-customer epilogue
-        const float rowtot = c.xx[(size_t)v * c.xx_stride + rowc];
+        // leave-one-out value in global memory (L2-resident at Reuters size); here: the common per-customer epilogue.
+        // The new-dish term is -AN rowtot + CN: the token total under the plug-in, -log2 f_new under DIRMULT (AN = 1, CN = 0)
+        const float rowtot = c.count_model ? __ldg(c.cnt_q[v] + rowc) : c.xx[(size_t)v * c.xx_stride + rowc];
         float acc[CAP];
         {
           const float4* __restrict__ src = reinterpret_cast<const float4*>(c.cnt_acc[v] + (size_t)rowc * CAP);
@@ -196,7 +197,7 @@ __global__ void __launch_bounds__(kSimtThreads, 1) k_draw_simt_wide(const Ctx c)
       const bool dbg = (c.debug_export & 1) && live;
       if (c.kind[v]) {
         // count view: the CAP log2 f values and the leave-one-out value that k_counts_loglik left in global memory
-        const float rowtot = c.xx[(size_t)v * c.xx_stride + rowc];
+        const float rowtot = c.count_model ? __ldg(c.cnt_q[v] + rowc) : c.xx[(size_t)v * c.xx_stride + rowc];
         const float acc_loo = __ldg(c.cnt_loo[v] + rowc);
         epi.view_begin(s_hot, s_cold, 0.0f);
         epi.A1r = 0.0f; epi.C1r = acc_loo;

@@ -597,6 +597,44 @@ __device__ __noinline__ double log_f_dish_counts(const int32_t* __restrict__ rp,
   return lf;
 }
 
+// The same under MVG_COUNT_DIRMULT (oracle/mv_oracle_dm.c:mvod_counts_log_f_vk): the collapsed Dirichlet-multinomial
+// conditional, sum_w [lnΓ(beta + c + x_w) - lnΓ(beta + c)] - [lnΓ(W beta + C + n) - lnΓ(W beta + C)], by lgamma_diff
+// (mv_device.cuh): at most ~2 kLgdLoop logs per nonzero and for the denominator, however long the row.
+// tk = -1 (a dish without tables, or a new dish): c = C = 0.
+__device__ __noinline__ double log_f_dish_counts_dm(const int32_t* __restrict__ rp, const int32_t* __restrict__ col,
+                                                    const float* __restrict__ val, const int32_t* __restrict__ cnt_d,
+                                                    const int cap, const double wbeta, const double beta, const double ctot_k,
+                                                    const int tk, const int row, const bool loo) {
+  int n = 0;
+  double lf = 0.0;
+  for (int j = rp[row]; j < rp[row + 1]; ++j) {
+    const int x = (int)val[j];
+    const int cd = (tk >= 0) ? cnt_d[(size_t)col[j] * cap + tk] - (loo ? x : 0) : 0;
+    lf += lgamma_diff(beta + (double)cd, x);
+    n += x;
+  }
+  const double den = wbeta + ((tk >= 0) ? ctot_k - (loo ? (double)n : 0.0) : 0.0);
+  return lf - lgamma_diff(den, n);
+}
+
+// B1 of k_finalize for a count view: log f of the candidate's ROW under dish k (tk, ctot_k as above) or a new dish, by the
+// handle's count model.  mode: bit 0 leave-one-out, bit 1 new dish, bit 2 Dirichlet-multinomial.  One out-of-line call with
+// few arguments keeps the finalize kernel's register budget.
+__device__ __noinline__ double birth_log_f_counts(const int32_t* __restrict__ rp, const int32_t* __restrict__ col,
+                                                  const float* __restrict__ val, const int32_t* __restrict__ cnt_d,
+                                                  const int cap, const int vocab, const float beta_f, const double ctot_k,
+                                                  const int tk, const int row, const int mode) {
+  const bool loo = (mode & 1) != 0, new_dish = (mode & 2) != 0, dm = (mode & 4) != 0;
+  const double beta = (double)beta_f, wbeta = (double)vocab * (double)beta_f;
+  if (dm) return log_f_dish_counts_dm(rp, col, val, cnt_d, cap, wbeta, beta, ctot_k, new_dish ? -1 : tk, row, loo && !new_dish);
+  if (new_dish) {                    // plug-in: log f_new = -|x| log W
+    double tot = 0.0;
+    for (int j = rp[row]; j < rp[row + 1]; ++j) tot += (double)val[j];
+    return -tot * fin_log((double)vocab);
+  }
+  return log_f_dish_counts(rp, col, val, cnt_d, cap, wbeta, beta, ctot_k, tk, row, loo);
+}
+
 // The Philox numbers of one level's hyper step, by the calling warp's lanes 0..5: rn/lu[which], which = 0 tau, 1 alpha,
 // 2 sigma.  Stream positions are those the reference's sequential code would use: tau_v at v, (alpha_v, sigma_v) at
 // V + 2v, the franchise pair at 3V.  `first`..`last`: the range of `which` this call draws.
@@ -728,16 +766,11 @@ __global__ void __launch_bounds__(kFinThreads, 1) k_finalize(const Ctx c, const 
         double val;
         if (is_count) {  // count view (one GPU per chain: the candidate's row is local)
           const int row = pkt_i32(c, S.cand_g[b], c.pkt.off_cand_row)[S.cand_j[b]];
-          if (k == cap) {
-            double tot = 0.0;
-            for (int j = c.rowptr[v][row]; j < c.rowptr[v][row + 1]; ++j) tot += (double)c.val[v][j];
-            val = -tot * fin_log((double)c.vocab[v]);
-          } else {
-            const int t0 = pkt_i32(c, S.cand_g[b], c.pkt.off_cand_t0)[S.cand_j[b]];
-            val = log_f_dish_counts(c.rowptr[v], c.col[v], c.val[v], c.cnt_d[v], cap, (double)c.vocab[v] * (double)c.count_beta,
-                                    (double)c.count_beta, S.s2k_start[k], S.table_of_dish[k], row,
-                                    (k == S.dish[t0]) && S.n_vk[k] > 0);
-          }
+          const int t0 = pkt_i32(c, S.cand_g[b], c.pkt.off_cand_t0)[S.cand_j[b]];
+          const bool own = (k < cap) && (k == S.dish[t0]) && S.n_vk[k] > 0;
+          val = birth_log_f_counts(c.rowptr[v], c.col[v], c.val[v], c.cnt_d[v], cap, c.vocab[v], c.count_beta,
+                                   (k < cap) ? S.s2k_start[k] : 0.0, (k < cap) ? S.table_of_dish[k] : -1, row,
+                                   (own ? 1 : 0) | (k == cap ? 2 : 0) | (c.count_model ? 4 : 0));
         } else if (k == cap) {   // new dish: N(x; 0, tau)   (multiview_utils.cpp:340-350)
           double q = 0.0;
           for (int dd = 0; dd < D; ++dd) q += (double)x[dd] * (double)x[dd];
@@ -1175,6 +1208,7 @@ __global__ void __launch_bounds__(kFinThreads, 1) k_finalize(const Ctx c, const 
     p.AN = (float)(kLog2e / (2.0 * tau));
     p.CN = (float)(kLog2e * (-0.5 * (double)D * fin_log(2.0 * kPi * tau)));
     if (is_count) { p.AN = (float)fin_log2((double)c.vocab[v]); p.CN = 0.f; }      // log2 f_new = -|x| log2 W
+    if (is_count && c.count_model) { p.AN = 1.f; p.CN = 0.f; }   // DIRMULT: the draw passes -log2 f_new itself (cnt_q)
     const double wn0 = alpha_l + (double)K_act * sigma_l, wn1 = alpha_l + (double)(K_act - 1) * sigma_l;
     p.WN0 = wn0 > 0.0 ? (float)fin_log2(wn0) : kMasked;
     p.WN1 = wn1 > 0.0 ? (float)fin_log2(wn1) : kMasked;

@@ -8,7 +8,8 @@
 //                   index (mcclust::arandi, :189) follows in closed form
 //   k_loglik        joint log marginal likelihood of the data given the partition: the sum over live dishes of
 //                   the reference's log p(y_S) (multiview_utils.cpp:316-320, per coordinate) — what the
-//                   declared-but-never-defined compute_log_likelihood() (multiview_gibbs.h:13) would return
+//                   declared-but-never-defined compute_log_likelihood() (multiview_gibbs.h:13) would return; for a
+//                   count view under MVG_COUNT_DIRMULT the collapsed Dirichlet-multinomial marginal
 #include "mv_ctx.h"
 
 namespace mv {
@@ -43,23 +44,56 @@ __global__ void k_contingency(const Ctx c, const int view, const int32_t* __rest
   if (k >= 0 && z >= 0 && z < n_classes) atomicAdd(&table[k * n_classes + z], 1);
 }
 
+// A count view under MVG_COUNT_DIRMULT: the collapsed marginal of the partition up to the multinomial coefficients (which
+// do not depend on it), sum over live dishes k of sum_w lnΓ(beta + c_kw) - lnΓ(beta)  -  [lnΓ(W beta + C_k) - lnΓ(W beta)],
+// the word counts read from the lowest table slot serving each dish (cnt_d, current after every rebuild).  Thread tid takes
+// the words w = tid mod blockDim.x over all live dishes, then its dish denominators; the block sums in ascending order.
+// (scalars and pointers, not `const Ctx&`: the address of the kernel parameter would copy the struct per thread)
+__device__ double loglik_dirmult_term(const int32_t* __restrict__ cd, const double* __restrict__ ctot, int vocab, int cap,
+                                      double beta, const int32_t* s_rep) {
+  double term = 0.0;
+  for (int w = threadIdx.x; w < vocab; w += blockDim.x)
+    for (int k = 0; k < cap; ++k) {
+      const int tk = s_rep[k];
+      if (tk < 0) continue;
+      const int x = cd[(size_t)w * cap + tk];
+      if (x > 0) term += lgamma_diff(beta, x);
+    }
+  for (int k = threadIdx.x; k < cap; k += blockDim.x)
+    if (s_rep[k] >= 0) term -= lgamma_diff((double)vocab * beta, (int)ctot[k]);
+  return term;
+}
+
 __global__ void __launch_bounds__(256) k_loglik(const Ctx c, double* __restrict__ out /* [V+1]: per view, then the total */) {
   __shared__ double s_term[256];
+  __shared__ int32_t s_rep[256];                  // DIRMULT: lowest table slot of every live dish, -1 = none
   const double kPi = 3.14159265358979323846;
   double total = 0.0;
   for (int v = 0; v < c.V; ++v) {
     const double tau = c.hyp[2 * c.V + v];
     const int D = c.D[v];
     double term = 0.0;
-    for (int k = threadIdx.x; k < c.cap; k += blockDim.x) {
-      const int n = c.n_vk[v * c.cap + k];
-      if (n <= 0) continue;
-      const double* S1 = c.S1k + (size_t)c.cap * c.doff[v] + (size_t)k * D;
-      double q = 0.0;
-      for (int dd = 0; dd < D; ++dd) q += S1[dd] * S1[dd];
-      const double nn = (double)n;
-      term += -0.5 * nn * (double)D * log(2.0 * kPi * tau) - 0.5 * (double)D * log(tau * (tau + nn)) -
-              0.5 * c.S2k[v * c.cap + k] / tau + 0.5 * q / (tau * (tau + nn));
+    if (c.kind[v] && c.count_model) {
+      if (threadIdx.x < c.cap) {
+        const int k = threadIdx.x;
+        int rep = -1;
+        if (c.n_vk[v * c.cap + k] > 0)
+          for (int t = c.cap - 1; t >= 0; --t) if (c.dish_of[v * c.cap + t] == k) rep = t;
+        s_rep[k] = rep;
+      }
+      __syncthreads();
+      term = loglik_dirmult_term(c.cnt_d[v], c.S2k + v * c.cap, c.vocab[v], c.cap, (double)c.count_beta, s_rep);
+    } else {
+      for (int k = threadIdx.x; k < c.cap; k += blockDim.x) {
+        const int n = c.n_vk[v * c.cap + k];
+        if (n <= 0) continue;
+        const double* S1 = c.S1k + (size_t)c.cap * c.doff[v] + (size_t)k * D;
+        double q = 0.0;
+        for (int dd = 0; dd < D; ++dd) q += S1[dd] * S1[dd];
+        const double nn = (double)n;
+        term += -0.5 * nn * (double)D * log(2.0 * kPi * tau) - 0.5 * (double)D * log(tau * (tau + nn)) -
+                0.5 * c.S2k[v * c.cap + k] / tau + 0.5 * q / (tau * (tau + nn));
+      }
     }
     s_term[threadIdx.x] = term;
     __syncthreads();

@@ -20,6 +20,7 @@ _HERE = Path(__file__).resolve().parent
 LIB_PATH = _HERE / "libmvg_b200.so"
 
 ENGINE_AUTO, ENGINE_SIMT, ENGINE_TCGEN05, ENGINE_TCGEN05_FAST = 0, 1, 2, 3
+COUNT_LIKELIHOODS = {"plugin": 0, "dirmult": 1}   # MVG_COUNT_PLUGIN / MVG_COUNT_DIRMULT
 NEW_TABLE = -1
 
 _i32p = C.POINTER(C.c_int32)
@@ -84,6 +85,8 @@ def lib():
         L.mvg_upload_view_csr.argtypes = [H, C.c_int32, _i32p, _i32p, _f32p, C.c_int64, C.c_int32]
         L.mvg_set_count_beta.argtypes = [H, C.c_double]
         L.mvg_get_count_tables.argtypes = [H, C.c_int32, _f32p, _i32p, _i32p]
+        L.mvg_set_count_likelihood.argtypes = [H, C.c_int32]
+        L.mvg_get_count_den.argtypes = [H, C.c_int32, _f32p, _i32p]
         L.mvg_get_debug_loo.argtypes = [H, _f32p]
         L.mvg_init_state_reference.argtypes = [H]
         L.mvg_set_state.argtypes = [H, C.POINTER(_StateHost)]
@@ -176,6 +179,7 @@ class Sampler:
         if rc != 0:
             raise MvgError(rc, self.L.mvg_last_error(None).decode())
         self._keep = []
+        self.count_likelihood = "plugin"
 
     # -- plumbing ---------------------------------------------------------------------------
     def _ck(self, rc):
@@ -219,8 +223,26 @@ class Sampler:
     def set_count_beta(self, beta):
         self._ck(self.L.mvg_set_count_beta(self.h, float(beta)))
 
+    def set_count_likelihood(self, model):
+        """"plugin" (default: the plug-in multinomial) or "dirmult" (the collapsed Dirichlet-multinomial) for every
+        count view; before the first state call."""
+        if model not in COUNT_LIKELIHOODS:
+            raise MvgError(-1, f"unknown count likelihood {model!r}: expected one of {sorted(COUNT_LIKELIHOODS)}")
+        self._ck(self.L.mvg_set_count_likelihood(self.h, COUNT_LIKELIHOODS[model]))
+        self.count_likelihood = model
+
+    def get_count_den(self, v):
+        """"dirmult" count view v: (den [n_max + 1, cap], n_max), den[n][t] = sum_{j<n} log2(W beta + C_k + j) of the dish
+        table slot t serves, for the NEXT sweep."""
+        n_max = C.c_int32(0)
+        self._ck(self.L.mvg_get_count_den(self.h, v, None, C.byref(n_max)))
+        den = np.empty((n_max.value + 1, self.cap), np.float32)
+        self._ck(self.L.mvg_get_count_den(self.h, v, _p(den, _f32p), C.byref(n_max)))
+        return den, n_max.value
+
     def get_count_tables(self, v):
-        """(log2 theta, dish counts, table counts), each [vocab, cap], of count view v for the NEXT sweep."""
+        """(log2 theta, dish counts, table counts), each [vocab, cap], of count view v for the NEXT sweep.  Under the
+        "dirmult" likelihood the first holds log2(beta + c) of the dish's word count c instead of log2 theta."""
         W = self.vocab[v]
         l2t = np.empty((W, self.cap), np.float32)
         cd = np.empty((W, self.cap), np.int32)
@@ -368,7 +390,8 @@ class Sampler:
         hyp = np.empty((max(n_saved_max, 1), 3 * self.V + 2), np.float64)
         ll = np.zeros(max(n_saved_max, 1), np.float64)
         ns = C.c_int32(0)
-        dense = all(d > 0 for d in self.dims)            # the log-likelihood kernel covers the Gaussian views
+        # the log-likelihood kernel covers the Gaussian views and the Dirichlet-multinomial count views
+        dense = all(d > 0 for d in self.dims) or self.count_likelihood == "dirmult"
         self._ck(self.L.mvg_run(self.h, M, burn_in, thin, n_saved_max, _p(tab, _i32p), _p(dish, _i32p),
                                 _p(hyp, _f64p), _p(ll, _f64p) if dense else None, C.byref(ns)))
         S = ns.value
@@ -489,14 +512,16 @@ def _as_csr(v):
     return None
 
 
-def run_gibbs(data_views, M, burn_in, thin, cap=64, seed=1999, device=0, engine=ENGINE_AUTO, start=None, blocks=1):
+def run_gibbs(data_views, M, burn_in, thin, cap=64, seed=1999, device=0, engine=ENGINE_AUTO, start=None, blocks=1,
+              count_likelihood="plugin"):
     """run_gibbs_cpp(data_views, M, burn_in, thin) on the GPU (multiview_gibbs.cpp:105-131).
 
     ``data_views`` is a list of per-view arrays (vectors as in New_Simulation.R:105-111, or [n, D]
     matrices); a sparse count view (the X_body / X_title / X_topics of dataset/reuters/data pre-process.R) is a
     scipy.sparse matrix or a dict {"rowptr", "col", "val", "vocab"}.  ``start`` = (table_of, dish_of) replaces the
     reference's random T = 4 / K = 2 start.  Returns a dict with the reference's eight keys; ``table_of`` is
-    0-based, ``dish_of`` is indexed [saved][view][table slot] with -1 for a free slot.
+    0-based, ``dish_of`` is indexed [saved][view][table slot] with -1 for a free slot.  ``count_likelihood`` is
+    "plugin" or "dirmult" (Sampler.set_count_likelihood).
     """
     csr = [_as_csr(v) for v in data_views]
     views = [None if c is not None else np.asarray(v, dtype=np.float64).reshape(len(v), -1) for v, c in zip(data_views, csr)]
@@ -510,6 +535,8 @@ def run_gibbs(data_views, M, burn_in, thin, cap=64, seed=1999, device=0, engine=
                 s.upload_view(v, x)
         if blocks > 1:
             s.set_sweep_blocks(blocks)
+        if count_likelihood != "plugin":
+            s.set_count_likelihood(count_likelihood)
         if start is None:
             s.init_state_reference()
         else:
