@@ -186,6 +186,15 @@ int mvg_set_stats_mode(mvg_handle* h, int32_t mode, int32_t rebuild_every);
  * reference's sequential order (multiview_gibbs.cpp:157-200) — the knob trades throughput for closeness to it.
  * The Philox addressing (sweep, row) is unchanged, so chains stay reproducible and shard-invariant. */
 int mvg_set_sweep_blocks(mvg_handle* h, int32_t blocks);
+/* Draw screening (tensor-core engines; on by default there, ignored by the CUDA-core engine and by debug handles).  Before every draw a
+ * screening kernel tests, for every row, a stored lower bound on how far its own table leads every other table; a tile of
+ * 128 rows that all lead by more than 2^31 in weight gets its draw (its own table) written without reading its features.
+ * The bound is exact: a chain draws the same tables with screening on or off.  It applies to sweeps with every table slot
+ * live and every dish served by one table; other sweeps evaluate every row.  Switching it changes no state. */
+int mvg_set_draw_screen(mvg_handle* h, int32_t on);
+/* What screening did in the most recent draw: enabled (0/1), rows whose draw was screened, row tiles (128 rows) the draw
+ * evaluated.  Any pointer may be NULL.  Synchronises. */
+int mvg_get_draw_screen_stats(mvg_handle* h, int32_t* enabled, int64_t* rows_screened, int64_t* tiles_evaluated);
 int mvg_hyper_step(mvg_handle* h);
 /* The same restricted to some of its Metropolis-Hastings updates: update_tau_v_MH alone
  * (multiview_hyper.cpp:211-231), the per-view alpha/sigma pairs (:242-265), the franchise pair (:268-291). */

@@ -113,6 +113,7 @@ struct mvg_handle {
   bool xattached = false;            // peer mappings exist (they live until mvg_destroy)
   double* loglik_dev = nullptr;      // [V + 1] scratch of mvg_run's per-kept-sweep log-likelihood
   int32_t* host_fault = nullptr;     // mapped pinned host word: the sticky exchange fault, readable without a sync
+  bool screen_want = true;           // mvg_set_draw_screen (effective on the tensor-core engines)
 };
 
 namespace {
@@ -215,7 +216,20 @@ int ensure_layout(mvg_handle* h) {
     if (posix_memalign(&h->tc_maps, 128, draw_tc_maps_bytes()) != 0) return fail(h, MVG_ENOMEM, "tensor map allocation");
     cudaError_t e = draw_tc_make_maps(c, h->tc_maps);
     if (e != cudaSuccess) return fail(h, MVG_ECUDA, std::string("cuTensorMapEncodeTiled: ") + cudaGetErrorString(e));
+    // draw screening (DESIGN.md §4.1.1): the verdict record, the reference parameters, a margin per row, the tile list
+    if ((rc = dev_alloc(h, &c.scr, 1)) != MVG_OK || (rc = dev_alloc(h, &c.scr_tp, V * cap)) != MVG_OK ||
+        (rc = dev_alloc(h, &c.scr_tm, cap)) != MVG_OK || (rc = dev_alloc(h, &c.scr_b, 2 * cap * dsum)) != MVG_OK ||
+        (rc = dev_alloc(h, &c.margin, N)) != MVG_OK || (rc = dev_alloc(h, &c.scr_tiles, (N + 127) / 128)) != MVG_OK)
+      return rc;
+    c.screen = (h->screen_want && !c.debug_export) ? 1 : 0;   // debug handles export what the full path computed
   }
+  return MVG_OK;
+}
+
+// The margins stand for the seating they were recorded at: anything that replaces it from outside drops the reference, and
+// the next screened draw evaluates every row (a refresh).  Stream-ordered; a no-op without screening state.
+int invalidate_screen(mvg_handle* h) {
+  if (h->c.scr) MVG_CUDA(h, cudaMemsetAsync(&h->c.scr->valid, 0, sizeof(uint32_t), h->stream));
   return MVG_OK;
 }
 
@@ -278,9 +292,15 @@ int prepare_count_model(mvg_handle* h) {
 }
 
 int launch_draw(mvg_handle* h, bool programmatic = false) {
-  if (h->engine == MVG_ENGINE_TCGEN05 || h->engine == MVG_ENGINE_TCGEN05_FAST)
+  if (h->engine == MVG_ENGINE_TCGEN05 || h->engine == MVG_ENGINE_TCGEN05_FAST) {
+    if (h->c.screen) {                 // the screening kernel takes the draw's place in the programmatic chain
+      MVG_CUDA(h, launch_draw_screen(h->c, programmatic, h->stream));
+      h->launches += 1;
+    }
     MVG_CUDA(h, launch_draw_tc(h->c, h->tc_maps, h->engine == MVG_ENGINE_TCGEN05_FAST, programmatic, h->stream));
-  else MVG_CUDA(h, launch_draw_simt(h->c, h->stream));
+  } else {
+    MVG_CUDA(h, launch_draw_simt(h->c, h->stream));
+  }
   h->launches += 1 + ((h->engine == MVG_ENGINE_SIMT && h->c.n_count_views) ? 1 : 0);
   return MVG_OK;
 }
@@ -594,6 +614,7 @@ int mvg_init_state_reference(mvg_handle* h) {
   if (rc == MVG_OK) rc = prepare_count_model(h);
   if (rc != MVG_OK) return rc;
   if (h->c.cap < 4) return fail(h, MVG_EINVAL, "reference initialisation needs cap >= 4");
+  if ((rc = invalidate_screen(h)) != MVG_OK) return rc;
   const uint32_t zero = 0;
   MVG_CUDA(h, cudaMemcpyAsync(h->c.sweep, &zero, sizeof(zero), cudaMemcpyHostToDevice, h->stream));
   MVG_CUDA(h, launch_init_tables(h->c, 0, h->stream));
@@ -613,6 +634,7 @@ int mvg_set_state(mvg_handle* h, const mvg_state_host* s) {
   int rc = ensure_layout(h);
   if (rc == MVG_OK) rc = prepare_count_model(h);
   if (rc != MVG_OK) return rc;
+  if ((rc = invalidate_screen(h)) != MVG_OK) return rc;
   const Ctx& c = h->c;
   if (!s->table_of || !s->dish_of || !s->alpha_v || !s->sigma_v || !s->tau_v || !s->alpha_sigma_global)
     return fail(h, MVG_EINVAL, "set_state needs table_of, dish_of, alpha_v, sigma_v, tau_v, alpha_sigma_global");
@@ -850,6 +872,33 @@ int mvg_set_sweep_blocks(mvg_handle* h, int32_t blocks) {
   h->c.blk_count = blocks;
   h->c.blk_index = 0;
   invalidate_graphs(h);
+  return MVG_OK;
+}
+
+int mvg_set_draw_screen(mvg_handle* h, int32_t on) {
+  if (!h) return MVG_EINVAL;
+  h->screen_want = on != 0;
+  invalidate_graphs(h);                              // the switch is part of the captured kernel arguments
+  if (h->c.scr) {
+    h->c.screen = (h->screen_want && !h->c.debug_export) ? 1 : 0;
+    MVG_CUDA(h, cudaSetDevice(h->cfg.device));
+    return invalidate_screen(h);                     // margins recorded before a stretch without screening are stale
+  }
+  return MVG_OK;
+}
+
+int mvg_get_draw_screen_stats(mvg_handle* h, int32_t* enabled, int64_t* rows_screened, int64_t* tiles_evaluated) {
+  if (!h) return MVG_EINVAL;
+  if (enabled) *enabled = h->c.screen;
+  if (rows_screened) *rows_screened = 0;
+  if (tiles_evaluated) *tiles_evaluated = 0;
+  if (!h->c.scr || !h->c.screen) return MVG_OK;
+  MVG_CUDA(h, cudaSetDevice(h->cfg.device));
+  ScreenRec r;
+  MVG_CUDA(h, cudaMemcpyAsync(&r, h->c.scr, sizeof(r), cudaMemcpyDeviceToHost, h->stream));
+  MVG_CUDA(h, cudaStreamSynchronize(h->stream));
+  if (rows_screened) *rows_screened = r.last_rows_screened;
+  if (tiles_evaluated) *tiles_evaluated = r.last_tiles_evaluated;
   return MVG_OK;
 }
 

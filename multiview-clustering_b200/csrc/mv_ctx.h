@@ -128,7 +128,41 @@ struct Ctx {
   double* dbg_birth_w;      // [cap][V][cap+1]
   int32_t* dbg_nseated;     // [1]
   long long* dbg_prof;      // [CTAs][16] cycles spent waiting per role of the tcgen05 kernel (debug_export & 2)
+
+  // draw screening (tensor-core engine, DESIGN.md §4.1.1): rows whose draw is provably their own table skip the draw
+  int32_t screen;           // k_draw_screen runs before every draw of this handle
+  struct ScreenRec* scr;    // [1] the screening kernel's verdict for the draw that follows, and the reference sweep
+  TableParam* scr_tp;       // [V][cap] parameter block of the reference sweep
+  TableMass* scr_tm;        // [cap]
+  float* scr_b;             // [2][cap*Dsum] its mean_hi, mean_lo
+  float* margin;            // [N] lower bound on (own-table log2 weight - best other) at the reference, see ScreenRec
+  int32_t* scr_tiles;       // [ceil(N/128)] row tiles the draw evaluates (mode kScreenSkip)
 };
+
+// What k_draw_screen hands to k_draw_tc, and the reference the margins are measured against.  Written by k_draw_screen:
+// mode, k, n_eval, last_*; by k_draw_tc (CTA 0, after it has waited for the screening kernel): valid, ref_sweep.
+enum { kScreenOff = 0, kScreenRefresh = 1, kScreenSkip = 2 };
+constexpr int kScreenPeriod = 64;      // sweeps between two full evaluations (new reference)
+struct ScreenRec {
+  int32_t mode;             // kScreenOff: every tile, nothing recorded; kScreenRefresh: every tile, new reference; kScreenSkip: the list
+  int32_t n_eval;           // tiles in scr_tiles
+  float k[1 + 2 * 3];       // row bound Q = k0 + sum_v kA_v |x_v|^2 + kB_v |x_v|: drift since the reference + evaluation error
+  uint32_t valid;           // the reference parameters and the margins stand for the current seating
+  uint32_t ref_sweep;
+  uint32_t cnt, done, rows; // scratch of one screening launch (tile counter, CTAs finished, rows screened), zero between launches
+  int64_t last_rows_screened, last_tiles_evaluated;
+};
+#ifdef __CUDACC__
+// The row's bound, rounded upward: k_draw_tc subtracts it when it records a margin, k_draw_screen when it tests one.
+__device__ __forceinline__ float screen_row_bound(const float* k, const float* xx, int V) {
+  float q = k[0];
+  for (int v = 0; v < V; ++v) {
+    q = __fmaf_ru(k[1 + v], xx[v], q);
+    q = __fmaf_ru(k[4 + v], __fsqrt_ru(xx[v]), q);
+  }
+  return q;
+}
+#endif
 
 // Programmatic dependent launch along the sweep: draw -> pack -> statistics -> reduce -> finalize -> draw.  Every kernel of
 // the chain lets its successor be scheduled at once (pdl_trigger) and orders itself behind its predecessor with pdl_wait
@@ -202,6 +236,7 @@ cudaError_t launch_draw_tc(const Ctx& c, const void* maps, bool fast_exp, bool p
 bool draw_tc_supported(const Ctx& c);
 size_t draw_tc_maps_bytes();                                   // host blob holding the TMA tensor maps
 cudaError_t draw_tc_make_maps(const Ctx& c, void* maps_out);  // (re)encode them for the current pointers
+cudaError_t launch_draw_screen(const Ctx& c, bool programmatic, cudaStream_t s);   // before launch_draw_tc when c.screen
 cudaError_t launch_pack(const Ctx& c, cudaStream_t s);
 // delta: only the rows that moved this sweep are visited; the per-CTA partials then hold the CHANGE of the statistics
 // (rows that arrived minus rows that left) and k_reduce_x adds it to the shard's running sums (mode flag there).

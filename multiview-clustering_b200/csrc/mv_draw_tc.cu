@@ -334,7 +334,8 @@ __global__ void __launch_bounds__(kThreads, 1) k_draw_tc(const Ctx c, const __gr
   TableMass* s_tm = reinterpret_cast<TableMass*>(smem + SmemLayout::tm_off);
   ViewParam* s_vp = reinterpret_cast<ViewParam*>(smem + SmemLayout::vp_off);
   float* s_lm = reinterpret_cast<float*>(smem + SmemLayout::lm_off);
-  uint32_t* s_misc = reinterpret_cast<uint32_t*>(smem + SmemLayout::misc_off);   // [0] TMEM base, [1] sweep, [2..3] GlobalParam floats
+  uint32_t* s_misc = reinterpret_cast<uint32_t*>(smem + SmemLayout::misc_off);   // [0] TMEM base, [1] sweep, [2..3] GlobalParam floats,
+                                                                                 // [4] all_lone, [5] screening mode, [6..12] its bound coefficients
 
   // barrier addresses
   const uint32_t bar0 = sbase + SmemLayout::bar_off;
@@ -372,6 +373,16 @@ __global__ void __launch_bounds__(kThreads, 1) k_draw_tc(const Ctx c, const __gr
   const uint32_t tmem_base = s_misc[0];
 
   const int n_tiles = (c.n_rows + kTileRows - 1) / kTileRows;
+  // The tiles this launch evaluates: all of them, or the list of k_draw_screen (DESIGN.md §4.1.1), which then exists only
+  // once this grid's dependency has resolved.  Every role walks the same sequence k = blockIdx.x, + gridDim.x, ...
+  auto work_list = [&](const int*& list) -> int {
+    list = nullptr;
+    if (!c.screen) return n_tiles;
+    grid_dependency_wait();
+    if (c.scr->mode != kScreenSkip) return n_tiles;
+    list = c.scr_tiles;
+    return c.scr->n_eval;
+  };
   const bool prof = DEBUG && (c.debug_export & 2) != 0 && c.dbg_prof != nullptr;
   const bool dbg_rows = DEBUG && (c.debug_export & 1) != 0;
   long long* prof_out = prof ? c.dbg_prof + (size_t)blockIdx.x * 16 : nullptr;
@@ -399,7 +410,12 @@ __global__ void __launch_bounds__(kThreads, 1) k_draw_tc(const Ctx c, const __gr
                           part ? &maps.mean_lo : &maps.mean_hi, b_full, h * kHalfCols, v * 64);
         b_loaded = true;
       };
-      for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x)
+      const int* list;
+      const int n_work = work_list(list);
+      for (int k = blockIdx.x; k < n_work; k += gridDim.x) {
+        const int tile = list ? list[k] : k;
+        const int kn = k + gridDim.x;
+        const int tn = (kn < n_work) ? (list ? list[kn] : kn) : -1;
         for (int v = 0; v < V; ++v)
 #pragma unroll 1
           for (int h = 0; h < 2; ++h) {
@@ -409,8 +425,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_draw_tc(const Ctx c, const __gr
             tma_load_2d_hint(sbase + SmemLayout::raw_off + r.stage * kHalfBytes, &maps.x[v], raw_full(r.stage),
                              h * kHalfCols, tile * kTileRows, stream_policy);
             {                                           // pull the same half of the CTA's next tile into L2 meanwhile
-              const int tn = tile + gridDim.x;
-              if (tn < n_tiles)
+              if (tn >= 0)
                 asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global.L2::cache_hint [%0, {%1, %2}], %3;"
                              ::"l"(reinterpret_cast<uint64_t>(&maps.x[v])), "r"(h * kHalfCols), "r"(tn * kTileRows),
                                "l"(stream_policy) : "memory");
@@ -418,6 +433,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_draw_tc(const Ctx c, const __gr
             r.next();
             ++issued;
           }
+      }
       if (!b_loaded) load_b();
       if (prof) { prof_out[0] = w0; prof_out[1] = clock64() - t_start; }
     } else if (warp >= 1 && warp <= kMmaWarps) {
@@ -435,7 +451,9 @@ __global__ void __launch_bounds__(kThreads, 1) k_draw_tc(const Ctx c, const __gr
       const uint32_t a_me = desc_lo(sbase + SmemLayout::raw_off + me * 2 * kHalfBytes);   // this warp's two raw stages
       const uint32_t b_lo0 = desc_lo(sbase + SmemLayout::b_off);
       const uint32_t lo_tmem = tmem_base + (uint32_t)(kLoCol0 + me * 64);                 // this warp's remainder stage
-      const int n_tv = ((n_tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x) * V;
+      const int* list;
+      const int n_work = work_list(list);
+      const int n_tv = (n_work > (int)blockIdx.x) ? ((n_work - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x) * V : 0;
       int v = me % V, ds = me;                       // view and accumulator stage of tile-view i
       const int vstep = kMmaWarps % V;
       uint32_t use = 0;                              // how many tile-views this warp has issued
@@ -497,7 +515,9 @@ __global__ void __launch_bounds__(kThreads, 1) k_draw_tc(const Ctx c, const __gr
     const uint32_t lane_base = (uint32_t)((warp & 3) * 32) << 16;
     const uint32_t line = (uint32_t)r * 128u;
     int i = 0;                                         // tile-view counter of this CTA
-    for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x)
+    const int* list;
+    const int n_work = work_list(list);
+    for (int k = blockIdx.x; k < n_work; k += gridDim.x)
       for (int v = 0; v < V; ++v, ++i) {
         const int rs = (2 * i + h) % kRawStages;
         const uint32_t rph = (uint32_t)((2 * i + h) / kRawStages) & 1u;
@@ -577,6 +597,29 @@ __global__ void __launch_bounds__(kThreads, 1) k_draw_tc(const Ctx c, const __gr
         s_misc[2] = __float_as_uint(g.LMN0);
         s_misc[3] = __float_as_uint(g.LMN1);
       }
+      if (c.screen) {
+        // The screening verdict of this sweep.  A refresh makes this sweep's parameters the reference of the margins every
+        // row records below (the CTAs copy a slice each; nothing reads the copy before the next screening launch); a sweep
+        // that does not screen leaves no valid reference behind.
+        const int mode = c.scr->mode;
+        if (et == 0) s_misc[5] = (uint32_t)mode;
+        if (et < 7) s_misc[6 + et] = __float_as_uint(c.scr->k[et]);
+        if (mode == kScreenRefresh) {
+          const int nb = c.cap * c.Dsum;
+          for (int i = blockIdx.x * 512 + et; i < 2 * nb + V * 64 + 64; i += gridDim.x * 512) {
+            if (i < nb) c.scr_b[i] = c.mean_hi[i];
+            else if (i < 2 * nb) c.scr_b[i] = c.mean_lo[i - nb];
+            else if (i < 2 * nb + V * 64) c.scr_tp[i - 2 * nb] = c.tparam[i - 2 * nb];
+            else c.scr_tm[i - 2 * nb - V * 64] = c.tmass[i - 2 * nb - V * 64];
+          }
+        }
+        if (blockIdx.x == 0 && et == 0) {
+          if (mode == kScreenRefresh) { c.scr->ref_sweep = c.gparam->sweep; c.scr->valid = 1u; }
+          else if (mode == kScreenOff) c.scr->valid = 0u;
+        }
+      } else if (et == 0) {
+        s_misc[5] = (uint32_t)kScreenOff;
+      }
       if (!lone_ok) atomicAnd(&s_misc[4], 0u);
       asm volatile("bar.sync 9, 512;" ::: "memory");    // the epilogue warpgroups only: the other roles never read these
     }
@@ -585,6 +628,9 @@ __global__ void __launch_bounds__(kThreads, 1) k_draw_tc(const Ctx c, const __gr
     gp.LMN0 = __uint_as_float(s_misc[2]);
     gp.LMN1 = __uint_as_float(s_misc[3]);
     const bool all_lone_rt = s_misc[4] != 0u;
+    const bool record_rt = s_misc[5] != (uint32_t)kScreenOff;   // then with_new is off and all_lone on (k_draw_screen's precondition)
+    const int* list;
+    const int n_work = work_list(list);
     // Two CTA-uniform properties of the sweep select one of four copies of the loop, so that the registers and the code of
     // the rarer cases stay out of the common one:
     //   with_new   a table slot is free: the new-table option has weight and the per-view marginals are evaluated;
@@ -606,8 +652,12 @@ __global__ void __launch_bounds__(kThreads, 1) k_draw_tc(const Ctx c, const __gr
     // the two threads of a customer sit in the same warp slot of the pair's two warpgroups: only those two warps meet
     auto rendezvous = [&]() { asm volatile("bar.sync %0, 64;" ::"r"(1 + pair * 4 + (warp & 3)) : "memory"); };
     const float4* base4 = reinterpret_cast<const float4*>(s_lm + tb);
+    // margins (DESIGN.md §4.1.1): only the variant without a new-table option and with lone dishes records them
+    constexpr bool can_record = !with_new && all_lone;
+    const bool record = can_record && record_rt;
     int j = pair;
-    const int tile0 = blockIdx.x + pair * gridDim.x;
+    const int k0 = blockIdx.x + pair * gridDim.x;
+    const int tile0 = (k0 < n_work) ? (list ? list[k0] : k0) : n_tiles;
     int t0_next = (tile0 < n_tiles) ? c.table_cur[min(tile0 * kTileRows + r, c.n_rows - 1)] : 0;
     // |x|^2 of the customer in every view: computed once when the view was uploaded (c.xx), fetched a tile ahead
     float xx_next[kMaxTcViews];
@@ -616,7 +666,9 @@ __global__ void __launch_bounds__(kThreads, 1) k_draw_tc(const Ctx c, const __gr
       xx_next[v] = (tile0 < n_tiles) ? c.xx[(size_t)v * c.xx_stride + min(tile0 * kTileRows + r, c.n_rows - 1)] : 0.0f;   // (xx has >= 3 rows)
     long long ph[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0}, tlast = prof ? clock64() : 0;      // DEBUG: cycles per phase of the tile loop
     auto phase = [&](int k) { if (prof) { const long long now = clock64(); ph[k] += now - tlast; tlast = now; } };
-    for (int tile = tile0; tile < n_tiles; tile += kEpiGroups * gridDim.x, j += kEpiGroups) {
+    int tile_next = tile0;
+    for (int k = k0; k < n_work; k += kEpiGroups * gridDim.x, j += kEpiGroups) {
+      const int tile = tile_next;
       const int row = tile * kTileRows + r;
       const bool live = row < c.n_rows;
       const int rowc = live ? row : (c.n_rows - 1);
@@ -628,7 +680,9 @@ __global__ void __launch_bounds__(kThreads, 1) k_draw_tc(const Ctx c, const __gr
 #pragma unroll
       for (int v = 0; v < kMaxTcViews; ++v) xxv[v] = xx_next[v];
       {                                               // the next tile's tables and norms travel while this one is computed
-        const int tn = tile + kEpiGroups * gridDim.x;
+        const int kn = k + kEpiGroups * gridDim.x;
+        const int tn = (kn < n_work) ? (list ? list[kn] : kn) : n_tiles;
+        tile_next = tn;
         if (tn < n_tiles) {
           const int rn = min(tn * kTileRows + r, c.n_rows - 1);
           t0_next = c.table_cur[rn];
@@ -762,6 +816,17 @@ __global__ void __launch_bounds__(kThreads, 1) k_draw_tc(const Ctx c, const __gr
         hmax = fmaxf(M0, M1);
       }
       ex_own[9 * kTileRows] = hmax;
+      if (can_record) {                               // this half's best table other than the customer's own
+        if (record) {
+          float X0 = kMasked, X1 = kMasked;
+#pragma unroll
+          for (int i = 0; i < 16; ++i) {
+            X0 = fmaxf(X0, (2 * i == rel) ? kMasked : lw2[i].x);
+            X1 = fmaxf(X1, (2 * i + 1 == rel) ? kMasked : lw2[i].y);
+          }
+          ex_own[0] = fmaxf(X0, X1);                  // field 0 belongs to the new-table marginal, absent here
+        }
+      }
       // which tables of this half lie within 2^-31 of its best one (see the shortcut below)
       uint32_t nmask = 0u;
       {
@@ -774,6 +839,8 @@ __global__ void __launch_bounds__(kThreads, 1) k_draw_tc(const Ctx c, const __gr
       phase(2);
       rendezvous();                                   // #1: dish sums, own-dish terms, half maxima, the uniform
       phase(3);
+      float second = kMasked;                         // best table other than the own one (read before the partner's next write)
+      if (can_record && record && hf == 0) second = fmaxf(ex_own[0], ex_oth[0]);
       float lnew = single ? gp.LMN1 : gp.LMN0;
       for (int v = 0; with_new && v < V; ++v) {
         const float mo = ex_oth[(2 * v) * kTileRows], so = ex_oth[(2 * v + 1) * kTileRows];
@@ -877,6 +944,16 @@ __global__ void __launch_bounds__(kThreads, 1) k_draw_tc(const Ctx c, const __gr
       }   // (full path)
       if (hf == 0) {
         if (c.blk_count > 1 && (int)((c.row_offset + rowc) % c.blk_count) != c.blk_index) choice = t0;   // not this pass's block
+        if (can_record && record && live) {
+          // The row's margin: its own table's lead over the best other, less this sweep's bound (drift since the reference,
+          // evaluation error), rounded down.  Only where the draw is provably the own table (the shortcut's condition).
+          float m = kMasked;
+          if (sure && choice == t0) {
+            const float* kq = reinterpret_cast<const float*>(s_misc + 6);
+            m = __fsub_rd(__fsub_rd(M, second), screen_row_bound(kq, xxv, V));
+          }
+          c.margin[row] = m;
+        }
         if (live) {
           c.choice[row] = choice;
           if (dbg_rows) { c.dbg_choice[row] = choice; c.dbg_lnew[row] = lnew; }

@@ -96,6 +96,8 @@ def lib():
         L.mvg_sweep.argtypes = [H, C.c_int32, C.c_int32]
         L.mvg_hyper_step.argtypes = [H]
         L.mvg_set_sweep_blocks.argtypes = [H, C.c_int32]
+        L.mvg_set_draw_screen.argtypes = [H, C.c_int32]
+        L.mvg_get_draw_screen_stats.argtypes = [H, C.POINTER(C.c_int32), C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
         L.mvg_set_stats_mode.argtypes = [H, C.c_int32, C.c_int32]
         L.mvg_hyper_step_parts.argtypes = [H, C.c_int32]
         L.mvg_sync.argtypes = [H]
@@ -355,6 +357,17 @@ class Sampler:
     def set_sweep_blocks(self, blocks):
         """One sweep = `blocks` passes over row blocks with the statistics refreshed in between (1 = synchronous)."""
         self._ck(self.L.mvg_set_sweep_blocks(self.h, int(blocks)))
+
+    def set_draw_screen(self, on):
+        """Exact draw screening on the tensor-core engines (on by default): rows whose draw is provably their own table
+        skip the likelihood.  The chain is the same either way."""
+        self._ck(self.L.mvg_set_draw_screen(self.h, 1 if on else 0))
+
+    def draw_screen_stats(self):
+        """{'enabled', 'rows_screened', 'tiles_evaluated'} of the most recent draw (tiles of 128 rows)."""
+        en, rows, tiles = C.c_int32(0), C.c_int64(0), C.c_int64(0)
+        self._ck(self.L.mvg_get_draw_screen_stats(self.h, C.byref(en), C.byref(rows), C.byref(tiles)))
+        return {"enabled": bool(en.value), "rows_screened": rows.value, "tiles_evaluated": tiles.value}
 
     def hyper_step(self):
         self._ck(self.L.mvg_hyper_step(self.h))
