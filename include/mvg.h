@@ -251,6 +251,27 @@ typedef struct mvg_params_host {
   float* m;     /* [cap*Dsum]: per view a [cap][D_v] block of per-table means, views concatenated */
 } mvg_params_host;
 int mvg_get_params(mvg_handle* h, const mvg_params_host* out);
+/* Draw screening (tensor-core engines, DESIGN.md §4.1.1): what the most recent draw's screening decided and what it left
+ * behind, read without changing it.  mode is that of the most recent screened draw (0 off, 1 refresh, 2 skip) and sweep the
+ * sweep it belongs to: after a replayed sweep that is the next sweep's draw, already issued (mvg_get_state's sweep); after a
+ * sweep launched directly, the sweep before.  valid / ref_sweep: whether a reference stands and the sweep it was taken at.
+ * k: the coefficients of the row bound that draw used (k0, kA[3], kB[3]; not written by a draw in off mode).  n_eval and
+ * tiles: the tile list of a skip draw (first n_eval entries meaningful).  margin: the per-row margins as they stand.  ref:
+ * the reference parameter block (dish, A, C, A1, C1, lone, LM, LM1 filled; the other pointers are ignored) and ref_b its
+ * [2][cap*Dsum] mean_hi, mean_lo.  Host buffers; NULL skips.  Synchronises; MVG_ESTATE on a handle without screening
+ * state (CUDA-core engine, or before the first state call).  For tests: nothing here is needed to run a chain. */
+typedef struct mvg_screen_host {
+  int32_t mode;
+  uint32_t sweep;
+  uint32_t valid, ref_sweep;
+  float k[7];
+  int32_t n_eval;
+  int32_t* tiles;      /* [ceil(n_rows/128)] */
+  float* margin;       /* [n_rows] */
+  mvg_params_host ref;
+  float* ref_b;        /* [2][cap*Dsum] */
+} mvg_screen_host;
+int mvg_get_draw_screen_record(mvg_handle* h, mvg_screen_host* out);
 /* With debug_export: per-row stage-A outputs of the LAST sweep: acc [n_rows][V][cap] dot products
  * x.m and xx [n_rows][V] squared norms, plus the raw draw (before births are seated) [n_rows].  A count view: acc is
  * log2 f under each table's dish and xx what the new-dish term read, the token total (plug-in) or -log2 f_new

@@ -902,6 +902,45 @@ int mvg_get_draw_screen_stats(mvg_handle* h, int32_t* enabled, int64_t* rows_scr
   return MVG_OK;
 }
 
+int mvg_get_draw_screen_record(mvg_handle* h, mvg_screen_host* o) {
+  if (!h || !o) return MVG_EINVAL;
+  const Ctx& c = h->c;
+  if (!c.scr) return fail(h, MVG_ESTATE, "no draw screening state (tensor-core engines, after the first state call)");
+  MVG_CUDA(h, cudaSetDevice(h->cfg.device));
+  const size_t vc = (size_t)c.V * c.cap;
+  ScreenRec r;
+  std::vector<TableParam> tp(vc);
+  std::vector<TableMass> tm(c.cap);
+  MVG_CUDA(h, cudaMemcpyAsync(&r, c.scr, sizeof(r), cudaMemcpyDeviceToHost, h->stream));
+  MVG_CUDA(h, cudaMemcpyAsync(tp.data(), c.scr_tp, sizeof(TableParam) * vc, cudaMemcpyDeviceToHost, h->stream));
+  MVG_CUDA(h, cudaMemcpyAsync(tm.data(), c.scr_tm, sizeof(TableMass) * c.cap, cudaMemcpyDeviceToHost, h->stream));
+  if (o->tiles)
+    MVG_CUDA(h, cudaMemcpyAsync(o->tiles, c.scr_tiles, sizeof(int32_t) * (size_t)((c.n_rows + 127) / 128), cudaMemcpyDeviceToHost, h->stream));
+  if (o->margin) MVG_CUDA(h, cudaMemcpyAsync(o->margin, c.margin, sizeof(float) * (size_t)c.n_rows, cudaMemcpyDeviceToHost, h->stream));
+  if (o->ref_b) MVG_CUDA(h, cudaMemcpyAsync(o->ref_b, c.scr_b, sizeof(float) * 2 * (size_t)c.cap * c.Dsum, cudaMemcpyDeviceToHost, h->stream));
+  MVG_CUDA(h, cudaStreamSynchronize(h->stream));
+  o->mode = r.mode;
+  o->sweep = r.sweep;
+  o->valid = r.valid;
+  o->ref_sweep = r.ref_sweep;
+  for (int i = 0; i < 7; ++i) o->k[i] = r.k[i];
+  o->n_eval = r.n_eval;
+  const mvg_params_host& p = o->ref;
+  for (size_t i = 0; i < vc; ++i) {
+    if (p.dish) p.dish[i] = tp[i].dish;
+    if (p.A) p.A[i] = tp[i].A;
+    if (p.C) p.C[i] = tp[i].C;
+    if (p.A1) p.A1[i] = tp[i].A1;
+    if (p.C1) p.C1[i] = tp[i].C1;
+    if (p.lone) p.lone[i] = tp[i].lone;
+  }
+  for (int t = 0; t < c.cap; ++t) {
+    if (p.LM) p.LM[t] = tm[t].LM;
+    if (p.LM1) p.LM1[t] = tm[t].LM1;
+  }
+  return MVG_OK;
+}
+
 int mvg_hyper_step_parts(mvg_handle* h, int32_t parts) {
   if (!h) return MVG_EINVAL;
   if (!h->state_ready) return fail(h, MVG_ESTATE, "no state yet");

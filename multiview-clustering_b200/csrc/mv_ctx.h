@@ -140,7 +140,7 @@ struct Ctx {
 };
 
 // What k_draw_screen hands to k_draw_tc, and the reference the margins are measured against.  Written by k_draw_screen:
-// mode, k, n_eval, last_*; by k_draw_tc (CTA 0, after it has waited for the screening kernel): valid, ref_sweep.
+// mode, sweep, k, n_eval, last_*; by k_draw_tc (CTA 0, after it has waited for the screening kernel): valid, ref_sweep.
 enum { kScreenOff = 0, kScreenRefresh = 1, kScreenSkip = 2 };
 constexpr int kScreenPeriod = 64;      // sweeps between two full evaluations (new reference)
 struct ScreenRec {
@@ -149,6 +149,7 @@ struct ScreenRec {
   float k[1 + 2 * 3];       // row bound Q = k0 + sum_v kA_v |x_v|^2 + kB_v |x_v|: drift since the reference + evaluation error
   uint32_t valid;           // the reference parameters and the margins stand for the current seating
   uint32_t ref_sweep;
+  uint32_t sweep;           // the sweep the most recent draw belongs to (mvg_get_draw_screen_record pairs it with its parameters)
   uint32_t cnt, done, rows; // scratch of one screening launch (tile counter, CTAs finished, rows screened), zero between launches
   int64_t last_rows_screened, last_tiles_evaluated;
 };

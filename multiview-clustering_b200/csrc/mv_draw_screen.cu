@@ -72,6 +72,7 @@ __global__ void __launch_bounds__(kScrThreads) k_draw_screen(const Ctx c) {
   if (chg) atomicOr(&s_flags, 2);
   __syncthreads();
   const int mode = (s_flags & 1) ? kScreenOff : ((s_flags & 2) ? kScreenRefresh : kScreenSkip);
+  if (blockIdx.x == 0 && tid == 0) R->sweep = g.sweep;
   if (mode == kScreenOff) {
     if (blockIdx.x == 0 && tid == 0) { R->mode = mode; R->last_rows_screened = 0; R->last_tiles_evaluated = n_tiles; }
     return;

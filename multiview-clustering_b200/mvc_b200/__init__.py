@@ -62,6 +62,14 @@ class _ParamsHost(C.Structure):
     ]
 
 
+class _ScreenHost(C.Structure):
+    _fields_ = [
+        ("mode", C.c_int32), ("sweep", C.c_uint32), ("valid", C.c_uint32), ("ref_sweep", C.c_uint32),
+        ("k", C.c_float * 7), ("n_eval", C.c_int32), ("tiles", _i32p), ("margin", _f32p), ("ref", _ParamsHost),
+        ("ref_b", _f32p),
+    ]
+
+
 _lib = None
 
 
@@ -98,6 +106,7 @@ def lib():
         L.mvg_set_sweep_blocks.argtypes = [H, C.c_int32]
         L.mvg_set_draw_screen.argtypes = [H, C.c_int32]
         L.mvg_get_draw_screen_stats.argtypes = [H, C.POINTER(C.c_int32), C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
+        L.mvg_get_draw_screen_record.argtypes = [H, C.POINTER(_ScreenHost)]
         L.mvg_set_stats_mode.argtypes = [H, C.c_int32, C.c_int32]
         L.mvg_hyper_step_parts.argtypes = [H, C.c_int32]
         L.mvg_sync.argtypes = [H]
@@ -368,6 +377,26 @@ class Sampler:
         en, rows, tiles = C.c_int32(0), C.c_int64(0), C.c_int64(0)
         self._ck(self.L.mvg_get_draw_screen_stats(self.h, C.byref(en), C.byref(rows), C.byref(tiles)))
         return {"enabled": bool(en.value), "rows_screened": rows.value, "tiles_evaluated": tiles.value}
+
+    def get_draw_screen_record(self):
+        """What the most recent screened draw decided and left behind (mvg_get_draw_screen_record): 'mode' (0 off,
+        1 refresh, 2 skip), 'sweep' it belongs to, 'valid', 'ref_sweep', 'k' [7], 'n_eval', 'tiles', 'margin' [n_rows],
+        'ref' (dish, A, C, A1, C1, lone [V, cap]; LM, LM1 [cap]) and 'ref_b' [2, cap*Dsum] (mean_hi, mean_lo)."""
+        V, cap = self.V, self.cap
+        ref = {"dish": np.empty((V, cap), np.int32), "A": np.empty((V, cap), np.float32), "C": np.empty((V, cap), np.float32),
+               "A1": np.empty((V, cap), np.float32), "C1": np.empty((V, cap), np.float32),
+               "lone": np.empty((V, cap), np.int32), "LM": np.empty(cap, np.float32), "LM1": np.empty(cap, np.float32)}
+        tiles = np.empty((self.n_rows + 127) // 128, np.int32)
+        margin = np.empty(self.n_rows, np.float32)
+        ref_b = np.empty((2, cap * self.Dsum), np.float32)
+        s = _ScreenHost()
+        for k, a in ref.items():
+            setattr(s.ref, k, _p(a, _i32p if a.dtype == np.int32 else _f32p))
+        s.tiles, s.margin, s.ref_b = _p(tiles, _i32p), _p(margin, _f32p), _p(ref_b, _f32p)
+        self._ck(self.L.mvg_get_draw_screen_record(self.h, C.byref(s)))
+        return {"mode": s.mode, "sweep": s.sweep, "valid": s.valid, "ref_sweep": s.ref_sweep,
+                "k": np.array(s.k[:], np.float32), "n_eval": s.n_eval, "tiles": tiles, "margin": margin, "ref": ref,
+                "ref_b": ref_b}
 
     def hyper_step(self):
         self._ck(self.L.mvg_hyper_step(self.h))
