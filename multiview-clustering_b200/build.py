@@ -11,7 +11,7 @@ from pathlib import Path
 HERE = Path(__file__).resolve().parent
 CSRC = HERE / "csrc"
 OUT = HERE / "mvc_b200" / "libmvg_b200.so"
-SOURCES = ["mv_capi.cu", "mv_draw_simt.cu", "mv_draw_tc.cu", "mv_draw_screen.cu", "mv_state_kernels.cu", "mv_stats_tile.cu", "mv_summary.cu", "mv_counts.cu", "mv_exchange.cu", "mv_seq.cu"]
+SOURCES = ["mv_capi.cu", "mv_draw_simt.cu", "mv_draw_tc.cu", "mv_state_kernels.cu", "mv_stats_tile.cu", "mv_summary.cu", "mv_counts.cu", "mv_exchange.cu", "mv_seq.cu"]
 # per-file overrides: the sequential engine must not contract a*b+c (the compiled reference does not either)
 EXTRA = {"mv_seq.cu": ["--fmad=false"]}
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")

@@ -144,6 +144,8 @@ int dev_alloc(mvg_handle* h, T** p, size_t count) {
 
 int align16(int x) { return (x + 15) & ~15; }
 
+float* xx_tmax_of(const Ctx& c, int v) { return c.xx_tmax + (size_t)v * ((c.n_rows + 127) / 128); }
+
 // Allocate everything that depends on the dims of all views; called once they are all known.
 int ensure_layout(mvg_handle* h) {
   if (h->layout_done) return MVG_OK;
@@ -216,10 +218,13 @@ int ensure_layout(mvg_handle* h) {
     if (posix_memalign(&h->tc_maps, 128, draw_tc_maps_bytes()) != 0) return fail(h, MVG_ENOMEM, "tensor map allocation");
     cudaError_t e = draw_tc_make_maps(c, h->tc_maps);
     if (e != cudaSuccess) return fail(h, MVG_ECUDA, std::string("cuTensorMapEncodeTiled: ") + cudaGetErrorString(e));
-    // draw screening (DESIGN.md §4.1.1): the verdict record, the reference parameters, a margin per row, the tile list
+    // draw screening (DESIGN.md §4.1.1): the verdict record, the reference parameters, a margin per row and its minimum
+    // per 32 rows, the tile lists, k_finalize's drift sums
     if ((rc = dev_alloc(h, &c.scr, 1)) != MVG_OK || (rc = dev_alloc(h, &c.scr_tp, V * cap)) != MVG_OK ||
         (rc = dev_alloc(h, &c.scr_tm, cap)) != MVG_OK || (rc = dev_alloc(h, &c.scr_b, 2 * cap * dsum)) != MVG_OK ||
-        (rc = dev_alloc(h, &c.margin, N)) != MVG_OK || (rc = dev_alloc(h, &c.scr_tiles, (N + 127) / 128)) != MVG_OK)
+        (rc = dev_alloc(h, &c.margin, N)) != MVG_OK || (rc = dev_alloc(h, &c.margin_min, (N + 31) / 32)) != MVG_OK ||
+        (rc = dev_alloc(h, &c.scr_tiles, (N + 127) / 128)) != MVG_OK || (rc = dev_alloc(h, &c.scr_work, (N + 127) / 128)) != MVG_OK ||
+        (rc = dev_alloc(h, &c.scr_sum, 3 * V * cap)) != MVG_OK)
       return rc;
     c.screen = (h->screen_want && !c.debug_export) ? 1 : 0;   // debug handles export what the full path computed
   }
@@ -293,10 +298,6 @@ int prepare_count_model(mvg_handle* h) {
 
 int launch_draw(mvg_handle* h, bool programmatic = false) {
   if (h->engine == MVG_ENGINE_TCGEN05 || h->engine == MVG_ENGINE_TCGEN05_FAST) {
-    if (h->c.screen) {                 // the screening kernel takes the draw's place in the programmatic chain
-      MVG_CUDA(h, launch_draw_screen(h->c, programmatic, h->stream));
-      h->launches += 1;
-    }
     MVG_CUDA(h, launch_draw_tc(h->c, h->tc_maps, h->engine == MVG_ENGINE_TCGEN05_FAST, programmatic, h->stream));
   } else {
     MVG_CUDA(h, launch_draw_simt(h->c, h->stream));
@@ -385,6 +386,13 @@ int mvg_create(const mvg_config* cfg, mvg_handle** out) {
     }
     h->owned.push_back(q);
     c.xx = static_cast<float*>(q);
+    const size_t tiles = (size_t)(c.n_rows + 127) / 128 * xx_rows;
+    if (cudaMalloc(&q, sizeof(float) * tiles) != cudaSuccess || cudaMemset(q, 0, sizeof(float) * tiles) != cudaSuccess) {
+      mvg_destroy(h);
+      return fail(nullptr, MVG_ENOMEM, "cudaMalloc: squared norms");
+    }
+    h->owned.push_back(q);
+    c.xx_tmax = static_cast<float*>(q);
   }
   if (c.world > 1) {                               // the sticky exchange fault, mirrored where the host reads it without a sync
     void* hp = nullptr;
@@ -451,7 +459,7 @@ int mvg_upload_view_f32(mvg_handle* h, int32_t v, const float* x_host, int32_t d
   h->c.x[v] = static_cast<const float*>(h->view_owned[v]);
   h->c.D[v] = dim;
   h->c.kind[v] = 0;
-  MVG_CUDA(h, launch_rownorms(h->c.x[v], h->c.xx + (size_t)v * h->c.xx_stride, h->c.n_rows, dim, h->stream));
+  MVG_CUDA(h, launch_rownorms(h->c.x[v], h->c.xx + (size_t)v * h->c.xx_stride, xx_tmax_of(h->c, v), h->c.n_rows, dim, h->stream));
   h->launches += 1;
   return MVG_OK;
 }
@@ -476,7 +484,7 @@ int mvg_upload_view_f64(mvg_handle* h, int32_t v, const double* y_host, int32_t 
   h->launches += 1;
   h->c.x[v] = static_cast<const float*>(h->view_owned[v]);
   h->c.D[v] = dim;
-  MVG_CUDA(h, launch_rownorms(h->c.x[v], h->c.xx + (size_t)v * h->c.xx_stride, h->c.n_rows, dim, h->stream));
+  MVG_CUDA(h, launch_rownorms(h->c.x[v], h->c.xx + (size_t)v * h->c.xx_stride, xx_tmax_of(h->c, v), h->c.n_rows, dim, h->stream));
   h->launches += 1;
   return MVG_OK;
 }
@@ -488,7 +496,7 @@ int mvg_attach_view_device_f32(mvg_handle* h, int32_t v, const float* x_dev, int
   if (h->view_owned[v]) { cudaFree(h->view_owned[v]); h->view_owned[v] = nullptr; }
   h->c.x[v] = x_dev;
   h->c.D[v] = dim;
-  MVG_CUDA(h, launch_rownorms(x_dev, h->c.xx + (size_t)v * h->c.xx_stride, h->c.n_rows, dim, h->stream));
+  MVG_CUDA(h, launch_rownorms(x_dev, h->c.xx + (size_t)v * h->c.xx_stride, xx_tmax_of(h->c, v), h->c.n_rows, dim, h->stream));
   h->launches += 1;
   return MVG_OK;
 }

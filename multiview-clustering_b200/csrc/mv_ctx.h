@@ -73,6 +73,7 @@ struct Ctx {
   int32_t* table_prev;         // [N] count views: the table every row's words are currently counted at in cnt_t
   float* xx;                // [V][xx_stride] squared norms of the rows (count views: the rows' total counts), computed once per upload
   int64_t xx_stride;        // n_rows rounded up to a multiple of 4
+  float* xx_tmax;           // [V][ceil(N/128)] largest xx of each tile of 128 rows (a NaN counts as +inf): draw screening
 
   int32_t* table_cur;
   int32_t* choice;
@@ -130,17 +131,20 @@ struct Ctx {
   long long* dbg_prof;      // [CTAs][16] cycles spent waiting per role of the tcgen05 kernel (debug_export & 2)
 
   // draw screening (tensor-core engine, DESIGN.md §4.1.1): rows whose draw is provably their own table skip the draw
-  int32_t screen;           // k_draw_screen runs before every draw of this handle
-  struct ScreenRec* scr;    // [1] the screening kernel's verdict for the draw that follows, and the reference sweep
+  int32_t screen;           // k_draw_tc screens its tiles in every draw of this handle
+  struct ScreenRec* scr;    // [1] the verdict of the most recent draw, and the reference sweep
   TableParam* scr_tp;       // [V][cap] parameter block of the reference sweep
   TableMass* scr_tm;        // [cap]
   float* scr_b;             // [2][cap*Dsum] its mean_hi, mean_lo
   float* margin;            // [N] lower bound on (own-table log2 weight - best other) at the reference, see ScreenRec
   int32_t* scr_tiles;       // [ceil(N/128)] row tiles the draw evaluates (mode kScreenSkip)
+  float* margin_min;        // [n_chunks] least margin of each 32 rows (a NaN counts as -inf), written with the margins
+  double* scr_sum;          // [V][cap][3] per table, from k_finalize: |b|^2, |b - b_ref|^2, |R b - R_ref b_ref|^2 (b = hi + lo)
+  int32_t* scr_work;        // [ceil(N/128)] each CTA's tiles to evaluate (mode kScreenSkip), at blockIdx.x + j * gridDim.x
 };
 
-// What k_draw_screen hands to k_draw_tc, and the reference the margins are measured against.  Written by k_draw_screen:
-// mode, sweep, k, n_eval, last_*; by k_draw_tc (CTA 0, after it has waited for the screening kernel): valid, ref_sweep.
+// What the screening of the most recent draw decided, and the reference the margins are measured against.  Written by
+// k_draw_tc: mode, sweep, k (CTA 0); n_eval, last_*, and in a refresh valid and ref_sweep (the last CTA to decide).
 enum { kScreenOff = 0, kScreenRefresh = 1, kScreenSkip = 2 };
 constexpr int kScreenPeriod = 64;      // sweeps between two full evaluations (new reference)
 struct ScreenRec {
@@ -150,11 +154,11 @@ struct ScreenRec {
   uint32_t valid;           // the reference parameters and the margins stand for the current seating
   uint32_t ref_sweep;
   uint32_t sweep;           // the sweep the most recent draw belongs to (mvg_get_draw_screen_record pairs it with its parameters)
-  uint32_t cnt, done, rows; // scratch of one screening launch (tile counter, CTAs finished, rows screened), zero between launches
+  uint32_t cnt, done, rows; // scratch of one draw (tile counter, CTAs decided, rows screened), zero between launches
   int64_t last_rows_screened, last_tiles_evaluated;
 };
 #ifdef __CUDACC__
-// The row's bound, rounded upward: k_draw_tc subtracts it when it records a margin, k_draw_screen when it tests one.
+// The row's bound, rounded upward: k_draw_tc subtracts it when it records a margin and when it tests one.
 __device__ __forceinline__ float screen_row_bound(const float* k, const float* xx, int V) {
   float q = k[0];
   for (int v = 0; v < V; ++v) {
@@ -237,7 +241,6 @@ cudaError_t launch_draw_tc(const Ctx& c, const void* maps, bool fast_exp, bool p
 bool draw_tc_supported(const Ctx& c);
 size_t draw_tc_maps_bytes();                                   // host blob holding the TMA tensor maps
 cudaError_t draw_tc_make_maps(const Ctx& c, void* maps_out);  // (re)encode them for the current pointers
-cudaError_t launch_draw_screen(const Ctx& c, bool programmatic, cudaStream_t s);   // before launch_draw_tc when c.screen
 cudaError_t launch_pack(const Ctx& c, cudaStream_t s);
 // delta: only the rows that moved this sweep are visited; the per-CTA partials then hold the CHANGE of the statistics
 // (rows that arrived minus rows that left) and k_reduce_x adds it to the shard's running sums (mode flag there).
@@ -248,7 +251,7 @@ cudaError_t launch_stats_tile(const Ctx& c, bool delta, cudaStream_t s);
 cudaError_t launch_reduce_x(const Ctx& c, int mode, bool delta, const XchgPeers& peers, unsigned char* recv_local, cudaStream_t s);
 cudaError_t launch_finalize(const Ctx& c, int32_t flags, cudaStream_t s);
 cudaError_t launch_init_tables(const Ctx& c, int32_t mode, cudaStream_t s);
-cudaError_t launch_rownorms(const float* x, float* xx, int n, int D, cudaStream_t s);
+cudaError_t launch_rownorms(const float* x, float* xx, float* xx_tmax, int n, int D, cudaStream_t s);
 cudaError_t launch_f64_to_f32(const double* src, float* dst, int64_t n, cudaStream_t s);
 int stats_smem_bytes(const Ctx& c);
 // count views (mv_counts.cu)

@@ -41,6 +41,7 @@
 #include <cuda.h>
 
 #include "mv_ctx.h"
+#include "mv_draw_screen.cuh"
 
 namespace mv {
 
@@ -80,11 +81,12 @@ struct SmemLayout {
   static constexpr int same_off = dlm_off + 64 * (int)sizeof(float);                        // u64[V][64]: same-dish table masks
   static constexpr int ex_off = same_off + kMaxTcViews * 64 * 8;
   static constexpr int bar_off = ex_off + 4 * kExFields * kTileRows * (int)sizeof(float);   // ex: [pair][half][field][row]
-  static constexpr int n_bars = 2 * kRawStages + 2 * kLoStages + 2 * kDStages + 1;
+  static constexpr int n_bars = 2 * kRawStages + 2 * kLoStages + 2 * kDStages + 2;
   static constexpr int misc_off = bar_off + n_bars * 8;
   static constexpr int total = misc_off + 64;
 };
 static_assert(SmemLayout::total <= 227 * 1024, "shared memory budget");
+static_assert(sizeof(screen::Scratch) <= 4 * kExFields * kTileRows * sizeof(float), "screening scratch in the exchange area");
 
 // ---- PTX helpers ----------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -335,7 +337,8 @@ __global__ void __launch_bounds__(kThreads, 1) k_draw_tc(const Ctx c, const __gr
   ViewParam* s_vp = reinterpret_cast<ViewParam*>(smem + SmemLayout::vp_off);
   float* s_lm = reinterpret_cast<float*>(smem + SmemLayout::lm_off);
   uint32_t* s_misc = reinterpret_cast<uint32_t*>(smem + SmemLayout::misc_off);   // [0] TMEM base, [1] sweep, [2..3] GlobalParam floats,
-                                                                                 // [4] all_lone, [5] screening mode, [6..12] its bound coefficients
+                                                                                 // [4] all_lone, [5] screening mode, [6..12] its bound coefficients,
+                                                                                 // [13] tiles of this CTA on the screening list
 
   // barrier addresses
   const uint32_t bar0 = sbase + SmemLayout::bar_off;
@@ -346,6 +349,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_draw_tc(const Ctx c, const __gr
   auto d_full = [&](int s) { return bar0 + 8u * (2 * kRawStages + 2 * kLoStages + s); };
   auto d_empty = [&](int s) { return bar0 + 8u * (2 * kRawStages + 2 * kLoStages + kDStages + s); };
   const uint32_t b_full = bar0 + 8u * (2 * kRawStages + 2 * kLoStages + 2 * kDStages);
+  const uint32_t list_full = b_full + 8u;            // the screening verdict and this CTA's tile list are in place
 
   // ---- one-time setup --------------------------------------------------------------------------
   // Nothing here depends on the previous kernels of the sweep: with a programmatic launch it runs — like the first
@@ -361,6 +365,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_draw_tc(const Ctx c, const __gr
     // (arrivals are per WARP — one lane after __syncwarp — not per thread: a waiter sleeping on the barrier is woken by every
     //  arrival, and 256 wake-ups per phase cost the epilogue's schedulers issue slots)
     mbar_init(b_full, 1);
+    mbar_init(list_full, 1);
     fence_barrier_init();
   }
   if (warp == 1) {   // TMEM allocation: one warp, address published through shared memory
@@ -373,15 +378,16 @@ __global__ void __launch_bounds__(kThreads, 1) k_draw_tc(const Ctx c, const __gr
   const uint32_t tmem_base = s_misc[0];
 
   const int n_tiles = (c.n_rows + kTileRows - 1) / kTileRows;
-  // The tiles this launch evaluates: all of them, or the list of k_draw_screen (DESIGN.md §4.1.1), which then exists only
-  // once this grid's dependency has resolved.  Every role walks the same sequence k = blockIdx.x, + gridDim.x, ...
+  // The tiles this launch evaluates: all of them, or those of its own tiles that the screening of the epilogue warpgroups
+  // (DESIGN.md §4.1.1) could not settle, listed at scr_work[blockIdx.x + j * gridDim.x], j < s_misc[13].  Every role walks
+  // the same sequence k = blockIdx.x, + gridDim.x, ... below the returned bound.
   auto work_list = [&](const int*& list) -> int {
     list = nullptr;
     if (!c.screen) return n_tiles;
-    grid_dependency_wait();
-    if (c.scr->mode != kScreenSkip) return n_tiles;
-    list = c.scr_tiles;
-    return c.scr->n_eval;
+    mbar_wait(list_full, 0);
+    if (s_misc[5] != (uint32_t)kScreenSkip) return n_tiles;
+    list = c.scr_work;
+    return (int)blockIdx.x + (int)s_misc[13] * (int)gridDim.x;
   };
   const bool prof = DEBUG && (c.debug_export & 2) != 0 && c.dbg_prof != nullptr;
   const bool dbg_rows = DEBUG && (c.debug_export & 1) != 0;
@@ -598,37 +604,23 @@ __global__ void __launch_bounds__(kThreads, 1) k_draw_tc(const Ctx c, const __gr
         s_misc[3] = __float_as_uint(g.LMN1);
       }
       if (c.screen) {
-        // The screening verdict of this sweep.  A refresh makes this sweep's parameters the reference of the margins every
-        // row records below (the CTAs copy a slice each; nothing reads the copy before the next screening launch); a sweep
-        // that does not screen leaves no valid reference behind.
-        const int mode = c.scr->mode;
+        // The screening verdict of this sweep, its bound coefficients and, in a skip sweep, this CTA's list
+        const int mode = screen::run(c, et, reinterpret_cast<screen::Scratch*>(smem + SmemLayout::ex_off),
+                                     reinterpret_cast<float*>(s_misc + 6), s_misc + 13);
         if (et == 0) s_misc[5] = (uint32_t)mode;
-        if (et < 7) s_misc[6 + et] = __float_as_uint(c.scr->k[et]);
-        if (mode == kScreenRefresh) {
-          const int nb = c.cap * c.Dsum;
-          for (int i = blockIdx.x * 512 + et; i < 2 * nb + V * 64 + 64; i += gridDim.x * 512) {
-            if (i < nb) c.scr_b[i] = c.mean_hi[i];
-            else if (i < 2 * nb) c.scr_b[i] = c.mean_lo[i - nb];
-            else if (i < 2 * nb + V * 64) c.scr_tp[i - 2 * nb] = c.tparam[i - 2 * nb];
-            else c.scr_tm[i - 2 * nb - V * 64] = c.tmass[i - 2 * nb - V * 64];
-          }
-        }
-        if (blockIdx.x == 0 && et == 0) {
-          if (mode == kScreenRefresh) { c.scr->ref_sweep = c.gparam->sweep; c.scr->valid = 1u; }
-          else if (mode == kScreenOff) c.scr->valid = 0u;
-        }
       } else if (et == 0) {
         s_misc[5] = (uint32_t)kScreenOff;
       }
       if (!lone_ok) atomicAnd(&s_misc[4], 0u);
       asm volatile("bar.sync 9, 512;" ::: "memory");    // the epilogue warpgroups only: the other roles never read these
+      if (c.screen && et == 0) mbar_arrive(list_full);  // ... except the verdict and the list, which they wait for
     }
     const uint32_t sweep = s_misc[1];
     GlobalParam gp;
     gp.LMN0 = __uint_as_float(s_misc[2]);
     gp.LMN1 = __uint_as_float(s_misc[3]);
     const bool all_lone_rt = s_misc[4] != 0u;
-    const bool record_rt = s_misc[5] != (uint32_t)kScreenOff;   // then with_new is off and all_lone on (k_draw_screen's precondition)
+    const bool record_rt = s_misc[5] != (uint32_t)kScreenOff;   // then with_new is off and all_lone on (screening's precondition)
     const int* list;
     const int n_work = work_list(list);
     // Two CTA-uniform properties of the sweep select one of four copies of the loop, so that the registers and the code of
@@ -944,7 +936,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_draw_tc(const Ctx c, const __gr
       }   // (full path)
       if (hf == 0) {
         if (c.blk_count > 1 && (int)((c.row_offset + rowc) % c.blk_count) != c.blk_index) choice = t0;   // not this pass's block
-        if (can_record && record && live) {
+        if (can_record && record) {
           // The row's margin: its own table's lead over the best other, less this sweep's bound (drift since the reference,
           // evaluation error), rounded down.  Only where the draw is provably the own table (the shortcut's condition).
           float m = kMasked;
@@ -952,7 +944,12 @@ __global__ void __launch_bounds__(kThreads, 1) k_draw_tc(const Ctx c, const __gr
             const float* kq = reinterpret_cast<const float*>(s_misc + 6);
             m = __fsub_rd(__fsub_rd(M, second), screen_row_bound(kq, xxv, V));
           }
-          c.margin[row] = m;
+          if (live) c.margin[row] = m;
+          // and the least margin of these 32 rows, for the tile test of later sweeps (a NaN margin counts as -inf)
+          float mn = live ? ((m == m) ? m : -INFINITY) : INFINITY;
+#pragma unroll
+          for (int o = 16; o > 0; o >>= 1) mn = fminf(mn, __shfl_xor_sync(0xffffffffu, mn, o));
+          if (lane == 0 && (row >> 5) < c.n_chunks) c.margin_min[row >> 5] = mn;
         }
         if (live) {
           c.choice[row] = choice;

@@ -1129,6 +1129,23 @@ __global__ void __launch_bounds__(kFinThreads, 1) k_finalize(const Ctx c, const 
         else mask.clear();
         const int t1 = mask.lowest();
         const Set more = mask.without_lowest();
+        // Draw screening (DESIGN.md §4.1.1) bounds the drift of the scaled means b = hi + lo since its reference sweep from
+        // three sums per table, formed here in FP64 by the same lanes and shuffle tree as |m|^2: |b|^2, |b - b_ref|^2 and
+        // |R b - R_ref b_ref|^2 (R = A1 / A as k_draw_tc rounds it; A1 as in the parameter block below).
+        const bool scr = c.scr_sum != nullptr && c.mean_hi != nullptr;
+        double rq = 0.0, rp = 0.0;
+        if (scr) {
+          float A1_f = 0.f;
+          if (k >= 0 && !is_count && (double)S.n_vk[k] >= 2.0) {
+            const double tau = tau_l, n = (double)S.n_vk[k];
+            A1_f = (float)(kLog2e * ((tau + n) / (2.0 * tau * (tau + n - 1.0))));
+          }
+          const TableParam p = c.scr_tp[v * cap + t];
+          rq = (A_f != 0.0f) ? (double)__fdiv_rn(A1_f, A_f) : 0.0;
+          rp = (p.A != 0.0f) ? (double)__fdiv_rn(p.A1, p.A) : 0.0;
+        }
+        const size_t half = (size_t)cap * c.Dsum;
+        double sb = 0.0, sd = 0.0, sr = 0.0;
         double mm = 0.0;
         for (int dd = lane; dd < D; dd += 32) {
           double s1 = (t1 >= 0) ? S1t[t1 * D + dd] : 0.0;
@@ -1143,12 +1160,31 @@ __global__ void __launch_bounds__(kFinThreads, 1) k_finalize(const Ctx c, const 
             asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(lb) : "f"(__fadd_rn(bm, -hi)));
             c.mean_hi[off + dd] = hi;
             c.mean_lo[off + dd] = __uint_as_float(lb);
+            if (scr) {
+              const double b = (double)hi + (double)__uint_as_float(lb);
+              const double bp = (double)c.scr_b[off + dd] + (double)c.scr_b[half + off + dd];
+              const double db = b - bp, dr = __fma_rn(b, rq, -__dmul_rn(rp, bp));
+              sb = __fma_rn(b, b, sb);
+              sd = __fma_rn(db, db, sd);
+              sr = __fma_rn(dr, dr, sr);
+            }
           }
           mm += (double)m * (double)m;
         }
 #pragma unroll
-        for (int o = 16; o > 0; o >>= 1) mm += __shfl_xor_sync(0xffffffffu, mm, o);
+        for (int o = 16; o > 0; o >>= 1) {
+          mm += __shfl_xor_sync(0xffffffffu, mm, o);
+          if (scr) {
+            sb += __shfl_xor_sync(0xffffffffu, sb, o);
+            sd += __shfl_xor_sync(0xffffffffu, sd, o);
+            sr += __shfl_xor_sync(0xffffffffu, sr, o);
+          }
+        }
         if (lane == 0) S.s1sq[t] = mm;               // (s1sq is free again: reused for |m_t|^2)
+        if (scr && lane == 0) {
+          double* o3 = c.scr_sum + 3 * ((size_t)v * cap + t);
+          o3[0] = sb; o3[1] = sd; o3[2] = sr;
+        }
       }
     }
     if (!s1_in_smem) {                               // the next launch re-reads sum_s1t; nothing to write back
@@ -1291,18 +1327,28 @@ cudaError_t launch_init_tables(const Ctx& c, int32_t mode, cudaStream_t s) {
 }
 
 // Squared norms of the rows of one view, xx[i] = sum_d x[i][d]^2 as one ascending fmaf chain (the order
-// the CUDA-core draw kernel and the CPU mirror use).  The data never change, so this runs once per upload.
-__global__ void k_rownorms(const float* __restrict__ x, float* __restrict__ xx, int n, int D) {
+// the CUDA-core draw kernel and the CPU mirror use), and the largest of each tile of 128 rows (one block), a NaN taken
+// as +inf, for the tile test of draw screening.  The data never change, so this runs once per upload.
+__global__ void __launch_bounds__(128) k_rownorms(const float* __restrict__ x, float* __restrict__ xx, float* __restrict__ xx_tmax, int n, int D) {
+  __shared__ float s_max[4];
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  const float* r = x + (size_t)i * D;
   float q = 0.0f;
-  for (int d = 0; d < D; ++d) q = __fmaf_rn(r[d], r[d], q);
-  xx[i] = q;
+  if (i < n) {
+    const float* r = x + (size_t)i * D;
+    for (int d = 0; d < D; ++d) q = __fmaf_rn(r[d], r[d], q);
+    xx[i] = q;
+  }
+  if (!xx_tmax) return;
+  float m = (q == q) ? q : INFINITY;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+  if ((threadIdx.x & 31) == 0) s_max[threadIdx.x >> 5] = m;
+  __syncthreads();
+  if (threadIdx.x == 0) xx_tmax[blockIdx.x] = fmaxf(fmaxf(s_max[0], s_max[1]), fmaxf(s_max[2], s_max[3]));
 }
-cudaError_t launch_rownorms(const float* x, float* xx, int n, int D, cudaStream_t s) {
+cudaError_t launch_rownorms(const float* x, float* xx, float* xx_tmax, int n, int D, cudaStream_t s) {
   if (n <= 0) return cudaSuccess;
-  k_rownorms<<<(n + 255) / 256, 256, 0, s>>>(x, xx, n, D);
+  k_rownorms<<<(n + 127) / 128, 128, 0, s>>>(x, xx, xx_tmax, n, D);
   return cudaGetLastError();
 }
 
