@@ -272,6 +272,10 @@ typedef struct mvg_screen_host {
   float* ref_b;        /* [2][cap*Dsum] */
 } mvg_screen_host;
 int mvg_get_draw_screen_record(mvg_handle* h, mvg_screen_host* out);
+/* Read-only: the draw's per-row buffers as the most recent sweep left them: choice [n_rows] (the draw, a seated birth -2),
+ * table_cur [n_rows] (the seating), birthmask and movedmask [ceil(n_rows/32)] (bit r of word w: row 32 w + r drew a new
+ * table / a table other than its own).  Any pointer may be NULL. */
+int mvg_get_draw_rows(mvg_handle* h, int32_t* choice, int32_t* table_cur, uint32_t* birthmask, uint32_t* movedmask);
 /* With debug_export: per-row stage-A outputs of the LAST sweep: acc [n_rows][V][cap] dot products
  * x.m and xx [n_rows][V] squared norms, plus the raw draw (before births are seated) [n_rows].  A count view: acc is
  * log2 f under each table's dish and xx what the new-dish term read, the token total (plug-in) or -log2 f_new

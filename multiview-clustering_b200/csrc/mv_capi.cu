@@ -910,6 +910,20 @@ int mvg_get_draw_screen_stats(mvg_handle* h, int32_t* enabled, int64_t* rows_scr
   return MVG_OK;
 }
 
+int mvg_get_draw_rows(mvg_handle* h, int32_t* choice, int32_t* table_cur, uint32_t* birthmask, uint32_t* movedmask) {
+  if (!h) return MVG_EINVAL;
+  const Ctx& c = h->c;
+  if (!c.choice) return fail(h, MVG_ESTATE, "no state yet");
+  MVG_CUDA(h, cudaSetDevice(h->cfg.device));
+  const size_t n = (size_t)c.n_rows, w = (size_t)c.n_chunks;
+  if (choice) MVG_CUDA(h, cudaMemcpyAsync(choice, c.choice, sizeof(int32_t) * n, cudaMemcpyDeviceToHost, h->stream));
+  if (table_cur) MVG_CUDA(h, cudaMemcpyAsync(table_cur, c.table_cur, sizeof(int32_t) * n, cudaMemcpyDeviceToHost, h->stream));
+  if (birthmask) MVG_CUDA(h, cudaMemcpyAsync(birthmask, c.birthmask, sizeof(uint32_t) * w, cudaMemcpyDeviceToHost, h->stream));
+  if (movedmask) MVG_CUDA(h, cudaMemcpyAsync(movedmask, c.movedmask, sizeof(uint32_t) * w, cudaMemcpyDeviceToHost, h->stream));
+  MVG_CUDA(h, cudaStreamSynchronize(h->stream));
+  return MVG_OK;
+}
+
 int mvg_get_draw_screen_record(mvg_handle* h, mvg_screen_host* o) {
   if (!h || !o) return MVG_EINVAL;
   const Ctx& c = h->c;

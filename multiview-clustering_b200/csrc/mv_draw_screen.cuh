@@ -8,8 +8,9 @@
 // Q_row(s) = k0 + sum_v kA_v |x_v|^2 + kB_v |x_v| bounds the change of every log-weight between the parameters of the
 // REFERENCE sweep and those of sweep s (each term counted twice: own table and best other) plus the error of the FP32 /
 // 3-pass TF32 evaluation.  In a later sweep s' the row's gap is then at least g' - Q_row(s'); if that exceeds 31 its draw
-// is t0 without reading x.  A tile of 128 rows in which every row passes is screened: it gets exactly what the draw would
-// have written (choice = t0, no birth bit, no moved bit) and is left off the list of tiles the draw evaluates.
+// is t0 without reading x.  A tile of 128 rows in which every row passes is screened: it is left off the list of tiles the
+// draw evaluates and written nothing, because what the draw would write there (choice = t0, no birth bit, no moved bit)
+// is already in place (DESIGN.md §4.1.1: a finite margin is only ever recorded beside exactly these values).
 //
 // The reference (a copy of the parameter block and the scaled means) is taken in a refresh sweep, in which every tile is
 // evaluated.  A refresh happens when no reference is valid (new handle, set_state, a sweep that did not screen), every
@@ -20,7 +21,8 @@
 // Every CTA of k_draw_tc decides the mode and the coefficients for itself, from the same inputs, and tests its own tiles
 // (blockIdx.x, + gridDim.x, ...: the tiles it would evaluate without screening).  An arrival counter finds the last CTA
 // to have decided, and only that one writes what the decision reads (the reference, its sweep and the valid flag): a CTA
-// that starts late still sees the inputs the others saw.
+// that starts late still sees the inputs the others saw.  The other roles of the CTA are released (list_full) between
+// decide() and publish(), so the arrival counter is not on their path.
 #pragma once
 #include "mv_ctx.h"
 
@@ -59,10 +61,58 @@ __device__ __forceinline__ bool tile_passes(const float* k, const float* xx_max,
   return __fsub_rd(m_min, screen_row_bound(k, xx_max, V)) > 31.0f;
 }
 
-// Run by the 512 epilogue threads (et = 0..511) once the grid dependency has resolved.  Decides the sweep's mode, writes the
-// bound coefficients to k_out[7] and, in a skip sweep, screens this CTA's tiles and lists the others at
-// c.scr_work[blockIdx.x + j * gridDim.x], j < *n_eval_out.  Returns the mode.
-__device__ int run(const Ctx& c, int et, Scratch* S, float* k_out, uint32_t* n_eval_out) {
+// What the verdict reads, per epilogue thread et: (view, table) et < V * 64, table et - 256's masses for 256 <= et < 320,
+// and the summaries of this warp's first batch of tiles (lane 4 i + j: chunk j and view j of tile i).  k_draw_tc loads it
+// in the same round as the parameters it stages, right after the grid dependency.  margin_min must not be read earlier:
+// the previous draw triggers this grid before it writes its margins.
+struct Inputs {
+  GlobalParam g;
+  uint32_t valid, ref_sweep;
+  TableParam q, p;                            // this sweep's and the reference's parameters of (view, table) et
+  double s3[3];                               // k_finalize's sums of (view, table) et
+  TableMass m, pm;                            // this sweep's and the reference's masses of table et - 256
+  float mn, xm;                               // margin_min of chunk j, xx_tmax of view j of tile i of the first batch
+};
+
+constexpr int kBatch = 8;                     // tiles a warp tests together: lane 4 i + j reads chunk j and view j of tile i
+
+__device__ __forceinline__ int batch_tile(int base, int lane) { return base + (lane >> 2) * kWarps * (int)gridDim.x; }
+
+// Lane 4 i + j's summary loads for the batch of tiles base, + kWarps * gridDim.x, ... (tiles past the end: +inf / 0).
+__device__ __forceinline__ void load_batch(const Ctx& c, int base, int lane, int n_tiles, float& mn, float& xm) {
+  const int tile = batch_tile(base, lane), j = lane & 3;
+  mn = INFINITY;
+  xm = 0.0f;
+  if (tile < n_tiles) {
+    if (tile * (kTile / 32) + j < c.n_chunks) mn = c.margin_min[tile * (kTile / 32) + j];
+    if (j < c.V) xm = c.xx_tmax[(size_t)j * n_tiles + tile];
+  }
+}
+
+__device__ __forceinline__ void load(const Ctx& c, int et, Inputs& in) {
+  const int lane = et & 31, n_tiles = (c.n_rows + kTile - 1) / kTile;
+  in.g = *c.gparam;
+  in.valid = c.scr->valid;
+  in.ref_sweep = c.scr->ref_sweep;
+  in.s3[0] = in.s3[1] = in.s3[2] = 0.0;
+  if (et < c.V * 64) {
+    in.q = c.tparam[et];
+    in.p = c.scr_tp[et];
+    const double* s3 = c.scr_sum + 3 * et;
+    in.s3[0] = s3[0]; in.s3[1] = s3[1]; in.s3[2] = s3[2];
+  } else if (et >= 256 && et < 256 + 64) {
+    in.m = c.tmass[et - 256];
+    in.pm = c.scr_tm[et - 256];
+  }
+  load_batch(c, blockIdx.x + (et >> 5) * gridDim.x, lane, n_tiles, in.mn, in.xm);
+}
+
+// Run by the 512 epilogue threads (et = 0..511) on what load() read.  Decides the sweep's mode, writes the bound
+// coefficients to k_out[7] and, in a skip sweep, tests this CTA's tiles and lists the others at
+// c.scr_work[blockIdx.x + j * gridDim.x], j < S->n_eval.  Returns the mode; the tile list is complete when it returns.
+// A screened tile is written nothing: its rows already hold choice == table_cur and its birth and moved words are zero
+// (DESIGN.md §4.1.1, the invariant of the margins).
+__device__ int decide(const Ctx& c, int et, const Inputs& in, Scratch* S, float* k_out) {
   const int warp = et >> 5, lane = et & 31;
   const int V = c.V;
   ScreenRec* R = c.scr;
@@ -75,18 +125,18 @@ __device__ int run(const Ctx& c, int et, Scratch* S, float* k_out, uint32_t* n_e
   // threads 256 + t table t's masses.  Per (view, table) k_finalize has summed |b|^2, |b - b_ref|^2, |R b - R_ref b_ref|^2.
   // Masked C1 / LM1 (a table of one customer) are left out: they are masked in the reference as well (a change
   // refreshes), and a row at such a table never records a margin (its own weight is masked).
-  const GlobalParam g = *c.gparam;
+  const GlobalParam& g = in.g;
   int off = (c.debug_export != 0 || c.blk_count != 1 || !masked(g.LMN0) || !masked(g.LMN1)) ? 1 : 0;
-  int chg = (R->valid == 0u || g.sweep - R->ref_sweep >= (uint32_t)kScreenPeriod) ? 1 : 0;
+  int chg = (in.valid == 0u || g.sweep - in.ref_sweep >= (uint32_t)kScreenPeriod) ? 1 : 0;
   double w[7] = {0, 0, 0, 0, 0, 0, 1.0};
   if (et < V * 64) {
-    const TableParam q = c.tparam[et], p = c.scr_tp[et];
+    const TableParam& q = in.q;
+    const TableParam& p = in.p;
     if (q.dish < 0 || !q.lone) off = 1;
     if (q.dish != p.dish || q.lone != p.lone || masked(q.C1) != masked(p.C1)) chg = 1;
-    const double* s3 = c.scr_sum + 3 * et;
     const bool m1 = masked(q.C1);
-    w[0] = sqrt(s3[0]);
-    w[1] = fmax(sqrt(s3[1]), sqrt(s3[2]));
+    w[0] = sqrt(in.s3[0]);
+    w[1] = fmax(sqrt(in.s3[1]), sqrt(in.s3[2]));
     w[2] = fabs((double)q.C - (double)p.C);
     if (!m1) w[2] = fmax(w[2], fabs((double)q.C1 - (double)p.C1));
     w[3] = fmax(fabs((double)q.A - (double)p.A), fabs((double)q.A1 - (double)p.A1));
@@ -95,7 +145,8 @@ __device__ int run(const Ctx& c, int et, Scratch* S, float* k_out, uint32_t* n_e
     w[5] = fmax(fabs((double)q.A), fabs((double)q.A1));
     w[6] = fmax(1.0, (double)ratio(q));
   } else if (et >= 256 && et < 256 + 64) {
-    const TableMass m = c.tmass[et - 256], p = c.scr_tm[et - 256];
+    const TableMass& m = in.m;
+    const TableMass& p = in.pm;
     if (masked(m.LM) != masked(p.LM) || masked(m.LM1) != masked(p.LM1)) chg = 1;
     w[2] = fabs((double)m.LM - (double)p.LM);
     if (!masked(m.LM1)) w[2] = fmax(w[2], fabs((double)m.LM1 - (double)p.LM1));
@@ -141,68 +192,64 @@ __device__ int run(const Ctx& c, int et, Scratch* S, float* k_out, uint32_t* n_e
   sync();
   if (blockIdx.x == 0 && et < 7) R->k[et] = k_out[et];
   if (blockIdx.x == 0 && et == 0) R->mode = mode;
+  if (!skip) return mode;
 
-  // ---- the tiles of this CTA: one warp per tile of 128 -------------------------------------------------------------------
-  if (skip) {
-    float kk[7];
+  // ---- the tiles of this CTA: each warp tests kBatch tiles at a time from their summaries ------------------------------
+  float kk[7];
 #pragma unroll
-    for (int i = 0; i < 7; ++i) kk[i] = k_out[i];
-    unsigned rows = 0u;
-    for (int tile = blockIdx.x + warp * gridDim.x; tile < n_tiles; tile += kWarps * gridDim.x) {
-      // the tile's summaries (largest norms, least margin of each 32 rows) and its rows' tables, loaded together
-      float xm[3] = {0.0f, 0.0f, 0.0f}, mn = INFINITY;
+  for (int i = 0; i < 7; ++i) kk[i] = k_out[i];
+  const int stride = kWarps * (int)gridDim.x;
+  float mn = in.mn, xm = in.xm;
+  unsigned rows = 0u;
+  for (int base = blockIdx.x + warp * gridDim.x; base < n_tiles; base += kBatch * stride) {
+    if (base != (int)blockIdx.x + warp * (int)gridDim.x) load_batch(c, base, lane, n_tiles, mn, xm);
+    // lane 4 i: the least margin of tile i and its largest norms (a tile past the end passes with no rows)
+    mn = fminf(mn, __shfl_xor_sync(0xffffffffu, mn, 1));
+    mn = fminf(mn, __shfl_xor_sync(0xffffffffu, mn, 2));
+    float xx[3];
 #pragma unroll
-      for (int v = 0; v < 3; ++v)
-        if (v < V) xm[v] = c.xx_tmax[(size_t)v * n_tiles + tile];
-#pragma unroll
-      for (int q = 0; q < kTile / 32; ++q) {
-        const int chunk = tile * (kTile / 32) + q;
-        if (chunk < c.n_chunks) mn = fminf(mn, c.margin_min[chunk]);
-      }
-      int t0[4];
-      int nlive = 0;
+    for (int v = 0; v < 3; ++v) xx[v] = __shfl_sync(0xffffffffu, xm, (lane & ~3) + v);
+    const int tile = batch_tile(base, lane);
+    const bool lead = (lane & 3) == 0 && tile < n_tiles;
+    const bool pass = lead && tile_passes(kk, xx, mn, V);
+    if (pass) rows += (unsigned)min(kTile, c.n_rows - tile * kTile);
+    unsigned failed = __ballot_sync(0xffffffffu, lead && !pass);
+    while (failed) {                                // today's per-row test: the verdict of the tile is exactly its rows'
+      const int ft = __shfl_sync(0xffffffffu, tile, __ffs(failed) - 1);
+      failed &= failed - 1u;
+      bool ok = true;
 #pragma unroll
       for (int j = 0; j < 4; ++j) {
-        const int row = tile * kTile + j * 32 + lane;
-        t0[j] = (row < c.n_rows) ? c.table_cur[row] : 0;
-        nlive += (row < c.n_rows) ? 1 : 0;
-      }
-      bool pass = tile_passes(kk, xm, mn, V);
-      if (!pass) {                                  // today's per-row test: the verdict of the tile is exactly its rows'
-        pass = true;
+        const int row = ft * kTile + j * 32 + lane;
+        if (row < c.n_rows) {
+          float xr[3];
 #pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          const int row = tile * kTile + j * 32 + lane;
-          if (row < c.n_rows) {
-            float xx[3];
-#pragma unroll
-            for (int v = 0; v < 3; ++v) xx[v] = (v < V) ? c.xx[(size_t)v * c.xx_stride + row] : 0.0f;
-            pass = pass && (__fsub_rd(c.margin[row], screen_row_bound(kk, xx, V)) > 31.0f);
-          }
+          for (int v = 0; v < 3; ++v) xr[v] = (v < V) ? c.xx[(size_t)v * c.xx_stride + row] : 0.0f;
+          ok = ok && (__fsub_rd(c.margin[row], screen_row_bound(kk, xr, V)) > 31.0f);
         }
-        pass = __all_sync(0xffffffffu, pass);
       }
-      if (pass) {
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          const int row = tile * kTile + j * 32 + lane;
-          if (row < c.n_rows) c.choice[row] = t0[j];
-        }
-        const int chunk = tile * (kTile / 32) + lane;
-        if (lane < kTile / 32 && chunk < c.n_chunks) { c.birthmask[chunk] = 0u; c.movedmask[chunk] = 0u; }
-        rows += (unsigned)nlive;
+      if (__all_sync(0xffffffffu, ok)) {
+        if (lane == 0) rows += (unsigned)min(kTile, c.n_rows - ft * kTile);
       } else if (lane == 0) {
         const int j = atomicAdd(&S->n_eval, 1);
-        c.scr_work[blockIdx.x + j * gridDim.x] = tile;
-        c.scr_tiles[atomicAdd(&R->cnt, 1u)] = tile;
+        c.scr_work[blockIdx.x + j * gridDim.x] = ft;
+        c.scr_tiles[atomicAdd(&R->cnt, 1u)] = ft;
       }
     }
-    rows = __reduce_add_sync(0xffffffffu, rows);
-    if (lane == 0 && rows) atomicAdd(&S->rows, rows);
   }
+  rows = __reduce_add_sync(0xffffffffu, rows);
+  if (lane == 0 && rows) atomicAdd(&S->rows, rows);
   sync();
+  return mode;
+}
 
-  // ---- the last CTA out publishes the list and writes the reference of a refresh --------------------------------------
+// After decide(), once the other roles have the verdict and the list: the last CTA out publishes the counts and, in a
+// refresh, writes the reference.
+__device__ void publish(const Ctx& c, int et, int mode, uint32_t sweep, Scratch* S) {
+  ScreenRec* R = c.scr;
+  const int V = c.V;
+  const int n_tiles = (c.n_rows + kTile - 1) / kTile;
+  const bool skip = (mode == kScreenSkip);
   if (et == 0) {
     if (S->rows) atomicAdd(&R->rows, S->rows);
     __threadfence();
@@ -220,7 +267,6 @@ __device__ int run(const Ctx& c, int et, Scratch* S, float* k_out, uint32_t* n_e
         R->last_tiles_evaluated = n_tiles;
       }
     }
-    *n_eval_out = (uint32_t)S->n_eval;
   }
   sync();
   if (S->last && !skip) {
@@ -240,9 +286,8 @@ __device__ int run(const Ctx& c, int et, Scratch* S, float* k_out, uint32_t* n_e
         c.scr_tm[i - 2 * nb - V * 64] = c.tmass[i - 2 * nb - V * 64];
       }
     }
-    if (et == 0) { R->ref_sweep = g.sweep; R->valid = 1u; }
+    if (et == 0) { R->ref_sweep = sweep; R->valid = 1u; }
   }
-  return mode;
 }
 
 }  // namespace screen

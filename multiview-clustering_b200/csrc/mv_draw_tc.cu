@@ -440,7 +440,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_draw_tc(const Ctx c, const __gr
             ++issued;
           }
       }
-      if (!b_loaded) load_b();
+      if (!b_loaded && n_work > (int)blockIdx.x) load_b();   // a CTA whose screened list is empty needs no B operand
       if (prof) { prof_out[0] = w0; prof_out[1] = clock64() - t_start; }
     } else if (warp >= 1 && warp <= kMmaWarps) {
       // ---- MMA issuers: warps 1 and 2 take alternate tile-views.  One tcgen05.mma of this shape keeps the
@@ -451,8 +451,6 @@ __global__ void __launch_bounds__(kThreads, 1) k_draw_tc(const Ctx c, const __gr
       //      warp i % 2, and raw stages (4 = 2 per tile-view), remainder stages (2) and accumulator stages
       //      (6) all give consecutive uses of a stage the same parity of i.  The whole warp walks the loop
       //      (descriptor arithmetic stays warp-uniform); one elected lane issues. ----
-      mbar_wait(b_full, 0);
-      tc_fence_after();
       const int me = warp - 1;
       const uint32_t a_me = desc_lo(sbase + SmemLayout::raw_off + me * 2 * kHalfBytes);   // this warp's two raw stages
       const uint32_t b_lo0 = desc_lo(sbase + SmemLayout::b_off);
@@ -460,6 +458,10 @@ __global__ void __launch_bounds__(kThreads, 1) k_draw_tc(const Ctx c, const __gr
       const int* list;
       const int n_work = work_list(list);
       const int n_tv = (n_work > (int)blockIdx.x) ? ((n_work - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x) * V : 0;
+      if (n_tv > 0) {                                // the producer loads the B operand exactly when this CTA has work
+        mbar_wait(b_full, 0);
+        tc_fence_after();
+      }
       int v = me % V, ds = me;                       // view and accumulator stage of tile-view i
       const int vstep = kMmaWarps % V;
       uint32_t use = 0;                              // how many tile-views this warp has issued
@@ -574,10 +576,26 @@ __global__ void __launch_bounds__(kThreads, 1) k_draw_tc(const Ctx c, const __gr
         // read ahead of their own wait (k_finalize: the sweep-start state) must come from a COMPLETED previous finalize.
         pdl_trigger();
       }
+      // One round of loads for the staging and the screening verdict (screen::load): threads et < V * 64 take (view, table)
+      // et, threads 256 + t table t's masses.
+      screen::Inputs in;
+      unsigned long long same = 0ull;
+      float cv[kMaxTcViews] = {0.0f, 0.0f, 0.0f};
+      if (c.screen) {
+        screen::load(c, et, in);
+      } else {
+        in.g = *c.gparam;
+        if (et < V * 64) in.q = c.tparam[et];
+        else if (et >= 256 && et < 256 + 64) in.m = c.tmass[et - 256];
+      }
+      if (et < V * 64) same = c.tsame[et];
+      else if (et >= 256 && et < 256 + 64)
+        for (int v = 0; v < V; ++v) cv[v] = c.tparam[v * 64 + et - 256].C;
+      const ViewParam vp = (et < V) ? c.vparam[et] : ViewParam{};
       int lone_ok = 1;                                  // every live table's dishes are served by that table alone?
-      for (int i = et; i < V * 64; i += 512) {
-        const int v = i >> 6, t = i & 63;
-        const TableParam q = c.tparam[i];
+      if (et < V * 64) {
+        const int v = et >> 6, t = et & 63;
+        const TableParam& q = in.q;
         TcViewParams& P = s_p[v];
         P.A[t] = q.A; P.C[t] = q.C; P.W[t] = q.W; P.CW[t] = __fadd_rn(q.C, q.W);
         P.A1[t] = q.A1; P.C1[t] = q.C1; P.W1[t] = q.W1;
@@ -586,34 +604,38 @@ __global__ void __launch_bounds__(kThreads, 1) k_draw_tc(const Ctx c, const __gr
         // or n < 2), where removing the customer changes its likelihood by orders of magnitude (see lse_chunk)
         P.lone[t] = (q.lone ? 1 : 0) | ((q.dish >= 0 && (P.R[t] > 1.004f || P.R[t] == 0.0f)) ? 2 : 0);
         if (q.dish >= 0 && !q.lone) lone_ok = 0;
-        s_same[i] = c.tsame[i];
-      }
-      for (int t = et; t < 64; t += 512) {
-        const TableMass m = c.tmass[t];
+        s_same[et] = same;
+      } else if (et >= 256 && et < 256 + 64) {
+        const int t = et - 256;
+        const TableMass& m = in.m;
         s_tm[t] = m;
         float b = m.LM;
-        for (int v = 0; v < V; ++v) b = __fadd_rn(b, c.tparam[v * 64 + t].C);
+        for (int v = 0; v < V; ++v) b = __fadd_rn(b, cv[v]);
         s_lm[t] = b;                                    // base: log2 table mass + the views' offsets, in view order
         s_dlm[t] = __fadd_rn(m.LM1, -m.LM);             // what changes for the customer's own table (n_t - 1)
       }
-      if (et < V) s_vp[et] = c.vparam[et];
+      if (et < V) s_vp[et] = vp;
       if (et == 64) {
-        const GlobalParam g = *c.gparam;
-        s_misc[1] = g.sweep;
-        s_misc[2] = __float_as_uint(g.LMN0);
-        s_misc[3] = __float_as_uint(g.LMN1);
+        s_misc[1] = in.g.sweep;
+        s_misc[2] = __float_as_uint(in.g.LMN0);
+        s_misc[3] = __float_as_uint(in.g.LMN1);
       }
       if (c.screen) {
-        // The screening verdict of this sweep, its bound coefficients and, in a skip sweep, this CTA's list
-        const int mode = screen::run(c, et, reinterpret_cast<screen::Scratch*>(smem + SmemLayout::ex_off),
-                                     reinterpret_cast<float*>(s_misc + 6), s_misc + 13);
-        if (et == 0) s_misc[5] = (uint32_t)mode;
+        // The screening verdict of this sweep, its bound coefficients and, in a skip sweep, this CTA's list.  The other
+        // roles wait for the verdict and the list only; the bookkeeping of the last CTA comes after their release.
+        screen::Scratch* S = reinterpret_cast<screen::Scratch*>(smem + SmemLayout::ex_off);
+        const int mode = screen::decide(c, et, in, S, reinterpret_cast<float*>(s_misc + 6));
+        if (et == 0) {
+          s_misc[5] = (uint32_t)mode;
+          s_misc[13] = (uint32_t)S->n_eval;
+          mbar_arrive(list_full);
+        }
+        if (mode != kScreenOff) screen::publish(c, et, mode, in.g.sweep, S);
       } else if (et == 0) {
         s_misc[5] = (uint32_t)kScreenOff;
       }
       if (!lone_ok) atomicAnd(&s_misc[4], 0u);
       asm volatile("bar.sync 9, 512;" ::: "memory");    // the epilogue warpgroups only: the other roles never read these
-      if (c.screen && et == 0) mbar_arrive(list_full);  // ... except the verdict and the list, which they wait for
     }
     const uint32_t sweep = s_misc[1];
     GlobalParam gp;

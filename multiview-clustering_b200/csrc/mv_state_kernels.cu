@@ -649,7 +649,8 @@ __device__ __forceinline__ void draw_level_randoms(FS& S, uint64_t seed, uint32_
 }
 
 template <int MAXCAP>
-__global__ void __launch_bounds__(kFinThreads, 1) k_finalize(const Ctx c, const int32_t flags, const int32_t s1_in_smem) {
+__global__ void __launch_bounds__(kFinThreads, 1) k_finalize(const Ctx c, const int32_t flags, const int32_t s1_in_smem,
+                                                           const int32_t ref_in_smem) {
   extern __shared__ __align__(16) unsigned char fin_smem[];
   using FS = FinShared<MAXCAP>;
   using Set = SlotSet<FS::kWords>;
@@ -670,6 +671,11 @@ __global__ void __launch_bounds__(kFinThreads, 1) k_finalize(const Ctx c, const 
   // The per-table sums of this view, S1t [cap][D], live in shared memory behind FinShared when they fit (32 KB at C3):
   // the dish statistics and the posterior means are then built from on-chip data instead of global round trips.
   double* const S1t = s1_in_smem ? reinterpret_cast<double*>(fin_smem + fin_shared_bytes<MAXCAP>()) : (c.S1t + (size_t)cap * doff);
+  // Draw screening's reference of this view (scaled means hi, lo [cap][D], then the parameter block [cap]), which the drift
+  // sums of E1 read, follows in shared memory when it fits (32 KB at C3); otherwise E1 reads it from global memory.
+  auto ref_smem = [&]() {
+    return reinterpret_cast<float*>(fin_smem + fin_shared_bytes<MAXCAP>() + (s1_in_smem ? sizeof(double) * (size_t)cap * D : 0));
+  };
   const uint32_t sweep = *reinterpret_cast<volatile uint32_t*>(c.sweep);
   double& alpha_l = S.hyp[0];                       // alpha_v / alpha_global
   double& sigma_l = S.hyp[1];                       // sigma_v / sigma_global
@@ -712,6 +718,14 @@ __global__ void __launch_bounds__(kFinThreads, 1) k_finalize(const Ctx c, const 
       for (int i = tid; i < n_s1; i += kFinThreads) S1t[i] = src[i];
     }
     for (int t = tid; t < cap; t += kFinThreads) S.s2t[t] = c.sum_s2t[v * cap + t];
+    if (ref_in_smem) {                              // after the wait: a refresh draw of this sweep wrote the reference
+      const float* src = c.scr_b + (size_t)cap * doff;
+      float* dst = ref_smem();
+      const size_t half = (size_t)cap * c.Dsum;
+      for (int i = tid; i < cap * D; i += kFinThreads) { dst[i] = src[i]; dst[cap * D + i] = src[half + i]; }
+      TableParam* tp = reinterpret_cast<TableParam*>(dst + 2 * (size_t)cap * D);
+      for (int t = tid; t < cap; t += kFinThreads) tp[t] = c.scr_tp[v * cap + t];
+    }
   }
   __syncthreads();
   if (is_view && !s1_in_smem) {                     // large views: the sums stay in global memory (own block of S1t)
@@ -1140,11 +1154,11 @@ __global__ void __launch_bounds__(kFinThreads, 1) k_finalize(const Ctx c, const 
             const double tau = tau_l, n = (double)S.n_vk[k];
             A1_f = (float)(kLog2e * ((tau + n) / (2.0 * tau * (tau + n - 1.0))));
           }
-          const TableParam p = c.scr_tp[v * cap + t];
+          const TableParam p = ref_in_smem ? reinterpret_cast<const TableParam*>(ref_smem() + 2 * (size_t)cap * D)[t]
+                                           : c.scr_tp[v * cap + t];
           rq = (A_f != 0.0f) ? (double)__fdiv_rn(A1_f, A_f) : 0.0;
           rp = (p.A != 0.0f) ? (double)__fdiv_rn(p.A1, p.A) : 0.0;
         }
-        const size_t half = (size_t)cap * c.Dsum;
         double sb = 0.0, sd = 0.0, sr = 0.0;
         double mm = 0.0;
         for (int dd = lane; dd < D; dd += 32) {
@@ -1162,7 +1176,9 @@ __global__ void __launch_bounds__(kFinThreads, 1) k_finalize(const Ctx c, const 
             c.mean_lo[off + dd] = __uint_as_float(lb);
             if (scr) {
               const double b = (double)hi + (double)__uint_as_float(lb);
-              const double bp = (double)c.scr_b[off + dd] + (double)c.scr_b[half + off + dd];
+              const float* rb = ref_in_smem ? ref_smem() + t * D : c.scr_b + off;   // hi; lo one half further on
+              const size_t rhalf = ref_in_smem ? (size_t)cap * D : (size_t)cap * c.Dsum;
+              const double bp = (double)rb[dd] + (double)rb[rhalf + dd];
               const double db = b - bp, dr = __fma_rn(b, rq, -__dmul_rn(rp, bp));
               sb = __fma_rn(b, b, sb);
               sd = __fma_rn(db, db, sd);
@@ -1265,11 +1281,17 @@ static cudaError_t launch_finalize_cap(const Ctx& c, int32_t flags, cudaStream_t
   int dmax = 0;
   for (int v = 0; v < c.V; ++v) dmax = c.D[v] > dmax ? c.D[v] : dmax;
   const size_t s1_bytes = sizeof(double) * (size_t)c.cap * dmax;
-  const int s1_in_smem = (fin_shared_bytes<MAXCAP>() + s1_bytes <= (size_t)227 * 1024) ? 1 : 0;
-  const int smem = fin_shared_bytes<MAXCAP>() + (s1_in_smem ? (int)s1_bytes : 0);
-  cudaError_t e = cudaFuncSetAttribute(k_finalize<MAXCAP>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+  const size_t ref_bytes = (2 * sizeof(float) * dmax + sizeof(TableParam)) * (size_t)c.cap;
+  const size_t smem_max = (size_t)227 * 1024;
+  const int s1_in_smem = (fin_shared_bytes<MAXCAP>() + s1_bytes <= smem_max) ? 1 : 0;
+  size_t smem = fin_shared_bytes<MAXCAP>() + (s1_in_smem ? s1_bytes : 0);
+  const bool scr = c.scr_sum != nullptr && c.mean_hi != nullptr;   // the drift sums of draw screening are formed
+  const int ref_in_smem = (scr && smem + ref_bytes <= smem_max) ? 1 : 0;
+  if (ref_in_smem) smem += ref_bytes;
+  cudaError_t e = cudaFuncSetAttribute(k_finalize<MAXCAP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
-  return launch_chain(k_finalize<MAXCAP>, dim3(c.V + 1), dim3(kFinThreads), (size_t)smem, s, c.pdl != 0, c, flags, (int32_t)s1_in_smem);
+  return launch_chain(k_finalize<MAXCAP>, dim3(c.V + 1), dim3(kFinThreads), smem, s, c.pdl != 0, c, flags, (int32_t)s1_in_smem,
+                      (int32_t)ref_in_smem);
 }
 
 // The cap-64 instance keeps the shared-memory footprint of the small capacities; 128 and 256 take the wide one.

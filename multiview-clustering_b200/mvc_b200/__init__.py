@@ -107,6 +107,7 @@ def lib():
         L.mvg_set_draw_screen.argtypes = [H, C.c_int32]
         L.mvg_get_draw_screen_stats.argtypes = [H, C.POINTER(C.c_int32), C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
         L.mvg_get_draw_screen_record.argtypes = [H, C.POINTER(_ScreenHost)]
+        L.mvg_get_draw_rows.argtypes = [H, _i32p, _i32p, _u32p, _u32p]
         L.mvg_set_stats_mode.argtypes = [H, C.c_int32, C.c_int32]
         L.mvg_hyper_step_parts.argtypes = [H, C.c_int32]
         L.mvg_sync.argtypes = [H]
@@ -397,6 +398,16 @@ class Sampler:
         return {"mode": s.mode, "sweep": s.sweep, "valid": s.valid, "ref_sweep": s.ref_sweep,
                 "k": np.array(s.k[:], np.float32), "n_eval": s.n_eval, "tiles": tiles, "margin": margin, "ref": ref,
                 "ref_b": ref_b}
+
+    def get_draw_rows(self):
+        """The draw's per-row buffers as the most recent sweep left them (mvg_get_draw_rows): 'choice', 'table_cur'
+        [n_rows] and 'birthmask', 'movedmask' [ceil(n_rows / 32)] (bit r of word w: row 32 w + r)."""
+        n, w = self.n_rows, (self.n_rows + 31) // 32
+        out = {"choice": np.empty(n, np.int32), "table_cur": np.empty(n, np.int32),
+               "birthmask": np.empty(w, np.uint32), "movedmask": np.empty(w, np.uint32)}
+        self._ck(self.L.mvg_get_draw_rows(self.h, _p(out["choice"], _i32p), _p(out["table_cur"], _i32p),
+                                          _p(out["birthmask"], _u32p), _p(out["movedmask"], _u32p)))
+        return out
 
     def hyper_step(self):
         self._ck(self.L.mvg_hyper_step(self.h))
