@@ -149,6 +149,24 @@ int mvg_set_count_beta(mvg_handle* h, double beta);
  * that never calls it runs the plug-in kernels unchanged. */
 enum { MVG_COUNT_PLUGIN = 0, MVG_COUNT_DIRMULT = 1 };
 int mvg_set_count_likelihood(mvg_handle* h, int32_t model);
+/* Learn beta: under MVG_COUNT_DIRMULT, every count view v gets its own beta_v (starting at mvg_set_count_beta's value)
+ * and one Metropolis-Hastings step per hyper step (mvg_sweep with do_hyper, mvg_run, mvg_hyper_step) at the seating the
+ * sweep ends with: prior beta_v ~ Gamma(shape, rate), proposal log beta' = log beta + step z, acceptance
+ *   log A = L(beta') - L(beta) + shape (log beta' - log beta) - rate (beta' - beta),
+ * L(beta) = sum over live dishes k of sum_w [lnΓ(beta + c_kw) - lnΓ(beta)] - [lnΓ(W beta + C_k) - lnΓ(W beta)].
+ * z and the uniform u are Philox numbers of domain 7, slot v, index 0 (normal) and 1 (uniform), at the sweep index of the
+ * same hyper step's tau draws (mvg_philox_normal / mvg_philox_uniform_f64 regenerate them).  Before the first state call;
+ * non-finite or non-positive arguments: MVG_EINVAL; no count view, the plug-in model or after the first state call:
+ * MVG_ESTATE.  Without it beta stays where mvg_set_count_beta put it. */
+int mvg_set_count_beta_prior(mvg_handle* h, double shape, double rate, double step);
+/* beta [V]: beta_v of every count view, 0 for a dense view.  Synchronises. */
+int mvg_get_count_beta(mvg_handle* h, double* beta);
+/* The most recent beta step (read-only; any pointer may be NULL): log_accept [V] its log A per count view, accepted [V]
+ * 1 where it moved beta_v.  MVG_ESTATE without a prior or before the first state call.  Synchronises. */
+int mvg_get_count_beta_step(mvg_handle* h, double* log_accept, int32_t* accepted);
+/* Host buffer [n_saved_max][V] that later mvg_run calls fill with beta_v (as mvg_get_count_beta) on every kept sweep,
+ * beside saved_hypers; NULL turns it off. */
+int mvg_set_count_beta_trace(mvg_handle* h, double* saved_beta);
 
 /* ---- state ----------------------------------------------------------------------------- */
 int mvg_init_state_reference(mvg_handle* h);
@@ -157,7 +175,9 @@ int mvg_init_state_reference(mvg_handle* h);
 int mvg_set_state(mvg_handle* h, const mvg_state_host* s);
 int mvg_get_state(mvg_handle* h, const mvg_state_host* out);
 /* Binary checkpoint of the chain state in a file (SURVEY.md §8 f4; the reference keeps its chain in process globals and has
- * no resume: multiview_state.cpp:4-16, multiview_gibbs.cpp:117): assignments, dish_of, hyperparameters, sweep counter.
+ * no resume: multiview_state.cpp:4-16, multiview_gibbs.cpp:117): assignments, dish_of, hyperparameters, sweep counter,
+ * and for a handle with count views their beta_v [V] after the hyperparameters (a file without it loads and keeps the
+ * handle's beta).
  * Loading into a handle of the same shape with the same views restarts the chain bit-identically (statistics are rebuilt in
  * a fixed order, draws are addressed by (seed, sweep, row)); with the views of a row shard, each rank saves / loads its own file. */
 int mvg_save_checkpoint(mvg_handle* h, const char* path);
@@ -197,8 +217,10 @@ int mvg_set_draw_screen(mvg_handle* h, int32_t on);
 int mvg_get_draw_screen_stats(mvg_handle* h, int32_t* enabled, int64_t* rows_screened, int64_t* tiles_evaluated);
 int mvg_hyper_step(mvg_handle* h);
 /* The same restricted to some of its Metropolis-Hastings updates: update_tau_v_MH alone
- * (multiview_hyper.cpp:211-231), the per-view alpha/sigma pairs (:242-265), the franchise pair (:268-291). */
-enum { MVG_HYPER_TAU = 1, MVG_HYPER_LOCAL = 2, MVG_HYPER_GLOBAL = 4 };
+ * (multiview_hyper.cpp:211-231), the per-view alpha/sigma pairs (:242-265), the franchise pair (:268-291), the beta step
+ * of the count views (mvg_set_count_beta_prior; without a prior MVG_ESTATE).  mvg_hyper_step includes the beta step when
+ * a prior is set. */
+enum { MVG_HYPER_TAU = 1, MVG_HYPER_LOCAL = 2, MVG_HYPER_GLOBAL = 4, MVG_HYPER_COUNT_BETA = 8 };
 int mvg_hyper_step_parts(mvg_handle* h, int32_t parts);
 int mvg_sync(mvg_handle* h);
 /* gibbs_sampler(M, burn_in, thin): M sweeps; after sweep `iter` with iter >= burn_in and

@@ -6,6 +6,7 @@
 #include <dlfcn.h>
 #include <nvtx3/nvToolsExt.h>     // header-only NVTX 3: ranges per stage of a sweep (SURVEY.md §5); no-ops without a tool attached
 
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -114,6 +115,8 @@ struct mvg_handle {
   double* loglik_dev = nullptr;      // [V + 1] scratch of mvg_run's per-kept-sweep log-likelihood
   int32_t* host_fault = nullptr;     // mapped pinned host word: the sticky exchange fault, readable without a sync
   bool screen_want = true;           // mvg_set_draw_screen (effective on the tensor-core engines)
+  float count_beta = 0.5f;           // mvg_set_count_beta: every count view's beta_v until the first state call
+  double* saved_beta = nullptr;      // mvg_set_count_beta_trace: [n_saved_max][V] host buffer mvg_run fills, or null
 };
 
 namespace {
@@ -177,7 +180,7 @@ int ensure_layout(mvg_handle* h) {
   A(c.table_cur, N + 4 /* bulk copies read whole 16-byte groups */); A(c.choice, N + 4); A(c.birthmask, (size_t)c.n_chunks); A(c.movedmask, (size_t)c.n_chunks + 2); A(c.chunk_prefix, (size_t)c.n_chunks);
   A(c.n_t, cap); A(c.dish_of, V * cap); A(c.n_vk, V * cap); A(c.l_vk, V * cap);
   A(c.S1t, cap * dsum); A(c.S2t, V * cap); A(c.S1k, cap * dsum); A(c.S2k, V * cap);
-  A(c.hyp, 3 * V + 2); A(c.sweep, 1); A(c.status, 4);
+  A(c.hyp, 3 * V + 2); A(c.sweep, 1); A(c.status, 4); A(c.beta_v, V);
   A(c.sum_cnt, cap); A(c.sum_s1t, cap * dsum); A(c.sum_s2t, V * cap); A(c.xseq, 1); A(c.fin_arrive, 1); A(c.kclock, (size_t)kClockSlots);
   A(c.tparam, V * cap); A(c.vparam, V); A(c.tmass, cap); A(c.gparam, 1); A(c.tsame, V * cap);
   A(c.mean, cap * dsum); A(c.mean_hi, cap * dsum); A(c.mean_lo, cap * dsum);
@@ -204,6 +207,14 @@ int ensure_layout(mvg_handle* h) {
       A(c.cnt_acc[v], N * cap); A(c.cnt_loo[v], N);
       if (!c.table_prev) { A(c.table_prev, N); }
     }
+  if (c.n_count_views) {             // the beta step: a fixed grid per handle (one summation tree whatever the seating)
+    size_t max_cells = 0;
+    for (int v = 0; v < c.V; ++v)
+      if (c.kind[v] && (size_t)c.vocab[v] * cap > max_cells) max_cells = (size_t)c.vocab[v] * cap;
+    const size_t ctas = (max_cells + 1023) / 1024;   // about four cells per thread at the most
+    c.cb_ctas = (int32_t)std::min<size_t>(std::max<size_t>(ctas, 1), 296);
+    A(c.cb_part, V * (size_t)c.cb_ctas); A(c.cb_arrive, V); A(c.cb_accept, V); A(c.cb_logA, V);
+  }
 #undef A
   h->layout_done = true;
   // engine choice
@@ -272,17 +283,27 @@ int rebuild_pipeline(mvg_handle* h, int32_t flags, cudaEvent_t* marks /* 4 event
     MVG_CUDA(h, launch_counts_rebuild(h->c, /*delta=*/h->counts_valid, h->stream));
     h->counts_valid = true;            // cnt_t and table_prev now stand for the current seating
     h->launches += 2;
+    if (h->c.cb_on && (flags & kFinHyper) && (flags & kFinHyperCountBeta)) {   // the beta step needs the dish counts
+      NvtxRange r("mvg:count beta step");
+      MVG_CUDA(h, launch_count_beta(h->c, flags, /*refresh_only=*/false, h->stream));
+      h->launches += 3;
+    }
   }
   if (marks) MVG_CUDA(h, cudaEventRecord(marks[3], h->stream));
   h->launches += 2;
   return MVG_OK;
 }
 
-// MVG_COUNT_DIRMULT, at the first state call (beta and the views are frozen from then on): the denominator tables and the
-// per-row new-dish terms of every count view.  A no-op for the plug-in model.
+// At the first state call (the views, the model and the setter's beta are frozen from then on): beta_v of every count view,
+// then under MVG_COUNT_DIRMULT the denominator tables and the per-row new-dish terms.
 int prepare_count_model(mvg_handle* h) {
   Ctx& c = h->c;
-  if (h->state_ready || !c.count_model || !c.n_count_views) return MVG_OK;
+  if (h->state_ready || !c.n_count_views) return MVG_OK;
+  std::vector<double> beta((size_t)c.V, 0.0);
+  for (int v = 0; v < c.V; ++v) if (c.kind[v]) beta[(size_t)v] = (double)h->count_beta;
+  MVG_CUDA(h, cudaMemcpyAsync(c.beta_v, beta.data(), sizeof(double) * beta.size(), cudaMemcpyHostToDevice, h->stream));
+  MVG_CUDA(h, cudaStreamSynchronize(h->stream));       // (a host temporary)
+  if (!c.count_model) return MVG_OK;
   for (int v = 0; v < c.V; ++v) {
     if (!c.kind[v]) continue;
     if (c.cnt_nmax[v] >= (1 << 24))
@@ -374,7 +395,6 @@ int mvg_create(const mvg_config* cfg, mvg_handle** out) {
   c.debug_export = cfg->debug_export;
   c.blk_count = 1;
   c.blk_index = 0;
-  c.count_beta = 0.5f;
   {
     void* q = nullptr;
     c.xx_stride = ((int64_t)c.n_rows + 3) & ~(int64_t)3;        // rows of xx start 16-byte aligned (bulk copies)
@@ -505,7 +525,54 @@ int mvg_set_count_beta(mvg_handle* h, double beta) {
   if (!h) return MVG_EINVAL;
   if (!(beta > 0.0) || beta > 1.0e6) return fail(h, MVG_EINVAL, "count_beta must be positive");
   if (h->state_ready) return fail(h, MVG_ESTATE, "count_beta is frozen after the first state call");
-  h->c.count_beta = (float)beta;
+  h->count_beta = (float)beta;
+  return MVG_OK;
+}
+
+int mvg_set_count_beta_prior(mvg_handle* h, double shape, double rate, double step) {
+  if (!h) return MVG_EINVAL;
+  if (!(std::isfinite(shape) && shape > 0.0) || !(std::isfinite(rate) && rate > 0.0) || !(std::isfinite(step) && step > 0.0))
+    return fail(h, MVG_EINVAL, "the count beta prior needs finite positive shape, rate and step");
+  bool any_count = false;
+  for (int v = 0; v < h->c.V; ++v) any_count = any_count || h->c.kind[v] != 0;
+  if (h->c.count_model != MVG_COUNT_DIRMULT || !any_count)
+    return fail(h, MVG_ESTATE, "the beta step needs a count view under MVG_COUNT_DIRMULT (the plug-in likelihood has no marginal)");
+  if (h->state_ready) return fail(h, MVG_ESTATE, "the count beta prior is frozen after the first state call");
+  h->c.cb_on = 1;
+  h->c.cb_shape = shape;
+  h->c.cb_rate = rate;
+  h->c.cb_step = step;
+  invalidate_graphs(h);
+  return MVG_OK;
+}
+
+int mvg_get_count_beta(mvg_handle* h, double* beta) {
+  if (!h || !beta) return MVG_EINVAL;
+  const Ctx& c = h->c;
+  if (!h->state_ready) {               // nothing on the device yet: what the first state call will set
+    for (int v = 0; v < c.V; ++v) beta[v] = c.kind[v] ? (double)h->count_beta : 0.0;
+    return MVG_OK;
+  }
+  MVG_CUDA(h, cudaSetDevice(h->cfg.device));
+  MVG_CUDA(h, cudaMemcpyAsync(beta, c.beta_v, sizeof(double) * (size_t)c.V, cudaMemcpyDeviceToHost, h->stream));
+  MVG_CUDA(h, cudaStreamSynchronize(h->stream));
+  return MVG_OK;
+}
+
+int mvg_get_count_beta_step(mvg_handle* h, double* log_accept, int32_t* accepted) {
+  if (!h) return MVG_EINVAL;
+  const Ctx& c = h->c;
+  if (!c.cb_on || !h->state_ready) return fail(h, MVG_ESTATE, "no count beta step has run (set a prior, then a state)");
+  MVG_CUDA(h, cudaSetDevice(h->cfg.device));
+  if (log_accept) MVG_CUDA(h, cudaMemcpyAsync(log_accept, c.cb_logA, sizeof(double) * (size_t)c.V, cudaMemcpyDeviceToHost, h->stream));
+  if (accepted) MVG_CUDA(h, cudaMemcpyAsync(accepted, c.cb_accept, sizeof(int32_t) * (size_t)c.V, cudaMemcpyDeviceToHost, h->stream));
+  MVG_CUDA(h, cudaStreamSynchronize(h->stream));
+  return MVG_OK;
+}
+
+int mvg_set_count_beta_trace(mvg_handle* h, double* saved_beta) {
+  if (!h) return MVG_EINVAL;
+  h->saved_beta = saved_beta;
   return MVG_OK;
 }
 
@@ -706,6 +773,12 @@ int mvg_save_checkpoint(mvg_handle* h, const char* path) {
             fwrite(tab.data(), sizeof(int32_t), tab.size(), f) == tab.size() &&
             fwrite(dish.data(), sizeof(int32_t), dish.size(), f) == dish.size() &&
             fwrite(hyp.data(), sizeof(double), hyp.size(), f) == hyp.size();
+  if (ok && c.n_count_views) {       // count views: beta_v [V] follows (a dense-only file ends with the hyperparameters)
+    std::vector<double> beta((size_t)c.V);
+    rc = mvg_get_count_beta(h, beta.data());
+    ok = rc == MVG_OK && fwrite(beta.data(), sizeof(double), beta.size(), f) == beta.size();
+    if (rc != MVG_OK) { fclose(f); return rc; }
+  }
   ok = (fclose(f) == 0) && ok;
   return ok ? MVG_OK : fail(h, MVG_EINVAL, std::string("short write to ") + path);
 }
@@ -726,13 +799,33 @@ int mvg_load_checkpoint(mvg_handle* h, const char* path) {
   }
   ok = ok && fread(tab.data(), sizeof(int32_t), tab.size(), f) == tab.size() &&
        fread(dish.data(), sizeof(int32_t), dish.size(), f) == dish.size() && fread(hyp.data(), sizeof(double), hyp.size(), f) == hyp.size();
+  // a file of a handle with count views may carry their beta_v; one written before it did keeps the handle's
+  std::vector<double> beta((size_t)c.V);
+  bool has_beta = false;
+  if (ok) {
+    for (int v = 0; v < c.V; ++v) has_beta = has_beta || c.kind[v] != 0;
+    has_beta = has_beta && fread(beta.data(), sizeof(double), beta.size(), f) == beta.size();
+  }
   fclose(f);
   if (!ok) return fail(h, MVG_EINVAL, std::string("not a checkpoint or truncated: ") + path);
+  if (has_beta)
+    for (int v = 0; v < c.V; ++v)
+      if (c.kind[v] && !(std::isfinite(beta[v]) && beta[v] > 0.0)) return fail(h, MVG_EINVAL, "checkpoint holds a non-positive count beta");
   uint32_t sweep = (uint32_t)hdr[7];
   mvg_state_host st{};
   st.table_of = tab.data(); st.dish_of = dish.data(); st.alpha_v = hyp.data(); st.sigma_v = hyp.data() + c.V; st.tau_v = hyp.data() + 2 * c.V;
   st.alpha_sigma_global = hyp.data() + 3 * c.V; st.sweep = &sweep;
-  return mvg_set_state(h, &st);
+  int rc = mvg_set_state(h, &st);
+  if (rc != MVG_OK || !has_beta) return rc;
+  // beta_v, then everything that depends on it, by the refresh that follows an accepted beta step (every count view)
+  std::vector<int32_t> all((size_t)c.V);
+  for (int v = 0; v < c.V; ++v) all[(size_t)v] = c.kind[v] ? 1 : 0;
+  MVG_CUDA(h, cudaMemcpyAsync(c.beta_v, beta.data(), sizeof(double) * beta.size(), cudaMemcpyHostToDevice, h->stream));
+  MVG_CUDA(h, cudaMemcpyAsync(c.cb_accept, all.data(), sizeof(int32_t) * all.size(), cudaMemcpyHostToDevice, h->stream));
+  MVG_CUDA(h, launch_count_beta(c, 0, /*refresh_only=*/true, h->stream));
+  h->launches += 2;
+  MVG_CUDA(h, cudaStreamSynchronize(h->stream));       // (host temporaries)
+  return MVG_OK;
 }
 
 int mvg_get_state(mvg_handle* h, const mvg_state_host* o) {
@@ -966,7 +1059,8 @@ int mvg_get_draw_screen_record(mvg_handle* h, mvg_screen_host* o) {
 int mvg_hyper_step_parts(mvg_handle* h, int32_t parts) {
   if (!h) return MVG_EINVAL;
   if (!h->state_ready) return fail(h, MVG_ESTATE, "no state yet");
-  if (parts & ~(MVG_HYPER_TAU | MVG_HYPER_LOCAL | MVG_HYPER_GLOBAL)) return fail(h, MVG_EINVAL, "unknown hyper part");
+  if (parts & ~(MVG_HYPER_TAU | MVG_HYPER_LOCAL | MVG_HYPER_GLOBAL | MVG_HYPER_COUNT_BETA)) return fail(h, MVG_EINVAL, "unknown hyper part");
+  if ((parts & MVG_HYPER_COUNT_BETA) && !h->c.cb_on) return fail(h, MVG_ESTATE, "no count beta prior set (mvg_set_count_beta_prior)");
   h->draw_pending = false;                           // the parameters are about to change
   MVG_CUDA(h, cudaSetDevice(h->cfg.device));
   // rebuild the statistics of the current assignment, then the selected Metropolis-Hastings updates
@@ -977,10 +1071,14 @@ int mvg_hyper_step_parts(mvg_handle* h, int32_t parts) {
   if (parts & MVG_HYPER_TAU) flags |= kFinHyperTau;
   if (parts & MVG_HYPER_LOCAL) flags |= kFinHyperLocal;
   if (parts & MVG_HYPER_GLOBAL) flags |= kFinHyperGlobal;
+  if (parts & MVG_HYPER_COUNT_BETA) flags |= kFinHyperCountBeta;
   return rebuild_pipeline(h, flags, nullptr);
 }
 
-int mvg_hyper_step(mvg_handle* h) { return mvg_hyper_step_parts(h, MVG_HYPER_TAU | MVG_HYPER_LOCAL | MVG_HYPER_GLOBAL); }
+int mvg_hyper_step(mvg_handle* h) {
+  if (!h) return MVG_EINVAL;
+  return mvg_hyper_step_parts(h, MVG_HYPER_TAU | MVG_HYPER_LOCAL | MVG_HYPER_GLOBAL | (h->c.cb_on ? MVG_HYPER_COUNT_BETA : 0));
+}
 
 int mvg_sync(mvg_handle* h) {
   if (!h) return MVG_EINVAL;
@@ -1021,6 +1119,9 @@ int mvg_run(mvg_handle* h, int32_t M, int32_t burn_in, int32_t thin, int32_t n_s
       if (saved_hypers)
         MVG_CUDA(h, cudaMemcpyAsync(saved_hypers + (size_t)saved * (3 * c.V + 2), c.hyp,
                                     sizeof(double) * (size_t)(3 * c.V + 2), cudaMemcpyDeviceToHost, h->stream));
+      if (h->saved_beta && c.beta_v)
+        MVG_CUDA(h, cudaMemcpyAsync(h->saved_beta + (size_t)saved * c.V, c.beta_v, sizeof(double) * (size_t)c.V,
+                                    cudaMemcpyDeviceToHost, h->stream));
       if (saved_loglik) {           // saved_loglik of the reference's state (multiview_state.h:38): filled on every kept sweep
         if (!h->loglik_dev) {
           void* q = nullptr;

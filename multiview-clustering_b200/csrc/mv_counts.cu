@@ -64,10 +64,14 @@ __global__ void k_counts_scatter(const Ctx c, const int delta) {
 
 // MAXCAP: 64 (one mask word per slot) or 256; cap is a power of two <= MAXCAP.
 // DM (MVG_COUNT_DIRMULT): the cell is log2(beta + cd) instead of log2 theta, and the denominator table follows the cells.
+// gate != null: the refresh after a beta step (launch_count_beta): only the views whose step accepted (gate[v] != 0) run,
+// with the new beta_v; the same cells and denominators, and TableParam::C1 of the view's live tables.
 template <int MAXCAP, bool DM>
-__global__ void k_counts_tables(const Ctx c, const int log2cap) {
+__global__ void k_counts_tables(const Ctx c, const int log2cap, const int32_t* __restrict__ gate) {
   constexpr int kWords = MAXCAP / 64;
   const int v = nth_count_view(c, blockIdx.y);
+  if (gate && gate[v] == 0) return;
+  const double beta = c.beta_v[v];
   __shared__ int32_t s_dish[MAXCAP];
   __shared__ double s_den[MAXCAP];
   __shared__ float s_l2zero[MAXCAP];                         // log2 theta of a word the dish has never seen: most cells of the table
@@ -77,9 +81,11 @@ __global__ void k_counts_tables(const Ctx c, const int log2cap) {
     const int k = c.dish_of[v * cap + threadIdx.x];
     s_dish[threadIdx.x] = k;
     // S2k of a count view holds the token total of the dish (an exact integer)
-    s_den[threadIdx.x] = (k >= 0) ? (double)c.vocab[v] * (double)c.count_beta + c.S2k[v * cap + k] : 1.0;
-    if constexpr (DM) s_l2zero[threadIdx.x] = (float)log2((double)c.count_beta);
-    else s_l2zero[threadIdx.x] = (float)log2(((double)c.count_beta + 0.0) / s_den[threadIdx.x]);   // the cell expression at cd = 0
+    s_den[threadIdx.x] = (k >= 0) ? count_wbeta_total(c.vocab[v], beta, c.S2k[v * cap + k]) : 1.0;
+    if constexpr (DM) s_l2zero[threadIdx.x] = (float)log2(beta);
+    else s_l2zero[threadIdx.x] = (float)log2((beta + 0.0) / s_den[threadIdx.x]);   // the cell expression at cd = 0
+    // (k_finalize wrote C1 by the same expression at the beta it saw)
+    if (gate && blockIdx.x == 0 && k >= 0) c.tparam[v * cap + threadIdx.x].C1 = (float)s_den[threadIdx.x];
   }
   __syncthreads();
   if (threadIdx.x < cap) {
@@ -95,7 +101,7 @@ __global__ void k_counts_tables(const Ctx c, const int log2cap) {
   __syncthreads();
   // (every view's scatter has read table_prev by now — this kernel follows it in the stream: the seating the counts now
   //  stand for is the current one)
-  if (blockIdx.y == 0)
+  if (!gate && blockIdx.y == 0)
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < c.n_rows; i += gridDim.x * blockDim.x) c.table_prev[i] = c.table_cur[i];
   const size_t total = (size_t)c.vocab[v] * cap;
   for (size_t e = (size_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (size_t)gridDim.x * blockDim.x) {
@@ -109,8 +115,8 @@ __global__ void k_counts_tables(const Ctx c, const int log2cap) {
 #pragma unroll
       for (int wi = 0; wi < kWords; ++wi)
         for (unsigned long long m = s_mask[t][wi]; m; m &= m - 1ull) cd += row[64 * wi + __ffsll((long long)m) - 1];
-      if constexpr (DM) l2 = (cd == 0) ? s_l2zero[t] : (float)log2((double)c.count_beta + (double)cd);
-      else l2 = (cd == 0) ? s_l2zero[t] : (float)log2(((double)c.count_beta + (double)cd) / s_den[t]);
+      if constexpr (DM) l2 = (cd == 0) ? s_l2zero[t] : (float)log2(beta + (double)cd);
+      else l2 = (cd == 0) ? s_l2zero[t] : (float)log2((beta + (double)cd) / s_den[t]);
     }
     c.cnt_d[v][e] = cd;
     c.l2t[v][e] = l2;
@@ -126,14 +132,16 @@ __global__ void k_counts_tables(const Ctx c, const int log2cap) {
   }
 }
 
-// MVG_COUNT_DIRMULT, once per chain (beta is frozen at the first state call and the rows never change):
+// MVG_COUNT_DIRMULT, at the first state call and again whenever beta_v moves (the rows never change):
 // q[i] = -log2 f_new(x_i) = -(sum_w lnΓ(beta + x_w) - lnΓ(beta)  -  [lnΓ(W beta + n) - lnΓ(W beta)]) / ln 2, FP64, ascending
 // over the row's nonzeros, rounded once.  The draw's new-dish term reads it where the plug-in reads the token total.
-__global__ void k_counts_newdish(const Ctx c) {
+// gate as in k_counts_tables.
+__global__ void k_counts_newdish(const Ctx c, const int32_t* __restrict__ gate) {
   const int v = nth_count_view(c, blockIdx.y);
+  if (gate && gate[v] == 0) return;
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= c.n_rows) return;
-  const double beta = (double)c.count_beta;
+  const double beta = c.beta_v[v];
   double lf = 0.0;
   int n = 0;
   for (int j = c.rowptr[v][i]; j < c.rowptr[v][i + 1]; ++j) {
@@ -167,6 +175,7 @@ __global__ void __launch_bounds__(512) k_counts_loglik(const Ctx c) {
   const int32_t* __restrict__ cdt = c.cnt_d[v];
   const TableParam* __restrict__ tp = c.tparam + v * CAP;
   const int32_t* __restrict__ order = c.row_order[v];
+  const float beta = (float)c.beta_v[v];
   constexpr int kFlight = 8;                         // table rows in flight per warp
   for (int ri = warp; ri < c.n_rows; ri += nwarps) {
     const int row = order ? __ldg(order + ri) : ri;
@@ -187,7 +196,7 @@ __global__ void __launch_bounds__(512) k_counts_loglik(const Ctx c) {
       float term_l = 0.0f;
       if (has) {
         const float cown = (float)__ldg(cdt + (size_t)col_l * CAP + t0);
-        term_l = __fadd_rn(log2m(__fadd_rn(__fadd_rn(c.count_beta, cown), -xv_l)), -lden);
+        term_l = __fadd_rn(log2m(__fadd_rn(__fadd_rn(beta, cown), -xv_l)), -lden);
       }
       const int cnt = min(32, j1 - jb);
       for (int u0 = 0; u0 < cnt; u0 += kFlight) {
@@ -250,7 +259,7 @@ __global__ void __launch_bounds__(512) k_counts_loglik_dm(const Ctx c) {
   const float* __restrict__ den = c.cnt_den[v];
   const TableParam* __restrict__ tp = c.tparam + v * CAP;
   const int32_t* __restrict__ order = c.row_order[v];
-  const float beta = c.count_beta;
+  const float beta = (float)c.beta_v[v];
   constexpr int kFlight = 8;
   for (int ri = warp; ri < c.n_rows; ri += nwarps) {
     const int row = order ? __ldg(order + ri) : ri;
@@ -357,12 +366,27 @@ cudaError_t launch_counts_loglik(const Ctx& c, cudaStream_t s) {
 
 cudaError_t launch_counts_newdish(const Ctx& c, cudaStream_t s) {
   if (!c.n_count_views || !c.count_model || c.n_rows <= 0) return cudaSuccess;
-  k_counts_newdish<<<dim3((c.n_rows + 255) / 256, c.n_count_views), 256, 0, s>>>(c);
+  k_counts_newdish<<<dim3((c.n_rows + 255) / 256, c.n_count_views), 256, 0, s>>>(c, nullptr);
   return cudaGetLastError();
 }
 
 cudaError_t launch_rowtotals(const int32_t* rowptr, const float* val, float* out, int n, cudaStream_t s) {
   k_rowtotals<<<(n + 255) / 256, 256, 0, s>>>(rowptr, val, out, n);
+  return cudaGetLastError();
+}
+
+static cudaError_t launch_counts_tables(const Ctx& c, size_t max_cells, const int32_t* gate, cudaStream_t s) {
+  int tb = (int)((max_cells + 255) / 256);
+  if (tb > 148 * 8) tb = 148 * 8;
+  const int log2cap = __builtin_ctz((unsigned)c.cap);
+  if (c.count_model) {
+    if (c.cap <= 64) k_counts_tables<64, true><<<dim3(tb, c.n_count_views), 256, 0, s>>>(c, log2cap, gate);
+    else k_counts_tables<256, true><<<dim3(tb, c.n_count_views), 256, 0, s>>>(c, log2cap, gate);
+  } else if (c.cap <= 64) {
+    k_counts_tables<64, false><<<dim3(tb, c.n_count_views), 256, 0, s>>>(c, log2cap, gate);
+  } else {
+    k_counts_tables<256, false><<<dim3(tb, c.n_count_views), 256, 0, s>>>(c, log2cap, gate);   // one thread per slot: 256 threads
+  }
   return cudaGetLastError();
 }
 
@@ -381,17 +405,106 @@ cudaError_t launch_counts_rebuild(const Ctx& c, bool delta, cudaStream_t s) {
   int blocks = (c.n_rows + 7) / 8;                 // 8 warps per block, one row per warp per step
   if (blocks > 148 * 4) blocks = 148 * 4;
   k_counts_scatter<<<dim3(blocks, c.n_count_views), 256, 0, s>>>(c, delta ? 1 : 0);
-  int tb = (int)((max_cells + 255) / 256);
-  if (tb > 148 * 8) tb = 148 * 8;
-  const int log2cap = __builtin_ctz((unsigned)c.cap);
-  if (c.count_model) {
-    if (c.cap <= 64) k_counts_tables<64, true><<<dim3(tb, c.n_count_views), 256, 0, s>>>(c, log2cap);
-    else k_counts_tables<256, true><<<dim3(tb, c.n_count_views), 256, 0, s>>>(c, log2cap);
-  } else if (c.cap <= 64) {
-    k_counts_tables<64, false><<<dim3(tb, c.n_count_views), 256, 0, s>>>(c, log2cap);
-  } else {
-    k_counts_tables<256, false><<<dim3(tb, c.n_count_views), 256, 0, s>>>(c, log2cap);   // one thread per slot: 256 threads
+  return launch_counts_tables(c, max_cells, nullptr, s);
+}
+
+// ---- the beta step (MVG_COUNT_DIRMULT with a prior; DESIGN.md §4.5) -----------------------------------------------------
+// For count view v at the seating k_counts_tables just counted, with L(beta) = sum over live dishes k of
+//   sum_{w : c_kw > 0} lnΓ(beta + c_kw) - lnΓ(beta)  -  [lnΓ(W beta + C_k) - lnΓ(W beta)]
+// (the beta-dependent part of the collapsed marginal; k_loglik's cell expression, lowest table slot of each dish):
+//   z = Philox normal (kDomCountBeta, slot v, index 0),  log beta' = log beta + step z,
+//   log A = L(beta') - L(beta) + shape (log beta' - log beta) - rate (beta' - beta),
+//   u = Philox uniform (index 1): beta_v[v] = beta' when log u < log A.
+// The (word, live dish) cells and the dish denominators are spread over cb_ctas CTAs per view; every thread sums
+// lnΓ-differences at beta' minus those at beta of its cells in grid-stride order, the CTA by a fixed tree, and the last
+// CTA to arrive adds the CTA partials in ascending order and decides.  The grid is fixed per handle, so the sum (and the
+// decision) depends on neither timing nor graph replay.
+constexpr int kBetaThreads = 256;
+__global__ void __launch_bounds__(kBetaThreads) k_count_beta_step(const Ctx c, const int32_t advance) {
+  const int v = nth_count_view(c, blockIdx.y);
+  const int cap = c.cap;
+  __shared__ int32_t s_rep[256];                  // lowest table slot of every live dish, -1 = none
+  __shared__ int32_t s_lt[256], s_lk[256];        // the live dishes, ascending: representative slot, dish
+  __shared__ int32_t s_nlive;
+  __shared__ double s_red[kBetaThreads];
+  __shared__ bool s_last;
+  if (threadIdx.x < cap) {
+    const int k = threadIdx.x;
+    int rep = -1;
+    if (c.n_vk[v * cap + k] > 0)
+      for (int t = cap - 1; t >= 0; --t) if (c.dish_of[v * cap + t] == k) rep = t;
+    s_rep[k] = rep;
   }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    int n = 0;
+    for (int k = 0; k < cap; ++k)
+      if (s_rep[k] >= 0) { s_lt[n] = s_rep[k]; s_lk[n] = k; ++n; }
+    s_nlive = n;
+  }
+  __syncthreads();
+  const uint32_t sweep = *c.sweep - (advance ? 1u : 0u);   // k_finalize of this rebuild has advanced it already
+  const double beta = c.beta_v[v];
+  const U4 rz = stream_block(c.seed, c.chain, kDomCountBeta, (uint32_t)v, sweep, 0);
+  const double z = sqrt(-2.0 * log(uniform_f64_from(rz.x, rz.y))) * cos(6.283185307179586476925286766559 * uniform_f64_from(rz.z, rz.w));
+  const double lb = log(beta), lbp = lb + c.cb_step * z, betap = exp(lbp);
+  const double wb = (double)c.vocab[v] * beta, wbp = (double)c.vocab[v] * betap;
+  const int nl = s_nlive;
+  const int32_t* __restrict__ cd = c.cnt_d[v];
+  const size_t cells = (size_t)c.vocab[v] * nl;
+  double d = 0.0;
+  for (size_t e = (size_t)blockIdx.x * blockDim.x + threadIdx.x; e < cells + nl; e += (size_t)gridDim.x * blockDim.x) {
+    if (e < cells) {
+      const size_t w = e / nl;
+      const int x = cd[w * cap + s_lt[e - w * nl]];
+      if (x > 0) d += lgamma_diff(betap, x) - lgamma_diff(beta, x);   // a zero cell contributes exactly 0
+    } else {
+      const int tot = (int)c.S2k[v * cap + s_lk[e - cells]];        // the dish's token total (an exact integer)
+      d -= lgamma_diff(wbp, tot) - lgamma_diff(wb, tot);
+    }
+  }
+  s_red[threadIdx.x] = d;
+  __syncthreads();
+#pragma unroll
+  for (int o = kBetaThreads / 2; o > 0; o >>= 1) {
+    if (threadIdx.x < o) s_red[threadIdx.x] += s_red[threadIdx.x + o];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) {
+    c.cb_part[(size_t)v * gridDim.x + blockIdx.x] = s_red[0];
+    __threadfence();
+    s_last = atomicAdd(&c.cb_arrive[v], 1u) == gridDim.x - 1;
+  }
+  __syncthreads();
+  if (!s_last || threadIdx.x != 0) return;
+  __threadfence();
+  const volatile double* part = c.cb_part + (size_t)v * gridDim.x;
+  double dl = 0.0;
+  for (unsigned b = 0; b < gridDim.x; ++b) dl += part[b];
+  const double log_a = dl + c.cb_shape * (lbp - lb) - c.cb_rate * (betap - beta);
+  const U4 ru = stream_block(c.seed, c.chain, kDomCountBeta, (uint32_t)v, sweep, 1);
+  const bool acc = log(uniform_f64_from(ru.x, ru.y)) < log_a;
+  if (acc) c.beta_v[v] = betap;
+  c.cb_accept[v] = acc ? 1 : 0;
+  c.cb_logA[v] = log_a;
+  c.cb_arrive[v] = 0u;                                              // ready for the next launch
+}
+
+cudaError_t launch_count_beta(const Ctx& c, int32_t flags, bool refresh_only, cudaStream_t s) {
+  if (!c.n_count_views) return cudaSuccess;
+  if (!refresh_only) {
+    if (!c.cb_on || !(flags & kFinHyper) || !(flags & kFinHyperCountBeta)) return cudaSuccess;
+    k_count_beta_step<<<dim3(c.cb_ctas, c.n_count_views), kBetaThreads, 0, s>>>(c, (flags & kFinAdvance) ? 1 : 0);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+  }
+  // the refresh: every CTA of a view whose step rejected returns at once
+  size_t max_cells = 0;
+  for (int v = 0; v < c.V; ++v)
+    if (c.kind[v] && (size_t)c.vocab[v] * c.cap > max_cells) max_cells = (size_t)c.vocab[v] * c.cap;
+  cudaError_t e = launch_counts_tables(c, max_cells, c.cb_accept, s);
+  if (e != cudaSuccess) return e;
+  if (c.count_model) k_counts_newdish<<<dim3((c.n_rows + 255) / 256, c.n_count_views), 256, 0, s>>>(c, c.cb_accept);
   return cudaGetLastError();
 }
 

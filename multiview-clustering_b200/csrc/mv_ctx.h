@@ -62,15 +62,25 @@ struct Ctx {
   float* l2t[kMaxViews];       // [vocab][cap] log2 theta of that dish: log2((beta + cnt_d) / (W beta + total))
   float* cnt_acc[kMaxViews];   // [N][cap] log2 f of every row under every table slot's dish (stage A of the sweep)
   float* cnt_loo[kMaxViews];   // [N] the same under the row's own dish with the row removed
-  float count_beta;            // symmetric Dirichlet pseudo-count
+  double* beta_v;              // [V] symmetric Dirichlet pseudo-count of every count view (0 for a dense view); the one
+                               // source of beta on the device, for both count models
   int32_t n_count_views;
   // MVG_COUNT_DIRMULT (count_model = 1, every count view of the handle; DESIGN.md §4.5): l2t holds log2(beta + cnt_d)
   // instead of log2 theta, and
   int32_t count_model;
   int32_t cnt_nmax[kMaxViews]; // the longest row in tokens (known at upload)
   float* cnt_den[kMaxViews];   // [n_max+1][cap] sum_{j<n} log2(W beta + C_k + j) of the dish each slot serves, length-major
-  float* cnt_q[kMaxViews];     // [N] -log2 f_new of every row (fixed once beta is): what the new-dish term reads
-  int32_t* table_prev;         // [N] count views: the table every row's words are currently counted at in cnt_t
+  float* cnt_q[kMaxViews];     // [N] -log2 f_new of every row (a function of beta alone): what the new-dish term reads
+  // Metropolis-Hastings step for beta_v (MVG_COUNT_DIRMULT with mvg_set_count_beta_prior; DESIGN.md §4.5): prior
+  // Gamma(cb_shape, rate cb_rate), log-normal random walk of scale cb_step, one step per count view per hyper step
+  int32_t cb_on;
+  int32_t cb_ctas;             // CTAs per view of k_count_beta_step (fixed per handle: fixes the summation tree)
+  double cb_shape, cb_rate, cb_step;
+  double* cb_part;             // [V][cb_ctas] per-CTA partial sums of L(beta') - L(beta)
+  uint32_t* cb_arrive;         // [V] arrival counters of k_count_beta_step (zero between launches)
+  int32_t* cb_accept;          // [V] 1: the most recent step of view v moved beta_v[v] (the refresh kernels run), else 0
+  double* cb_logA;             // [V] log acceptance ratio of the most recent step (mvg_get_count_beta_step)
+  int32_t* table_prev;        // [N] count views: the table every row's words are currently counted at in cnt_t
   float* xx;                // [V][xx_stride] squared norms of the rows (count views: the rows' total counts), computed once per upload
   int64_t xx_stride;        // n_rows rounded up to a multiple of 4
   float* xx_tmax;           // [V][ceil(N/128)] largest xx of each tile of 128 rows (a NaN counts as +inf): draw screening
@@ -230,7 +240,8 @@ enum FinalizeFlags : int32_t {
   kFinHyperTau = 16,   //   tau_v            (update_tau_v_MH)
   kFinHyperLocal = 32, //   alpha_v, sigma_v
   kFinHyperGlobal = 64,//   alpha_global, sigma_global
-  kFinHyperAll = 2 | 16 | 32 | 64,
+  kFinHyperCountBeta = 128, //  beta_v of the count views (k_count_beta_step after the tables; only with a prior set)
+  kFinHyperAll = 2 | 16 | 32 | 64 | 128,
   kFinAdvance = 4,     // sweep += 1
   kFinTauInit = 8      // derive tau_v from pooled variance (reference init), alpha/sigma literals
 };
@@ -258,7 +269,12 @@ int stats_smem_bytes(const Ctx& c);
 cudaError_t launch_rowtotals(const int32_t* rowptr, const float* val, float* out, int n, cudaStream_t s);
 cudaError_t launch_counts_rebuild(const Ctx& c, bool delta, cudaStream_t s);   // per count view: word counts per table slot (from scratch, or only the rows that changed table), dish tables
 cudaError_t launch_counts_loglik(const Ctx& c, cudaStream_t s);    // per count view: log2 f of every row under every table
-cudaError_t launch_counts_newdish(const Ctx& c, cudaStream_t s);   // DIRMULT: cnt_q of every count view, once beta is frozen
+cudaError_t launch_counts_newdish(const Ctx& c, cudaStream_t s);   // DIRMULT: cnt_q of every count view at beta_v
+// the beta step of every count view (flags: the finalize flags of the same rebuild), then the refresh of what depends on
+// beta in the views whose step accepted; refresh_only: no step, refresh the views whose cb_accept is set
+cudaError_t launch_count_beta(const Ctx& c, int32_t flags, bool refresh_only, cudaStream_t s);
+// the (float) W beta + C_k of a count view's dish: TableParam::C1 and the base of its denominator table
+__host__ __device__ __forceinline__ double count_wbeta_total(int vocab, double beta, double total) { return (double)vocab * beta + total; }
 // posterior summaries (mv_summary.cu)
 cudaError_t launch_labels(const Ctx& c, int32_t* out, cudaStream_t s);
 cudaError_t launch_cocluster(const Ctx& c, int view, uint32_t* counts, cudaStream_t s);

@@ -27,7 +27,9 @@ enum PhiloxDomain : uint32_t {
   kDomHyperUnif = 3,    // hyper-step acceptance uniforms           (multiview_hyper.cpp:228,253,260,279,286)
   kDomInitTable = 4,    // random initial table                     (multiview_gibbs.cpp:26)
   kDomInitDish = 5,     // random initial dish, slot = view         (multiview_gibbs.cpp:56)
-  kDomCallSeq = 6       // call-ordered host stream (multiview_rng.h mirror)
+  kDomCallSeq = 6,      // call-ordered host stream (multiview_rng.h mirror)
+  kDomCountBeta = 7     // beta step of count view `slot`: index 0 the proposal normal, 1 the acceptance uniform
+                        // (sweep = the sweep index of the hyper step's tau draws)
 };
 
 struct U4 { uint32_t x, y, z, w; };

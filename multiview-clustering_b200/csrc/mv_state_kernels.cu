@@ -622,10 +622,10 @@ __device__ __noinline__ double log_f_dish_counts_dm(const int32_t* __restrict__ 
 // few arguments keeps the finalize kernel's register budget.
 __device__ __noinline__ double birth_log_f_counts(const int32_t* __restrict__ rp, const int32_t* __restrict__ col,
                                                   const float* __restrict__ val, const int32_t* __restrict__ cnt_d,
-                                                  const int cap, const int vocab, const float beta_f, const double ctot_k,
+                                                  const int cap, const int vocab, const double beta, const double ctot_k,
                                                   const int tk, const int row, const int mode) {
   const bool loo = (mode & 1) != 0, new_dish = (mode & 2) != 0, dm = (mode & 4) != 0;
-  const double beta = (double)beta_f, wbeta = (double)vocab * (double)beta_f;
+  const double wbeta = (double)vocab * beta;
   if (dm) return log_f_dish_counts_dm(rp, col, val, cnt_d, cap, wbeta, beta, ctot_k, new_dish ? -1 : tk, row, loo && !new_dish);
   if (new_dish) {                    // plug-in: log f_new = -|x| log W
     double tot = 0.0;
@@ -782,7 +782,7 @@ __global__ void __launch_bounds__(kFinThreads, 1) k_finalize(const Ctx c, const 
           const int row = pkt_i32(c, S.cand_g[b], c.pkt.off_cand_row)[S.cand_j[b]];
           const int t0 = pkt_i32(c, S.cand_g[b], c.pkt.off_cand_t0)[S.cand_j[b]];
           const bool own = (k < cap) && (k == S.dish[t0]) && S.n_vk[k] > 0;
-          val = birth_log_f_counts(c.rowptr[v], c.col[v], c.val[v], c.cnt_d[v], cap, c.vocab[v], c.count_beta,
+          val = birth_log_f_counts(c.rowptr[v], c.col[v], c.val[v], c.cnt_d[v], cap, c.vocab[v], c.beta_v[v],
                                    (k < cap) ? S.s2k_start[k] : 0.0, (k < cap) ? S.table_of_dish[k] : -1, row,
                                    (own ? 1 : 0) | (k == cap ? 2 : 0) | (c.count_model ? 4 : 0));
         } else if (k == cap) {   // new dish: N(x; 0, tau)   (multiview_utils.cpp:340-350)
@@ -1220,7 +1220,7 @@ __global__ void __launch_bounds__(kFinThreads, 1) k_finalize(const Ctx c, const 
       // count view: the dot products are log2 f already (C + A (2 acc - 0) = acc); C1 carries W beta + the token
       // total of the dish for the leave-one-out term of the kernel
       q.A = 0.5f; q.C = 0.f; q.A1 = 0.f;
-      q.C1 = (float)((double)c.vocab[v] * (double)c.count_beta + S.s2k[k]);
+      q.C1 = (float)count_wbeta_total(c.vocab[v], c.beta_v[v], S.s2k[k]);
       const bool rep = (S.tmask[k].lowest() == t);
       const double w = (double)S.l_live[k] - sigma_l, w1 = w - 1.0;
       q.W = (rep && w > 0.0) ? (float)fin_log2(w) : kMasked;

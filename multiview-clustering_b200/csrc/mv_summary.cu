@@ -82,7 +82,7 @@ __global__ void __launch_bounds__(256) k_loglik(const Ctx c, double* __restrict_
         s_rep[k] = rep;
       }
       __syncthreads();
-      term = loglik_dirmult_term(c.cnt_d[v], c.S2k + v * c.cap, c.vocab[v], c.cap, (double)c.count_beta, s_rep);
+      term = loglik_dirmult_term(c.cnt_d[v], c.S2k + v * c.cap, c.vocab[v], c.cap, c.beta_v[v], s_rep);
     } else {
       for (int k = threadIdx.x; k < c.cap; k += blockDim.x) {
         const int n = c.n_vk[v * c.cap + k];

@@ -95,6 +95,10 @@ def lib():
         L.mvg_get_count_tables.argtypes = [H, C.c_int32, _f32p, _i32p, _i32p]
         L.mvg_set_count_likelihood.argtypes = [H, C.c_int32]
         L.mvg_get_count_den.argtypes = [H, C.c_int32, _f32p, _i32p]
+        L.mvg_set_count_beta_prior.argtypes = [H, C.c_double, C.c_double, C.c_double]
+        L.mvg_get_count_beta.argtypes = [H, _f64p]
+        L.mvg_get_count_beta_step.argtypes = [H, _f64p, _i32p]
+        L.mvg_set_count_beta_trace.argtypes = [H, _f64p]
         L.mvg_get_debug_loo.argtypes = [H, _f32p]
         L.mvg_init_state_reference.argtypes = [H]
         L.mvg_set_state.argtypes = [H, C.POINTER(_StateHost)]
@@ -192,6 +196,7 @@ class Sampler:
             raise MvgError(rc, self.L.mvg_last_error(None).decode())
         self._keep = []
         self.count_likelihood = "plugin"
+        self.count_beta_prior = None
 
     # -- plumbing ---------------------------------------------------------------------------
     def _ck(self, rc):
@@ -242,6 +247,26 @@ class Sampler:
             raise MvgError(-1, f"unknown count likelihood {model!r}: expected one of {sorted(COUNT_LIKELIHOODS)}")
         self._ck(self.L.mvg_set_count_likelihood(self.h, COUNT_LIKELIHOODS[model]))
         self.count_likelihood = model
+
+    def set_count_beta_prior(self, shape, rate, step=0.3):
+        """Learn beta of every "dirmult" count view: a Gamma(shape, rate) prior and one log-normal random-walk
+        Metropolis-Hastings step of scale ``step`` per view per hyper step (step 0.3 as the tau step's proposal).  Before
+        the first state call."""
+        self._ck(self.L.mvg_set_count_beta_prior(self.h, float(shape), float(rate), float(step)))
+        self.count_beta_prior = (float(shape), float(rate), float(step))
+
+    def get_count_beta(self):
+        """[V] float64: beta of every count view (0 for a dense view)."""
+        out = np.empty(self.V, np.float64)
+        self._ck(self.L.mvg_get_count_beta(self.h, _p(out, _f64p)))
+        return out
+
+    def get_count_beta_step(self):
+        """(log A [V], accepted [V]) of the most recent beta step."""
+        la = np.empty(self.V, np.float64)
+        acc = np.empty(self.V, np.int32)
+        self._ck(self.L.mvg_get_count_beta_step(self.h, _p(la, _f64p), _p(acc, _i32p)))
+        return la, acc
 
     def get_count_den(self, v):
         """"dirmult" count view v: (den [n_max + 1, cap], n_max), den[n][t] = sum_{j<n} log2(W beta + C_k + j) of the dish
@@ -443,12 +468,20 @@ class Sampler:
         hyp = np.empty((max(n_saved_max, 1), 3 * self.V + 2), np.float64)
         ll = np.zeros(max(n_saved_max, 1), np.float64)
         ns = C.c_int32(0)
+        beta = np.empty((max(n_saved_max, 1), self.V), np.float64) if self.count_beta_prior else None
+        if beta is not None:
+            self._ck(self.L.mvg_set_count_beta_trace(self.h, _p(beta, _f64p)))
         # the log-likelihood kernel covers the Gaussian views and the Dirichlet-multinomial count views
         dense = all(d > 0 for d in self.dims) or self.count_likelihood == "dirmult"
         self._ck(self.L.mvg_run(self.h, M, burn_in, thin, n_saved_max, _p(tab, _i32p), _p(dish, _i32p),
                                 _p(hyp, _f64p), _p(ll, _f64p) if dense else None, C.byref(ns)))
+        if beta is not None:
+            self._ck(self.L.mvg_set_count_beta_trace(self.h, None))
         S = ns.value
-        return {"table_of": tab[:S], "dish_of": dish[:S], "hypers": hyp[:S], "loglik": ll[:S] if dense else ll[:0]}
+        out = {"table_of": tab[:S], "dish_of": dish[:S], "hypers": hyp[:S], "loglik": ll[:S] if dense else ll[:0]}
+        if beta is not None:
+            out["count_beta"] = beta[:S]
+        return out
 
     # -- multi-GPU ----------------------------------------------------------------------------
     @staticmethod
@@ -566,7 +599,7 @@ def _as_csr(v):
 
 
 def run_gibbs(data_views, M, burn_in, thin, cap=64, seed=1999, device=0, engine=ENGINE_AUTO, start=None, blocks=1,
-              count_likelihood="plugin"):
+              count_likelihood="plugin", count_beta_prior=None):
     """run_gibbs_cpp(data_views, M, burn_in, thin) on the GPU (multiview_gibbs.cpp:105-131).
 
     ``data_views`` is a list of per-view arrays (vectors as in New_Simulation.R:105-111, or [n, D]
@@ -574,7 +607,8 @@ def run_gibbs(data_views, M, burn_in, thin, cap=64, seed=1999, device=0, engine=
     scipy.sparse matrix or a dict {"rowptr", "col", "val", "vocab"}.  ``start`` = (table_of, dish_of) replaces the
     reference's random T = 4 / K = 2 start.  Returns a dict with the reference's eight keys; ``table_of`` is
     0-based, ``dish_of`` is indexed [saved][view][table slot] with -1 for a free slot.  ``count_likelihood`` is
-    "plugin" or "dirmult" (Sampler.set_count_likelihood).
+    "plugin" or "dirmult" (Sampler.set_count_likelihood).  ``count_beta_prior`` = (shape, rate) or (shape, rate, step)
+    learns beta of every "dirmult" count view (Sampler.set_count_beta_prior); the result then has "count_beta" [S][V].
     """
     csr = [_as_csr(v) for v in data_views]
     views = [None if c is not None else np.asarray(v, dtype=np.float64).reshape(len(v), -1) for v, c in zip(data_views, csr)]
@@ -590,6 +624,8 @@ def run_gibbs(data_views, M, burn_in, thin, cap=64, seed=1999, device=0, engine=
             s.set_sweep_blocks(blocks)
         if count_likelihood != "plugin":
             s.set_count_likelihood(count_likelihood)
+        if count_beta_prior is not None:
+            s.set_count_beta_prior(*count_beta_prior)
         if start is None:
             s.init_state_reference()
         else:
@@ -600,7 +636,7 @@ def run_gibbs(data_views, M, burn_in, thin, cap=64, seed=1999, device=0, engine=
         s.close()
     V = len(views)
     hyp = tr["hypers"]
-    return {
+    out = {
         "table_of": [t for t in tr["table_of"]],
         "dish_of": [[d[v] for v in range(V)] for d in tr["dish_of"]],
         "loglik": list(tr["loglik"]),                   # the reference declares it and never fills it (multiview_state.h:38)
@@ -610,6 +646,9 @@ def run_gibbs(data_views, M, burn_in, thin, cap=64, seed=1999, device=0, engine=
         "alpha_global": hyp[:, 3 * V],
         "sigma_global": hyp[:, 3 * V + 1],
     }
+    if "count_beta" in tr:
+        out["count_beta"] = tr["count_beta"]
+    return out
 
 
 def run_gibbs_seq(data_views, M, burn_in, thin, seed=1999, device=0, t_cap=1024, k_cap=None):
